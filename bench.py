@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this framework (CUDA, sm_100a)
     python bench.py --impl reference --steps K --warmup W     # reference algorithm on the host CPUs (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one full DDIMSampler.sample() call: 50 DDIM steps x UNet on [cond ; uncond] (batch 16) for 8
 images per GPU, guidance annealed (4 -> 1), eta 0, random-init SD-1.5-architecture weights, synthetic
@@ -84,6 +85,24 @@ class ClockSampler:
         loaded = sm[len(sm) // 2:] if sm else []
         med = loaded[len(loaded) // 2] if loaded else None
         return {"sm_mhz": med, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """--dump-outputs: writes each tensor as out_dir/<name>.npy (float64 stays float64, everything else becomes float32)
+    so that two builds run with the same arguments, hence the same seeded inputs, can be compared output for output."""
+    import numpy as np
+    import torch
+    host = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).numpy()
+            for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_config(world: int, graph: bool = True):
@@ -271,7 +290,14 @@ def main():
     ap.add_argument("--breakdown", action="store_true", help="print the per-kernel-class table to stderr")
     ap.add_argument("--no-train", action="store_true", help="skip the Stage-1 training leg (train_step key)")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity gate / GPU eager baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each leg returned (rank 0) as DIR/<name>.npy: the sampler's "
+                         "samples and intermediates, the decoded images, the training step's loss and gradient norm")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     # stdout carries exactly ONE line (the JSON record): anything a library prints there (NCCL's version banner on the
     # first communicator, ...) is sent to stderr for the duration of the run
     sys.stdout.flush()
@@ -324,13 +350,16 @@ def main():
     extra = {"use_layerwise_context": True, "use_conv_attn_kernel_size": -1, "placeholder2indices": None,
              "is_training": False}
 
-    def one_call(c, uc, x_T):
+    def sample(c, uc, x_T):
+        """-> (samples, intermediates), what DDIMSampler.sample returns to its caller."""
         cond = (c, prompts, dict(extra))
         uncond = (uc, [""] * b, dict(extra))
-        samples, _ = sampler.sample(DDIM_STEPS, b, [4, LATENT, LATENT], conditioning=cond,
-                                    unconditional_conditioning=uncond, guidance_scale=GUIDANCE, eta=0.0, x_T=x_T,
-                                    verbose=False)
-        return samples
+        return sampler.sample(DDIM_STEPS, b, [4, LATENT, LATENT], conditioning=cond,
+                              unconditional_conditioning=uncond, guidance_scale=GUIDANCE, eta=0.0, x_T=x_T,
+                              verbose=False)
+
+    def one_call(c, uc, x_T):
+        return sample(c, uc, x_T)[0]
 
     def fresh_device_inputs():
         return host["c"].to(dev), host["uc"].to(dev), host["x_T"].to(dev)
@@ -356,10 +385,12 @@ def main():
         return float(ms.item())
 
     # ---- value: inputs resident in HBM -------------------------------------------------------------------
+    resident = {}          # the result of the latest call (--dump-outputs writes the last timed one)
+
     def step_resident():
         # new context tensors per call => the per-prompt K/V projection cache is rebuilt inside the timed
         # region (SURVEY.md section 8(d): "KV cache warm-up included"); clones are device-to-device.
-        one_call(dev_in[0].clone(), dev_in[1].clone(), dev_in[2])
+        resident["out"] = sample(dev_in[0].clone(), dev_in[1].clone(), dev_in[2])
 
     dev_in = fresh_device_inputs()
     for _ in range(max(3, args.warmup)):
@@ -373,6 +404,13 @@ def main():
     clock_info = clocks.stop() if rank == 0 else None
     ms_per_step = ms_total / args.steps
     value = world * b * args.steps / (ms_total / 1e3)
+    dumps = {}
+    if args.dump_outputs:
+        samples, inter = resident.pop("out")
+        dumps["samples"] = samples
+        for key in ("x_inter", "pred_x0"):
+            dumps.update({f"{key}_{i}": t for i, t in enumerate(inter[key])})
+    resident.clear()
 
     # ---- e2e: host buffers in, host latents out, through the same public API ---------------------------------
     def step_e2e():
@@ -411,6 +449,8 @@ def main():
 
         step_e2e_rgb()
         ms_rgb = timed(step_e2e_rgb, args.steps) / args.steps
+        if args.dump_outputs:
+            dumps["images"] = rgb_host.clone()
         vae_info = {"decode_ms_per_8_images": ms_dec, "decode_tflops": b * VAE_GFLOP_PER_IMAGE / 1e3 / (ms_dec / 1e3),
                     "e2e_rgb_images_per_sec": world * b / (ms_rgb / 1e3), "d2h_bytes_per_step": rgb_host.numel() * 4,
                     "note": "sampling + decode_first_stage, host prompts/noise in, host 512x512 RGB out"}
@@ -512,7 +552,9 @@ def main():
         sampler.__dict__.pop("_step_graphs", None)
         sampler._graphs = {}
         torch.cuda.empty_cache()
-        train_info = train_leg(dev, unet, world, rank, max(2, args.steps))
+        train_info = train_leg(dev, unet, world, rank, args.steps)
+        if args.dump_outputs:
+            dumps.update({f"train_{k}": torch.tensor(train_info[k], dtype=torch.float64) for k in ("loss", "grad_norm")})
 
     # ---- CPU baseline (rank 0, N = 1 only): the oracle port on the host cores, bounded sample ---------------
     cpu_baseline = None
@@ -542,6 +584,8 @@ def main():
             "gpu_eager_baseline": oracle_legs.get("gpu_eager_baseline"),
             "train_step": train_info,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -292,3 +292,22 @@ def test_import_path_aliases_resolve_to_the_mirrors():
     finally:
         for k in [k for k in sys.modules if (k == "ldm" or k == "adaface" or k.startswith(("ldm.", "adaface."))) and k not in before]:
             del sys.modules[k]
+
+
+def test_bench_dump_outputs_format_and_limit(tmp_path):
+    import os
+    import subprocess
+    import sys
+
+    import bench
+    out = tmp_path / "dump"
+    x = torch.randn(2, 4, dtype=torch.bfloat16)
+    bench.dump_outputs(str(out), {"samples": x, "loss": torch.tensor(1.25, dtype=torch.float64)})
+    s, loss = np.load(out / "samples.npy"), np.load(out / "loss.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, x.float().numpy())
+    assert loss.dtype == np.float64 and loss == 1.25
+    with pytest.raises(SystemExit):      # over the 64 MB budget: nothing is written
+        bench.dump_outputs(str(tmp_path / "big"), {"x": torch.zeros(bench.DUMP_MAX_BYTES // 4 + 1)})
+    assert not (tmp_path / "big").exists()
+    r = subprocess.run([sys.executable, os.path.abspath(bench.__file__), "--steps", "0"], capture_output=True, text=True)
+    assert r.returncode == 2 and "--steps" in r.stderr
