@@ -367,6 +367,40 @@ static int launch_attention(const AttnParams& p, cudaStream_t stream) {
   return 0;
 }
 
+// A sample whose key mask keeps no key.  The reference fills masked scores with -finfo.max (attention.py:223-232), so
+// such a row's softmax is uniform over the sample's Nk keys and its output is the mean of V over them.  The attention
+// kernels end these rows with a zero row sum instead; this pass, run after whichever kernel ran, overwrites them with
+// that mean (fp32 sum, rounded to bf16) and their lse with +inf.  grid (ceil(heads*d / 32), B), 256 threads: a block
+// owns 32 channels of one sample and returns at once when the sample attends to any key.
+__global__ void __launch_bounds__(256) attention_empty_mask_kernel(const uint8_t* __restrict__ key_mask,
+                                                                   const __nv_bfloat16* __restrict__ Vt, long long ldvt,
+                                                                   int kv_stride, int heads, int Nq, int Nk, int d,
+                                                                   __nv_bfloat16* __restrict__ out, float* __restrict__ lse) {
+  const int b = blockIdx.y;
+  const int C = heads * d;
+  const int c0 = blockIdx.x * 32;
+  const uint8_t* m = key_mask + static_cast<size_t>(b) * Nk;
+  int any = 0;
+  for (int j = threadIdx.x; j < Nk; j += blockDim.x) any |= m[j];
+  if (__syncthreads_or(any)) return;
+  __shared__ float mean[32];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int c = warp; c < 32 && c0 + c < C; c += 8) {
+    const __nv_bfloat16* row = Vt + static_cast<size_t>(c0 + c) * ldvt + static_cast<size_t>(b) * kv_stride;
+    float s = 0.f;
+    for (int j = lane; j < Nk; j += 32) s += __bfloat162float(row[j]);
+    s = warp_sum(s);
+    if (lane == 0) mean[c] = s / static_cast<float>(Nk);
+  }
+  __syncthreads();
+  if (c0 + lane < C) {
+    const __nv_bfloat16 v = __float2bfloat16(mean[lane]);
+    for (int i = warp; i < Nq; i += 8) out[(static_cast<size_t>(b) * Nq + i) * C + c0 + lane] = v;
+  }
+  if (lse != nullptr && blockIdx.x == 0)
+    for (int i = threadIdx.x; i < heads * Nq; i += blockDim.x) lse[static_cast<size_t>(b) * heads * Nq + i] = INFINITY;
+}
+
 }  // namespace af
 
 namespace af {
@@ -405,9 +439,27 @@ extern "C" int af_attention_bf16_trace(const void* Q, long long ldq, const void*
   return attention_impl(Q, ldq, K, ldk, Vt, ldvt, kv_stride, nullptr, O, nullptr, trace, B, heads, Nq, Nk, d, stream);
 }
 
+// picks and launches one of the three kernel families from the shape
+static int attention_launch(const void* Q, long long ldq, const void* K, long long ldk, const void* Vt, long long ldvt,
+                            int kv_stride, const unsigned char* key_mask, void* O, float* lse, long long* trace, int B,
+                            int heads, int Nq, int Nk, int d, cudaStream_t stream);
+
 static int attention_impl(const void* Q, long long ldq, const void* K, long long ldk, const void* Vt, long long ldvt,
                           int kv_stride, const unsigned char* key_mask, void* O, float* lse, long long* trace, int B,
                           int heads, int Nq, int Nk, int d, cudaStream_t stream) {
+  const int rc = attention_launch(Q, ldq, K, ldk, Vt, ldvt, kv_stride, key_mask, O, lse, trace, B, heads, Nq, Nk, d,
+                                  stream);
+  if (rc != 0 || key_mask == nullptr) return rc;
+  dim3 grid((heads * d + 31) / 32, B);
+  attention_empty_mask_kernel<<<grid, 256, 0, stream>>>(key_mask, static_cast<const __nv_bfloat16*>(Vt), ldvt, kv_stride,
+                                                        heads, Nq, Nk, d, static_cast<__nv_bfloat16*>(O), lse);
+  AF_LAUNCH_CHECK("attention_empty_mask_kernel");
+  return 0;
+}
+
+static int attention_launch(const void* Q, long long ldq, const void* K, long long ldk, const void* Vt, long long ldvt,
+                            int kv_stride, const unsigned char* key_mask, void* O, float* lse, long long* trace, int B,
+                            int heads, int Nq, int Nk, int d, cudaStream_t stream) {
   AF_CHECK_ARG(Q && K && Vt && O, "af_attention_bf16: null pointer");
   AF_CHECK_ARG(d == 40 || d == 80 || d == 160, "af_attention_bf16: head dim %d unsupported (40/80/160)", d);
   AF_CHECK_ARG(B > 0 && heads > 0 && Nq > 0 && Nk > 0 && kv_stride >= Nk, "af_attention_bf16: bad sizes");

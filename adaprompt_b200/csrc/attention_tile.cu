@@ -556,7 +556,9 @@ static int launch_tile_m(const AttnTileParams& p, cudaStream_t stream) {
 }
 template <int D, int POLY>
 static int launch_tile(const AttnTileParams& p, cudaStream_t stream) {
-  if (p.key_mask != nullptr || p.Nk % TileCfg<D>::BLOCK_N != 0) return launch_tile_m<D, POLY, true, false>(p, stream);
+  // the masked kernel takes every exponential from fast_exp2: tile_exp2_poly clamps its argument to -126, so a masked
+  // key (score -inf) would get weight 2^-126 instead of 0 and enter P.V and the row sum
+  if (p.key_mask != nullptr || p.Nk % TileCfg<D>::BLOCK_N != 0) return launch_tile_m<D, 0, true, false>(p, stream);
   if (p.trace != nullptr) return launch_tile_m<D, POLY, false, true>(p, stream);
   return launch_tile_m<D, POLY, false, false>(p, stream);
 }

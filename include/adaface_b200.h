@@ -107,7 +107,9 @@ int af_conv3x3_gn_slots(int Ho, int Wo);
  * Q [B,Nq,ldq], K [B,Nk,ldk] bf16 with head h at column h*DP (DP = 48 for d = 40, zero padded, else d);
  * Q pre-scaled by d^-1/2 * log2(e).  Vt [heads*d, ldvt] bf16 = V transposed.  Sample b's keys start at row
  * b*kv_stride of K and at column b*kv_stride of Vt (kv_stride >= Nk; the cached 77-token context uses 80).
- * key_mask [B,Nk] bytes (1 = attend) or NULL (attention.py:223-232).  O [B,Nq,heads*d] bf16. */
+ * key_mask [B,Nk] bytes (1 = attend) or NULL (attention.py:223-232).  Masked scores are filled with -finfo.max as in
+ * the reference, so every query row of a sample whose mask keeps no key gets the mean of V over the sample's Nk keys
+ * (fp32 sum, bf16 result), and lse (af_attention_bf16_lse) is +inf in those rows.  O [B,Nq,heads*d] bf16. */
 int af_attention_bf16(const void* Q, long long ldq, const void* K, long long ldk, const void* Vt, long long ldvt,
                       int kv_stride, const unsigned char* key_mask, void* O, int B, int heads, int Nq, int Nk, int d,
                       af_stream_t stream);

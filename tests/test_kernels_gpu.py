@@ -146,10 +146,52 @@ def test_conv3x3_dual_source_rowbias_residual():
 
 
 # ------------------------------------------------------------------------------------------------ attention
-def _attn_case(B, N, Nk, d, seed=0, mask=False, cross=False, boost=None):
-    """boost = (first_key, factor): keys from first_key on are scaled, so that scores far above the first block's appear
-    late in the key loop (the lazy-reference / overflow paths of the attention kernels)."""
-    from adaprompt_b200 import ops
+ATTN_ROW_TOL = 1e-2       # worst rel-L2 over (sample, head, query row); 4.5e-3 seen on a B200
+# |lse - ref| in log2 units.  The tile kernels sum l from the bf16-rounded P, whose relative error is up to 2^-8; a row
+# dominated by one key (large scores) reaches log2(1 + 2^-8) = 5.62e-3 (seen: 5.63e-3, 2.3e-3 without dominant keys)
+ATTN_LSE_TOL = 6e-3
+POISON = 2.0 ** 127       # finite and exact in bf16; 0 * POISON = 0 where the kernels give a key exactly zero weight
+
+
+def _attn_ref(qs, kb, vb, km=None):
+    """af_attention_bf16 in float64 (attention.py:198-242) on the kernel's bf16 operands; CPU or CUDA tensors.
+    qs [B, Nq, h, d] carries d^-1/2 * log2(e), so the scores s are in the exp2 domain; kb, vb [B, Nk, h, d]; km [B, Nk]
+    (nonzero = attend) or None.  Masked scores are filled with -finfo.max as in the reference, so a sample that attends
+    to no key gets a uniform softmax.  -> (O [B, Nq, h*d], lse [B, h, Nq] = log2 sum_j 2^s_j over the attended keys, +inf
+    where there are none)."""
+    B, Nq, h, d = qs.shape
+    s = torch.einsum("bihd,bjhd->bhij", qs.double(), kb.double())
+    keep = torch.ones(B, kb.shape[1], dtype=torch.bool, device=s.device) if km is None else km.bool()
+    keep = keep[:, None, None, :]
+    p = torch.softmax(s.masked_fill(~keep, -torch.finfo(torch.float64).max) * math.log(2.0), dim=-1)
+    o = torch.einsum("bhij,bjhd->bihd", p, vb.double()).reshape(B, Nq, h * d)
+    lse = torch.logsumexp(s.masked_fill(~keep, float("-inf")) * math.log(2.0), dim=-1) / math.log(2.0)
+    return o, lse.masked_fill(torch.isneginf(lse), float("inf"))
+
+
+def _attn_errors(out, lse, ref, ref_lse):
+    """Global rel-L2 of O, the worst rel-L2 over (sample, head, query row) and the worst |lse - ref|.  Rows whose
+    reference lse is +inf must be +inf in lse too (a non-finite difference otherwise)."""
+    B, Nq, C = ref.shape
+    heads = lse.shape[1]
+    diff = out.double() - ref
+    rows = diff.view(B, Nq, heads, -1).norm(dim=-1) / ref.view(B, Nq, heads, -1).norm(dim=-1).clamp_min(1e-30)
+    inf = torch.isinf(ref_lse)
+    lse_d = lse.double()
+    lse_err = torch.where(inf, torch.where(lse_d == ref_lse, 0.0, float("inf")), (lse_d - ref_lse).abs())
+    return {"rel": (diff.norm() / ref.norm()).item(), "row": rows.max().item(), "lse": lse_err.max().item()}
+
+
+def _attn_case(B, N, Nk, d, seed=0, mask=False, cross=False, boost=None, poison=False, empty=None, tol=6e-3):
+    """Runs ops.attention_lse and ops.attention on one problem: the two O must be bit-identical, and O / lse must match
+    _attn_ref (global rel-L2 < tol, worst row < ATTN_ROW_TOL, lse < ATTN_LSE_TOL).
+    cross: keys stored with a sample stride padded to a multiple of 8 (the cached-context layout).
+    mask: random key mask that keeps key 0; empty: index of a sample whose mask keeps no key.
+    boost = (first_key, factor): keys from first_key on are scaled, so that scores far above the first block's appear
+    late in the key loop (the lazy-reference / overflow paths of the attention kernels).
+    poison: the V^T columns that must get zero weight hold +-2^127 - masked keys of samples that attend to some key,
+    [Nk, kv_stride) of every sample and [B*kv_stride, ldvt) - and masked keys' K rows are scaled by 2^10 (a maximum taken
+    before masking would see them).  Returns the errors."""
     heads = 8
     C = heads * d
     dp = 48 if d == 40 else d
@@ -161,34 +203,70 @@ def _attn_case(B, N, Nk, d, seed=0, mask=False, cross=False, boost=None):
         k[:, boost[0]:] *= boost[1]
     qs = (q * (scale * math.log2(math.e))).to(torch.bfloat16)
     kb, vb = k.to(torch.bfloat16), v.to(torch.bfloat16)
-    qbuf = torch.zeros(B, N, heads, dp, device=DEV, dtype=torch.bfloat16)
-    nk_pad = ((Nk + 7) // 8) * 8 if cross else Nk
-    kbuf = torch.zeros(B, nk_pad, heads, dp, device=DEV, dtype=torch.bfloat16)
-    qbuf[..., :d] = qs
-    kbuf[:, :Nk, :, :d] = kb
-    vt = torch.zeros(C, B * nk_pad, device=DEV, dtype=torch.bfloat16)
-    vt.view(C, B, nk_pad)[:, :, :Nk] = vb.permute(2, 3, 0, 1).reshape(C, B, Nk)
     km = None
-    if mask:
+    if mask or empty is not None:
         g = torch.Generator().manual_seed(seed + 9)
         km = (torch.rand(B, Nk, generator=g) > 0.3).to(torch.uint8).to(DEV)
         km[:, 0] = 1
-    out = torch.empty(B, N, C, device=DEV, dtype=torch.bfloat16)
-    ops.attention(qbuf, kbuf, vt, out, B=B, heads=heads, Nq=N, Nk=Nk, d=d, ldq=heads * dp, ldk=heads * dp,
-                  ldvt=B * nk_pad, kv_stride=nk_pad, key_mask=km)
-    # reference: attention.py:198-242 on the same bf16-rounded operands (q carries scale*log2e -> use exp2)
-    s = torch.einsum("bihd,bjhd->bhij", qs.float(), kb.float())
-    if km is not None:
-        s = s.masked_fill(~km.bool()[:, None, None, :], float("-inf"))
-    p = torch.softmax(s * math.log(2.0), dim=-1)
-    ref = torch.einsum("bhij,bjhd->bihd", p, vb.float()).reshape(B, N, C)
-    return _rel(out, ref)
+        if empty is not None:
+            km[empty] = 0
+    ref, ref_lse = _attn_ref(qs, kb, vb, km)
+
+    qbuf = torch.zeros(B, N, heads, dp, device=DEV, dtype=torch.bfloat16)
+    nk_pad = ((Nk + 7) // 8) * 8 if cross else Nk
+    ldvt = (max(64, B * nk_pad) + 7) // 8 * 8 + (64 if poison else 0)     # a multiple of 8 (16-byte TMA rows)
+    kbuf = torch.zeros(B, nk_pad, heads, dp, device=DEV, dtype=torch.bfloat16)
+    qbuf[..., :d] = qs
+    kbuf[:, :Nk, :, :d] = kb
+    vt = torch.zeros(C, ldvt, device=DEV, dtype=torch.bfloat16)
+    vt3 = vt[:, :B * nk_pad].view(C, B, nk_pad)
+    vt3[:, :, :Nk] = vb.permute(2, 3, 0, 1).reshape(C, B, Nk)
+    if poison:
+        g = torch.Generator().manual_seed(seed + 10)
+
+        def big(*shape):
+            return ((torch.randint(0, 2, shape, generator=g) * 2 - 1) * POISON).to(torch.bfloat16).to(DEV)
+
+        vt3[:, :, Nk:] = big(C, B, nk_pad - Nk)
+        vt[:, B * nk_pad:] = big(C, ldvt - B * nk_pad)
+        if km is not None:
+            dead = (km == 0) & (km.sum(1, keepdim=True) > 0)
+            vt3[:, :, :Nk] = torch.where(dead[None], big(C, B, Nk), vt3[:, :, :Nk])
+            kv = kbuf[:, :Nk]
+            kv[km == 0] = kv[km == 0] * 1024.0
+
+    return _attn_check(qbuf, kbuf, vt, ref, ref_lse, tol, dict(
+        B=B, heads=heads, Nq=N, Nk=Nk, d=d, ldq=heads * dp, ldk=heads * dp, ldvt=ldvt, kv_stride=nk_pad, key_mask=km),
+        f"mask={mask} cross={cross} boost={boost} poison={poison} empty={empty}")
+
+
+def _attn_check(q, k, vt, ref, ref_lse, tol, args, label=""):
+    """ops.attention_lse and ops.attention on the same operands (args: their keyword arguments): the two O must be
+    bit-identical, and O / lse must match the reference (global rel-L2 < tol, worst row < ATTN_ROW_TOL, lse <
+    ATTN_LSE_TOL).  Prints the errors and returns them."""
+    from adaprompt_b200 import ops
+    B, Nq, heads = args["B"], args["Nq"], args["heads"]
+    out = torch.full((B, Nq, ref.shape[-1]), float("nan"), device=DEV, dtype=torch.bfloat16)
+    out2 = torch.full_like(out, float("nan"))
+    lse = torch.full((B, heads, Nq), float("nan"), device=DEV)
+    ops.attention_lse(q, k, vt, out, lse, **args)
+    ops.attention(q, k, vt, out2, **args)
+    assert torch.equal(out, out2), "attention and attention_lse disagree"
+    e = _attn_errors(out, lse, ref, ref_lse)
+    print(f"\nattention B={B} Nq={Nq} Nk={args['Nk']} d={args['d']} {label}: rel {e['rel']:.2e}  "
+          f"worst row {e['row']:.2e}  lse {e['lse']:.2e}")
+    assert e["rel"] < tol and e["row"] < ATTN_ROW_TOL and e["lse"] < ATTN_LSE_TOL, e
+    return e
 
 
 @pytest.mark.parametrize("B,N,d", [(1, 4096, 40), (2, 1024, 80), (2, 256, 160), (3, 64, 160), (1, 2304, 80),
-                                   (2, 144, 160), (1, 576, 160)])
+                                   (2, 144, 160), (1, 576, 160),
+                                   (3, 296, 40),       # ragged last key block: masked tile kernel, d = 40
+                                   (2, 1600, 40),      # the 40x40 latent
+                                   (2, 144, 80),       # the 12x12 map: masked tile kernel, d = 80
+                                   (2, 64, 40)])       # generic kernel, d = 40
 def test_self_attention(B, N, d):
-    assert _attn_case(B, N, N, d) < 6e-3
+    _attn_case(B, N, N, d)
 
 
 @pytest.mark.parametrize("B,N,d,first,factor", [
@@ -200,18 +278,17 @@ def test_self_attention(B, N, d):
 def test_self_attention_large_scores_late_in_the_key_loop(B, N, d, first, factor):
     """Rows whose maximum moves far away from the first block's: the result must be the exact softmax (no inf / NaN, no
     stale reference) whichever path the kernel takes to get there."""
-    assert _attn_case(B, N, N, d, seed=11, boost=(first, factor)) < 8e-3
+    _attn_case(B, N, N, d, seed=11, boost=(first, factor), tol=8e-3)
 
 
 @pytest.mark.parametrize("B,N,d", [(2, 4096, 40), (2, 1024, 80), (2, 256, 160), (2, 64, 160)])
 def test_cross_attention_77(B, N, d):
-    assert _attn_case(B, N, 77, d, seed=5, cross=True) < 6e-3
+    _attn_case(B, N, 77, d, seed=5, cross=True)
 
 
 @pytest.mark.parametrize("B,N,d", [(2, 1024, 40), (2, 256, 80), (3, 64, 160), (2, 16, 160)])
 def test_self_attention_fused_qk_buffer(B, N, d):
     """Layout the UNet uses: one [tokens, Q|K] buffer (K = column view), V^T [C, tokens]."""
-    from adaprompt_b200 import ops
     heads, C = 8, 8 * d
     dp = 48 if d == 40 else d
     q = _rand(B, N, heads, d, seed=11)
@@ -226,18 +303,13 @@ def test_self_attention_fused_qk_buffer(B, N, d):
     ldvt = max(64, B * N)
     vt = torch.zeros(C, ldvt, device=DEV, dtype=torch.bfloat16)
     vt[:, :B * N] = vb.permute(2, 3, 0, 1).reshape(C, B * N)
-    out = torch.empty(B * N, C, device=DEV, dtype=torch.bfloat16)
-    ops.attention(qk, qk[:, heads * dp:], vt, out, B=B, heads=heads, Nq=N, Nk=N, d=d, ldq=2 * heads * dp,
-                  ldk=2 * heads * dp, ldvt=ldvt, kv_stride=N)
-    s = torch.einsum("bihd,bjhd->bhij", qs.float(), kb.float())
-    p = torch.softmax(s * math.log(2.0), dim=-1)
-    ref = torch.einsum("bhij,bjhd->bihd", p, vb.float()).reshape(B * N, C)
-    assert _rel(out, ref) < 6e-3
+    ref, ref_lse = _attn_ref(qs, kb, vb)
+    _attn_check(qk, qk[:, heads * dp:], vt, ref, ref_lse, 6e-3, dict(B=B, heads=heads, Nq=N, Nk=N, d=d,
+                ldq=2 * heads * dp, ldk=2 * heads * dp, ldvt=ldvt, kv_stride=N), "fused [Q|K]")
 
 
 def test_cross_attention_padded_kv_stride():
     """Cached-context layout: 77 keys stored with a sample stride of 80 rows (K) / columns (V^T)."""
-    from adaprompt_b200 import ops
     B, N, d, Nk, pad = 3, 256, 80, 77, 80
     heads, C = 8, 640
     q = _rand(B, N, heads, d, seed=21)
@@ -249,13 +321,9 @@ def test_cross_attention_padded_kv_stride():
     kbuf[:, :Nk] = kb.reshape(B, Nk, C)
     vt = torch.zeros(C, B, pad, device=DEV, dtype=torch.bfloat16)
     vt[:, :, :Nk] = vb.permute(2, 3, 0, 1).reshape(C, B, Nk)
-    out = torch.empty(B, N, C, device=DEV, dtype=torch.bfloat16)
-    ops.attention(qs.reshape(B * N, C).contiguous(), kbuf, vt, out, B=B, heads=heads, Nq=N, Nk=Nk, d=d, ldq=C, ldk=C,
-                  ldvt=B * pad, kv_stride=pad)
-    s = torch.einsum("bihd,bjhd->bhij", qs.float(), kb.float())
-    p = torch.softmax(s * math.log(2.0), dim=-1)
-    ref = torch.einsum("bhij,bjhd->bihd", p, vb.float()).reshape(B, N, C)
-    assert _rel(out, ref) < 6e-3
+    ref, ref_lse = _attn_ref(qs, kb, vb)
+    _attn_check(qs.reshape(B * N, C).contiguous(), kbuf, vt, ref, ref_lse, 6e-3, dict(B=B, heads=heads, Nq=N, Nk=Nk,
+                d=d, ldq=C, ldk=C, ldvt=B * pad, kv_stride=pad), "padded kv_stride")
 
 
 def test_attention_rejects_unaligned_sample_stride():
@@ -269,15 +337,222 @@ def test_attention_rejects_unaligned_sample_stride():
 
 
 def test_self_attention_key_mask():
-    assert _attn_case(2, 1024, 1024, 80, seed=7, mask=True) < 6e-3
+    _attn_case(2, 1024, 1024, 80, seed=7, mask=True)
 
 
 @pytest.mark.parametrize("B,N,Nk,d,mask", [(2, 2304, 77, 80, False), (1, 9216, 77, 40, False), (3, 300, 77, 40, True),
                                            (2, 1024, 128, 80, True), (3, 512, 24, 40, False), (16, 4096, 77, 40, False),
-                                           (5, 384, 100, 80, False)])
+                                           (5, 384, 100, 80, False),
+                                           # 16-key chunks NCH = 1, 1, 2, 3, 4, 6 at both head dims
+                                           (2, 300, 1, 40, False), (2, 256, 1, 80, True), (2, 300, 16, 40, True),
+                                           (2, 384, 16, 80, False), (2, 300, 17, 40, False), (2, 256, 17, 80, True),
+                                           (2, 300, 40, 40, True), (2, 640, 40, 80, False), (2, 256, 64, 40, False),
+                                           (2, 300, 64, 80, True), (2, 300, 96, 40, True), (2, 256, 96, 80, False),
+                                           (1, 256, 128, 40, False)])     # smallest query count that takes xattn
 def test_short_context_attention(B, N, Nk, d, mask):
     """xattn.cu: K / V resident per (sample, head), ragged query tiles, key masks, every key-count class."""
-    assert _attn_case(B, N, Nk, d, seed=31, mask=mask, cross=True) < 6e-3
+    _attn_case(B, N, Nk, d, seed=31, mask=mask, cross=True)
+
+
+# (B, Nq, Nk, d, mask, cross) -> the kernel af_attention_bf16 picks (attention.cu: attention_impl)
+ATTN_MATRIX = [
+    pytest.param(2, 1000, 1000, 40, True, False, id="tile40m-1000-mask"),
+    pytest.param(1, 4096, 4096, 40, True, False, id="tile40m-4096-mask"),
+    pytest.param(2, 300, 200, 40, False, True, id="tile40m-300x200-cross"),
+    pytest.param(1, 256, 129, 40, False, False, id="tile40m-boundary-129"),
+    pytest.param(2, 1000, 1000, 80, True, False, id="tile80m-1000-mask"),
+    pytest.param(3, 600, 300, 80, True, True, id="tile80m-600x300-mask-cross"),
+    pytest.param(1, 256, 129, 80, False, False, id="tile80m-boundary-129"),
+    pytest.param(2, 300, 1024, 40, False, False, id="tile40-300x1024"),
+    pytest.param(2, 200, 1024, 80, False, False, id="tile80-200x1024"),
+    pytest.param(1, 255, 128, 40, False, False, id="generic40-boundary-255"),
+    pytest.param(3, 200, 77, 40, True, True, id="generic40-200x77-mask"),
+    pytest.param(2, 144, 77, 80, False, True, id="generic80-144x77"),
+    pytest.param(2, 100, 100, 80, True, True, id="generic80-100-mask-cross"),
+    pytest.param(2, 64, 64, 160, True, False, id="generic160-64-mask"),
+    pytest.param(3, 96, 77, 160, True, True, id="generic160-96x77-mask"),
+]
+
+
+@pytest.mark.parametrize("B,Nq,Nk,d,mask,cross", ATTN_MATRIX)
+def test_attention_dispatch_matrix(B, Nq, Nk, d, mask, cross):
+    """Every kernel family and instantiation behind af_attention_bf16: key masks, ragged key and query tails, Nq != Nk,
+    and the shapes on either side of each dispatch threshold."""
+    _attn_case(B, Nq, Nk, d, seed=41, mask=mask, cross=cross)
+
+
+@pytest.mark.parametrize("B,Nq,Nk,d,mask,cross", [
+    pytest.param(2, 1000, 1000, 40, True, False, id="tile40m-mask"),
+    pytest.param(3, 296, 296, 40, False, False, id="tile40m-ragged"),
+    pytest.param(2, 300, 200, 40, True, True, id="tile40m-mask-cross"),
+    pytest.param(2, 1000, 1000, 80, True, False, id="tile80m-mask"),
+    pytest.param(3, 600, 300, 80, True, True, id="tile80m-mask-cross"),
+    pytest.param(2, 144, 144, 80, False, False, id="tile80m-ragged"),
+    pytest.param(3, 200, 77, 40, True, True, id="generic40-mask-cross"),
+    pytest.param(2, 100, 100, 80, True, True, id="generic80-mask-cross"),
+    pytest.param(3, 96, 77, 160, True, True, id="generic160-mask-cross"),
+    pytest.param(2, 300, 77, 40, True, True, id="xattn40-mask-cross"),
+    pytest.param(2, 256, 17, 80, True, True, id="xattn80-mask-cross"),
+])
+def test_attention_masked_keys_carry_no_weight(B, Nq, Nk, d, mask, cross):
+    """Masked keys, keys past Nk and V^T columns past the last sample hold +-2^127 in V^T (and masked keys a K scaled by
+    2^10): any nonzero weight on them shows up as a wrong output row."""
+    _attn_case(B, Nq, Nk, d, seed=51, mask=mask, cross=cross, poison=True)
+
+
+@pytest.mark.parametrize("B,Nq,Nk,d,cross,first,factor", [
+    (2, 1000, 1000, 40, False, 640, 40.0),      # masked tile kernel: per-block guard and lazy reference
+    (2, 1000, 1000, 80, False, 512, 30.0),
+    (2, 100, 100, 80, True, 64, 30.0),          # generic kernel
+])
+def test_masked_attention_large_scores_late_in_the_key_loop(B, Nq, Nk, d, cross, first, factor):
+    _attn_case(B, Nq, Nk, d, seed=13, mask=True, cross=cross, boost=(first, factor), tol=8e-3)
+
+
+@pytest.mark.parametrize("B,Nq,Nk,d,cross,empty", [
+    pytest.param(2, 300, 77, 40, True, 1, id="xattn40"),
+    pytest.param(3, 1000, 1000, 40, False, 1, id="tile40m"),
+    pytest.param(2, 1000, 1000, 80, False, 0, id="tile80m"),
+    pytest.param(3, 200, 77, 40, True, 2, id="generic40"),
+    pytest.param(2, 100, 100, 80, True, 1, id="generic80"),
+    pytest.param(2, 64, 64, 160, False, 0, id="generic160"),
+])
+def test_attention_fully_masked_sample(B, Nq, Nk, d, cross, empty):
+    """A sample whose key mask keeps no key: the reference's -finfo.max fill makes its softmax uniform, so each of its
+    rows is the mean of V over its Nk keys and its lse is +inf; the other samples (partial masks) are unaffected."""
+    _attn_case(B, Nq, Nk, d, seed=61, mask=True, cross=cross, empty=empty, poison=True)
+
+
+def test_attention_dispatch_runs_every_kernel():
+    """Each case of the dispatch matrix runs the kernel it is meant to: a moved threshold cannot silently leave an
+    instantiation untested."""
+    cases = [((2, 300, nk, d), dict(cross=True)) for d in (40, 80) for nk in (1, 17, 40, 64, 96)]
+    cases += [((1, 256, 256, 40), {}), ((1, 256, 129, 40), {}), ((1, 256, 256, 80), {}), ((1, 256, 129, 80), {}),
+              ((1, 255, 128, 40), {}), ((2, 144, 77, 80), dict(cross=True)), ((2, 64, 64, 160), dict(mask=True))]
+    want = [f"xattn_kernel<{d},{n}>" for d in (40, 80) for n in (1, 2, 3, 4, 6)]
+    want += ["attention_tile_kernel<40,3,false,false>", "attention_tile_kernel<40,0,true,false>",
+             "attention_tile_kernel<80,0,false,false>", "attention_tile_kernel<80,0,true,false>",
+             "attention_kernel<40>", "attention_kernel<80>", "attention_kernel<160>", "attention_empty_mask_kernel"]
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        for shape, kw in cases:
+            _attn_case(*shape, seed=71, **kw)
+        torch.cuda.synchronize()
+    names = {e.key.replace(" ", "") for e in prof.key_averages()}
+    missing = [w for w in want if not any(w in n for n in names)]
+    assert not missing, (missing, sorted(n for n in names if "attention" in n or "xattn" in n))
+
+
+@pytest.mark.parametrize("d,N", [(40, 1000), (160, 64)])
+def test_cross_attention_module_fully_masked_sample(d, N):
+    """CrossAttention.forward(x, mask=...) as self-attention, sample 0 masked out entirely, sample 1 partially, against
+    oracle.unet_oracle.cross_attention on the same weights."""
+    from adaprompt_b200.attention import CrossAttention
+    from oracle.unet_oracle import cross_attention
+    C = 8 * d
+    torch.manual_seed(3)
+    attn = CrossAttention(C, heads=8, dim_head=d).to(DEV)
+    x = _rand(2, N, C, seed=81)
+    g = torch.Generator().manual_seed(82)
+    mask = torch.rand(2, N, generator=g) > 0.5
+    mask[0] = False
+    with torch.no_grad():
+        out = attn(x, mask=mask.to(DEV))
+    sd = {f"a.{k}": v.detach().float().cpu() for k, v in attn.state_dict().items()}
+    ref = cross_attention(sd, "a", x.cpu(), mask=mask)
+    err = _rel(out.cpu(), ref)
+    print(f"\nCrossAttention d={d} N={N} with a fully masked sample: rel {err:.2e}")
+    assert err < 1e-2
+
+
+# ------------------------------------------------------------------------------------------------ materialised scores
+def _straddling_cols(M, nk):
+    """M distinct key columns below nk, starting with those on either side of the 31|32 and 63|64 boundaries (the
+    32-key lane groups of xattn_explicit)."""
+    cand = [c for c in [31, 32, 63, 64] + list(range(nk)) if c < nk]
+    return list(dict.fromkeys(cand))[:M]
+
+
+@pytest.mark.parametrize("ks", [2, 3, 4])
+@pytest.mark.parametrize("Hf,Wf", [(8, 8), (6, 10), (1, 7)])
+def test_conv_attn_scores(ks, Hf, Wf):
+    """ops.conv_attn_scores against oracle.unet_oracle.conv_attn_columns: sample 0 without the subject (cols = -1),
+    sample 1 with columns across the 31|32 and 63|64 boundaries, sample 2 with random columns.  The oracle's restatement
+    is pinned to the upstream replace_rows_by_conv_attn by a golden only at ks = 3; at ks = 2 and 4 (even kernels, uneven
+    padding) it is checked against the restatement alone."""
+    from adaprompt_b200 import ops
+    from oracle.unet_oracle import conv_attn_columns
+    B, heads, nk, M = 3, 8, 77, ks * ks
+    N = Hf * Wf
+    score = _rand(B, heads, N, nk, seed=91, scale=3.0)
+    g = torch.Generator().manual_seed(92)
+    cols = torch.stack([torch.full((M,), -1, dtype=torch.int64), torch.tensor(_straddling_cols(M, nk)),
+                        torch.randperm(nk, generator=g)[:M]])
+    ov = ops.conv_attn_scores(score, cols.to(torch.int32).to(DEV), B=B, heads=heads, Hf=Hf, Wf=Wf, nk=nk, ks=ks)
+    ref = torch.zeros(B, heads, N, M, dtype=torch.float64)
+    sc = score.double().cpu()
+    for b in (1, 2):
+        ref[b] = conv_attn_columns(sc[b], cols[b], (Hf, Wf), ks).permute(1, 2, 0)
+    assert torch.equal(ov[0], torch.zeros_like(ov[0]))
+    assert _rel(ov.cpu().double(), ref) < 1e-5
+
+
+def _xattn_explicit_params():
+    ps = []
+    for d in (40, 80, 160):
+        for nk in (1, 33, 77, 96):
+            for N in (1, 64, 100):
+                for ov in (False, True) if nk >= 18 else (False,):
+                    ps.append(pytest.param(d, nk, N, ov, id=f"d{d}-nk{nk}-N{N}{'-override' if ov else ''}"))
+    return ps
+
+
+@pytest.mark.parametrize("d,nk,N,override", _xattn_explicit_params())
+def test_xattn_explicit(d, nk, N, override):
+    """ops.xattn_explicit against a float64 restatement of oracle.unet_oracle.cross_attention (sim, column replacement,
+    softmax, attn.v, q * sqrt(scale)), two samples with the key stride padded to 8.  override: two subjects of ks = 3
+    (n_ov = 18 columns) replace score columns, sample 0 has only the first, sample 1 only the second.  nk = 96 at d = 160 is
+    the largest shared-memory configuration."""
+    from adaprompt_b200 import ops
+    B, heads = 2, 8
+    C = heads * d
+    dp = 48 if d == 40 else d
+    kv_stride = (nk + 7) // 8 * 8
+    scale = d ** -0.5
+    qs = (_rand(B, N, heads, d, seed=101) * (scale * math.log2(math.e))).to(torch.bfloat16)
+    kb = _rand(B, nk, heads, d, seed=102).to(torch.bfloat16)
+    vb = _rand(B, nk, heads, d, seed=103).to(torch.bfloat16)
+    qbuf = torch.zeros(B * N, heads, dp, device=DEV, dtype=torch.bfloat16)
+    qbuf[:, :, :d] = qs.reshape(B * N, heads, d)
+    kbuf = torch.zeros(B, kv_stride, heads, dp, device=DEV, dtype=torch.bfloat16)
+    kbuf[:, :nk, :, :d] = kb
+    kbuf[:, nk:, :, :d] = POISON           # padding keys are never read
+    ldvt = max(64, B * kv_stride)
+    vt = torch.full((C, ldvt), POISON, device=DEV, dtype=torch.bfloat16)
+    vt[:, :B * kv_stride].view(C, B, kv_stride)[:, :, :nk] = vb.permute(2, 3, 0, 1).reshape(C, B, nk)
+    ov = cols = None
+    if override:
+        M = 9
+        ov = _rand(B, heads, N, 2 * M, seed=104, scale=2.0)
+        c1, c2 = _straddling_cols(M, nk), list(range(nk - M, nk))[::-1]
+        cols = torch.tensor([c1 + [-1] * M, [-1] * M + c2], dtype=torch.int32, device=DEV)
+    r = ops.xattn_explicit(qbuf.reshape(B * N, heads * dp), kbuf.reshape(B * kv_stride, heads * dp), vt, B=B, heads=heads,
+                           N=N, nk=nk, d=d, ldq=heads * dp, ldk=heads * dp, ldvt=ldvt, kv_stride=kv_stride, override=ov,
+                           ov_cols=cols, want_out=True, want_scores=True, want_attn=True, want_q=True)
+    # reference (oracle cross_attention :220-239): q = qs / (scale log2 e) is the unscaled query
+    q = qs.double().permute(0, 2, 1, 3) / (scale * math.log2(math.e))
+    sim = torch.einsum("bhid,bjhd->bhij", q, kb.double()) * scale
+    if override:
+        for b in range(B):
+            for m in range(2 * M):
+                c = int(cols[b, m])
+                if c >= 0:
+                    sim[b, :, :, c] = ov[b, :, :, m].double()
+    attn = sim.softmax(dim=-1)
+    out = torch.einsum("bhij,bjhd->bihd", attn, vb.double()).reshape(B * N, C)
+    errs = {"attnscore": _rel(r["attnscore"].double(), sim), "attn": _rel(r["attn"].double(), attn),
+            "q": _rel(r["q"].double(), q * scale ** 0.5), "out": _rel(r["out"].double(), out)}
+    print(f"\nxattn_explicit d={d} nk={nk} N={N} override={override}: {errs}")
+    assert errs["attnscore"] < 1e-5 and errs["attn"] < 1e-5 and errs["q"] < 1e-5 and errs["out"] < 6e-3, errs
 
 
 # ------------------------------------------------------------------------------------------------ norms
