@@ -263,7 +263,9 @@ class CLIPTextModelWrapper(nn.Module):
         return _Output(last_hidden_state=last, pooler_output=pooled, hidden_states=None, attentions=None)
 
     def extend_clip_attention_MKV_multiplier(self, begin_layer_idx=-1, end_layer_idx=-1, multiplier=2, noise_std=0.1):
-        """arc2face_models.py:285-302."""
+        """arc2face_models.py:285-302.  Multipliers compound across calls.  The forward runs any total multiplier up to 4,
+        but the training backward (attention_small_bwd_kernel) holds the scores of a 77-token layer in shared memory and
+        refuses a total above 2 with ValueError."""
         n = 0
         for layer_idx, layer in enumerate(self.text_model.encoder.layers):
             if begin_layer_idx >= 0 and layer_idx < begin_layer_idx:
