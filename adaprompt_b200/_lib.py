@@ -67,6 +67,8 @@ SIGNATURES = {
     "af_attention_bf16": (c_int, [c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_longlong, c_int, c_void_p,
                                   c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "af_conv3x3_gn_slots": (c_int, [c_int, c_int]),
+    "af_conv3x3_down01_bf16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, POINTER(AfEpilogue),
+                                       c_int, c_void_p]),
     "af_xattn_explicit": (c_int, [c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_longlong, c_int, c_void_p, c_void_p,
                                   c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "af_conv_attn_scores": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
@@ -126,6 +128,8 @@ SIGNATURES = {
     "af_transpose_to_bf16": (c_int, [c_void_p, c_int, c_int, c_int, c_longlong, c_void_p, c_void_p]),
     "af_channel_mix4": (c_int, [c_void_p, c_void_p, c_void_p, c_float, c_int, c_int, c_int, c_longlong, c_void_p, c_void_p]),
     "af_softmax_rows": (c_int, [c_void_p, c_longlong, c_longlong, c_int, c_float, c_void_p, c_longlong, c_void_p]),
+    "af_vae_posterior": (c_int, [c_void_p, c_int, c_longlong, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                 c_void_p]),
     "af_prodigy_moments": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_float,
                                    c_float, c_float, c_float, c_float, c_float, c_void_p, c_void_p]),
     "af_prodigy_apply": (c_int, [c_void_p, c_void_p, c_void_p, c_longlong, c_float, c_float, c_float, c_void_p]),
@@ -178,7 +182,7 @@ KERNELS_PER_CALL = {
     "af_attention_bf16_lse": 1, "af_attention_bwd_bf16": 2, "af_xattn_explicit": 1, "af_conv_attn_scores": 1, "af_bgemm_bf16": 1, "af_groupnorm_bwd": 3, "af_layernorm_bwd": 1, "af_geglu_fwd": 1,
     "af_geglu_bwd": 1, "af_quick_gelu": 1, "af_rowdot_heads": 1, "af_attention_small_bwd": 1, "af_conv_out_dgrad": 1,
     "af_sumpool2x2": 1, "af_zero_insert2x": 1, "af_transpose_to_bf16": 1, "af_prodigy_moments": 1, "af_prodigy_apply": 1,
-    "af_softmax_rows": 1, "af_channel_mix4": 1,
+    "af_softmax_rows": 1, "af_channel_mix4": 1, "af_conv3x3_down01_bf16": 1, "af_vae_posterior": 1,
 }
 
 

@@ -7,7 +7,7 @@ weights are not available offline, so this mirror keeps the constructor and meth
 B200-native components instead: adaprompt_b200.clip_text (text encoder with the z_0..z_15 placeholder rows),
 adaprompt_b200.subj_basis_generator, adaprompt_b200.unet.UNetModel and adaprompt_b200.ddim.DDIMSampler.  Components are
 injected through keyword arguments (`unet`, `text_encoder`, `tokenizer`, `subj_basis_generator`,
-`arc2face_text_encoder`, `vae_decoder`); loading them from `base_model_path` / `adaface_ckpt_path` needs files that
+`arc2face_text_encoder`, `vae_decoder`, and for pipeline_name="img2img" `vae_encoder`); loading them from `base_model_path` / `adaface_ckpt_path` needs files that
 do not exist here and raises a clear error.  End-to-end numerics of the reference wrapper are "parity unpinned"
 (diffusers absent, SURVEY.md section 8(c)); its SubjBasisGenerator stage is covered by tests/test_text_gpu.py.
 """
@@ -21,7 +21,7 @@ import torch.nn.functional as F
 from torch import nn
 
 from .adaface_util import arc2face_forward_face_embs
-from .ddim import DDIMSampler
+from .ddim import DDIMSampler, img2img_t_enc
 from .ldm_lite import LatentDiffusionLite
 
 DEFAULT_NEGATIVE_PROMPT = (
@@ -35,7 +35,7 @@ class AdaFaceWrapper(nn.Module):
     def __init__(self, pipeline_name, base_model_path, adaface_ckpt_path, device, subject_string="z", num_vectors=16,
                  num_inference_steps=50, negative_prompt=None, use_840k_vae=False, use_ds_text_encoder=False,
                  is_training=False, *, unet=None, text_encoder=None, tokenizer=None, subj_basis_generator=None,
-                 arc2face_text_encoder=None, vae_decoder=None):
+                 arc2face_text_encoder=None, vae_decoder=None, vae_encoder=None):
         super().__init__()
         self.pipeline_name = pipeline_name
         self.base_model_path = base_model_path
@@ -49,7 +49,7 @@ class AdaFaceWrapper(nn.Module):
         self.is_training = is_training
         self._injected = dict(unet=unet, text_encoder=text_encoder, tokenizer=tokenizer,
                               subj_basis_generator=subj_basis_generator, arc2face_text_encoder=arc2face_text_encoder,
-                              vae_decoder=vae_decoder)
+                              vae_decoder=vae_decoder, vae_encoder=vae_encoder)
         self.initialize_pipeline()
         self.extend_tokenizer_and_text_encoder()
         self.negative_prompt = DEFAULT_NEGATIVE_PROMPT if negative_prompt is None else negative_prompt
@@ -82,6 +82,7 @@ class AdaFaceWrapper(nn.Module):
         self.text_encoder = inj["text_encoder"].to(self.device)      # clip_text.CLIPTextModelWrapper
         self.tokenizer = inj["tokenizer"]
         self.vae_decoder = inj["vae_decoder"]
+        self.vae_encoder = inj["vae_encoder"]          # vae.AutoencoderKL(with_encoder=True): img2img from RGB images
         if self.pipeline_name is not None:
             if inj["unet"] is None:
                 raise FileNotFoundError("unet must be injected (adaprompt_b200.unet.UNetModel with SD-1.5 weights)")
@@ -174,8 +175,14 @@ class AdaFaceWrapper(nn.Module):
                 generator=None, verbose=False):
         if self.sampler is None:
             raise RuntimeError("pipeline_name=None: the wrapper was built without a UNet")
+        t_enc = None
         if self.pipeline_name == "img2img":
-            raise NotImplementedError("img2img needs the VAE encoder (row N1)")
+            # host-side checks before any device work (a t_enc out of range would fault inside stochastic_encode)
+            t_enc = img2img_t_enc(ref_img_strength, self.num_inference_steps)
+            if noise.dim() != 4 or noise.shape[1] not in (3, 4):
+                raise ValueError("img2img: `noise` must be an NCHW image in [-1, 1] (3 channels) or latents (4 channels)")
+            if noise.shape[1] == 3 and self.vae_encoder is None:
+                raise RuntimeError("img2img from an RGB image needs vae_encoder (vae.AutoencoderKL(with_encoder=True))")
         pe, ne = self.encode_prompt(prompt, negative_prompt, device=self.device, verbose=verbose)
         b = out_image_count
         # the LDM UNet takes one context per cross-attention layer: the same prompt embedding for all 16
@@ -185,10 +192,30 @@ class AdaFaceWrapper(nn.Module):
                  "is_training": False}
         noise = noise.to(self.device).float()
         g = float(guidance_scale)
-        samples, _ = self.sampler.sample(self.num_inference_steps, b, list(noise.shape[1:]),
-                                         conditioning=(c, [prompt] * b, dict(extra)),
-                                         unconditional_conditioning=(uc, [negative_prompt or self.negative_prompt] * b, dict(extra)),
-                                         guidance_scale=(g, g), eta=0.0, x_T=noise, verbose=False)
+        if t_enc is not None:
+            samples = self._img2img(noise, b, c, uc, [prompt] * b, [negative_prompt or self.negative_prompt] * b, extra, g,
+                                    t_enc)
+        else:
+            samples, _ = self.sampler.sample(self.num_inference_steps, b, list(noise.shape[1:]),
+                                             conditioning=(c, [prompt] * b, dict(extra)),
+                                             unconditional_conditioning=(uc, [negative_prompt or self.negative_prompt] * b,
+                                                                         dict(extra)),
+                                             guidance_scale=(g, g), eta=0.0, x_T=noise, verbose=False)
         if self.vae_decoder is None:
             return samples          # latents; the VAE decoder is SURVEY.md section 8(f) row N1 ("next")
         return self.vae_decoder(samples / self.ldm.scale_factor)
+
+    def _img2img(self, init, b, c, uc, prompts, neg_prompts, extra, g, t_enc):
+        """SD scripts/img2img.py on the LDM sampler: encode (3-channel images; 4 channels are latents already, as in
+        diffusers' img2img pipeline), stochastic_encode to step t_enc, then DDIMSampler.decode with CFG."""
+        if init.shape[1] == 3:
+            from .vae import encode_first_stage
+            init = self.ldm.get_first_stage_encoding(encode_first_stage(self.vae_encoder, init))
+        if init.shape[0] != b:
+            if init.shape[0] != 1:
+                raise ValueError(f"img2img: {init.shape[0]} init images for out_image_count {b}")
+            init = init.repeat(b, 1, 1, 1)
+        self.sampler.make_schedule(ddim_num_steps=self.num_inference_steps, ddim_eta=0.0, verbose=False)
+        z_enc = self.sampler.stochastic_encode(init, torch.full((b,), t_enc, dtype=torch.long, device=init.device))
+        return self.sampler.decode(z_enc, (c, prompts, dict(extra)), t_enc, guidance_scale=g,
+                                   unconditional_conditioning=(uc, neg_prompts, dict(extra)))

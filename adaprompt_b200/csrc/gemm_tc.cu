@@ -10,6 +10,8 @@
 //     is TMA out-of-bounds fill - no im2col buffer exists anywhere.
 //   * conv3x3 stride 2 (Downsample, openaimodel.py:155): the input is viewed as
 //     [B, H/2, 2, W/2, 2*C] so every tap is a unit-stride 5-D box.
+//   * conv3x3 stride 2 after F.pad(x, (0,1,0,1)) (the VAE encoder's Downsample, model.py:61-79): the same 5-D view with
+//     input row 2*oh + ky; its own instantiations (DOWN01) so the other modes' producer loops stay as they are.
 //   * the skip-connection concat (openaimodel.py:1019) is never materialised: the K loop walks two
 //     tensor maps (A0 then A1).
 //
@@ -42,7 +44,7 @@ struct GemmParams {
   int num_kb;          // K blocks (64 wide) in total
   int cpb;             // K blocks per tap (== num_kb for linear)
   int kb_split;        // K blocks per tap served by A0 (rest by A1)
-  int amode;           // 0 linear, 1 conv3x3 s1, 2 conv3x3 s2
+  int amode;           // 0 linear, 1 conv3x3 s1, 2 conv3x3 s2, 3 conv3x3 s2 after F.pad(0,1,0,1)
   int B, H, W;         // conv: output pixel grid
   int C0;              // conv s2: channels of the (single) source
   int bw, bh, nb;      // conv: tile box (bw*bh*nb == 128)
@@ -126,7 +128,9 @@ __device__ __forceinline__ float gelu_tanh(float x) {
 // QuickGELU of the CLIP text MLP (transformers QuickGELUActivation): x * sigmoid(1.702 x)
 __device__ __forceinline__ float quick_gelu(float x) { return __fdividef(x, 1.0f + __expf(-1.702f * x)); }
 
-template <int BN, bool GEGLU, int SLOTS, bool CTA2>
+// DOWN01: the producer runs the amode-3 tap walk only (af_conv3x3_down01_bf16; convolution layout, one epilogue slot
+// per warp); otherwise it selects mode 0 / 1 / 2 from p.amode.
+template <int BN, bool GEGLU, int SLOTS, bool CTA2, bool DOWN01>
 __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_constant__ GemmParams p) {
   using Cfg = GemmCfg<BN, GEGLU, SLOTS, CTA2>;
   constexpr int kStages = Cfg::kStages;
@@ -271,10 +275,18 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
               } else if constexpr (AM == 1) {
                 if constexpr (CTA2) tma_load_4d_pair(sa, tmA, &full_bar[stage], kc, cw + kx - 1, ch + ky - 1, cn);
                 else tma_load_4d(sa, tmA, &full_bar[stage], kc, cw + kx - 1, ch + ky - 1, cn);
-              } else {
+              } else if constexpr (AM == 2) {
                 // stride 2: input row 2*oh + ky - 1  ->  (coarse row oh + dh, parity ph)
                 const int ph = (ky == 1) ? 0 : 1, dh = (ky == 0) ? -1 : 0;
                 const int pw = (kx == 1) ? 0 : 1, dw = (kx == 0) ? -1 : 0;
+                if constexpr (CTA2) tma_load_5d_pair(sa, tmA, &full_bar[stage], pw * p.C0 + kc, cw + dw, ph, ch + dh, cn);
+                else tma_load_5d(sa, tmA, &full_bar[stage], pw * p.C0 + kc, cw + dw, ph, ch + dh, cn);
+              } else {
+                // stride 2 after F.pad(0,1,0,1): input row 2*oh + ky  ->  (coarse row oh + (ky >> 1), parity ky & 1).
+                // ky == 2 on the last output row reads coarse row H/2: out of bounds, TMA fills zeros = the bottom pad
+                // (columns likewise: the right pad).
+                const int ph = ky & 1, dh = ky >> 1;
+                const int pw = kx & 1, dw = kx >> 1;
                 if constexpr (CTA2) tma_load_5d_pair(sa, tmA, &full_bar[stage], pw * p.C0 + kc, cw + dw, ph, ch + dh, cn);
                 else tma_load_5d(sa, tmA, &full_bar[stage], pw * p.C0 + kc, cw + dw, ph, ch + dh, cn);
               }
@@ -295,7 +307,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
           }
         };
         if (loads_a) {
-          if (p.amode == 0) a_loop(std::integral_constant<int, 0>{});
+          if constexpr (DOWN01) a_loop(std::integral_constant<int, 3>{});
+          else if (p.amode == 0) a_loop(std::integral_constant<int, 0>{});
           else if (p.amode == 1) a_loop(std::integral_constant<int, 1>{});
           else a_loop(std::integral_constant<int, 2>{});
         } else {
@@ -807,13 +820,13 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
 // No process-global switches: the tile schedule (af_epilogue.pair_mode) and the timeline probe (af_epilogue.trace) are
 // per-call options.
 
-template <int BN, bool GEGLU, int SLOTS, bool CTA2>
+template <int BN, bool GEGLU, int SLOTS, bool CTA2, bool DOWN01 = false>
 static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
   using Cfg = GemmCfg<BN, GEGLU, SLOTS, CTA2>;
+  void (*kernel)(GemmParams) = gemm_tc_kernel<BN, GEGLU, SLOTS, CTA2, DOWN01>;
   static bool configured = false;
   if (!configured) {
-    AF_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, GEGLU, SLOTS, CTA2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 Cfg::kSmemBytes));
+    AF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     configured = true;
   }
   if constexpr (CTA2) {
@@ -832,10 +845,10 @@ static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    AF_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, GEGLU, SLOTS, CTA2>, p));
+    AF_CUDA(cudaLaunchKernelEx(&cfg, kernel, p));
   } else {
     const int grid = p.num_units < num_sms() ? p.num_units : num_sms();
-    gemm_tc_kernel<BN, GEGLU, SLOTS, CTA2><<<grid, kGemmThreads, Cfg::kSmemBytes, stream>>>(p);
+    kernel<<<grid, kGemmThreads, Cfg::kSmemBytes, stream>>>(p);
   }
   AF_LAUNCH_CHECK("gemm_tc_kernel");
   return 0;
@@ -860,9 +873,9 @@ static bool want_pair(int pair_mode, int m_tiles, int n_tiles, int bn, int amode
   return false;
 }
 
-template <int BN, bool GEGLU, int SLOTS>
+template <int BN, bool GEGLU, int SLOTS, bool DOWN01 = false>
 static int launch_gemm_mode(const GemmParams& p, bool pair, cudaStream_t stream) {
-  return pair ? launch_gemm<BN, GEGLU, SLOTS, true>(p, stream) : launch_gemm<BN, GEGLU, SLOTS, false>(p, stream);
+  return pair ? launch_gemm<BN, GEGLU, SLOTS, true, DOWN01>(p, stream) : launch_gemm<BN, GEGLU, SLOTS, false, DOWN01>(p, stream);
 }
 
 // Split-K of the last partial wave (kernel comment "work units").  Cost model in units of one K block of main-loop
@@ -911,6 +924,15 @@ static void plan_split(GemmParams& p, int bn, bool pair, const af_epilogue* ep) 
 
 static int dispatch_gemm(int bn, const GemmParams& p, bool pair, cudaStream_t stream) {
   if (p.geglu) return launch_gemm_mode<256, true, 2>(p, pair, stream);
+  if (p.amode == 3) {
+    switch (bn) {
+      case 64: return launch_gemm_mode<64, false, 1, true>(p, pair, stream);
+      case 128: return launch_gemm_mode<128, false, 1, true>(p, pair, stream);
+      case 160: return launch_gemm_mode<160, false, 1, true>(p, pair, stream);
+      case 256: return launch_gemm_mode<256, false, 1, true>(p, pair, stream);
+      default: set_error("unsupported BN %d (64/128/160/256)", bn); return -1;
+    }
+  }
   // epilogue slots per warp: 3 (two residual chunks in flight) for the memory-bound linear GEMMs with a residual,
   // 1 for the K-deep convolutions (their epilogue has slack; the shared memory goes to the operand ring), else 2
   const int slots = p.amode != 0 ? 1 : (p.residual != nullptr ? 3 : 2);
@@ -1090,15 +1112,11 @@ extern "C" int af_conv3x3_gn_slots(int Ho, int Wo) {
   return ((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh) * (bw * bh / 32);
 }
 
-extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, const void* Wt, int B, int H, int W,
-                               int Cout, int stride, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
-  AF_CHECK_ARG(X0 && Wt && ep, "af_conv3x3_bf16: null pointer");
-  AF_CHECK_ARG(stride == 1 || stride == 2, "af_conv3x3_bf16: stride %d", stride);
-  AF_CHECK_ARG(C0 > 0 && C0 % 64 == 0 && C1 >= 0 && C1 % 64 == 0, "af_conv3x3_bf16: C0=%d C1=%d must be multiples of 64",
-               C0, C1);
-  AF_CHECK_ARG(Cout % 8 == 0, "af_conv3x3_bf16: Cout=%d must be a multiple of 8", Cout);
-  AF_CHECK_ARG(stride == 1 || (C1 == 0 && H % 2 == 0 && W % 2 == 0), "af_conv3x3_bf16: stride 2 needs single source, even H/W");
-  AF_CHECK_ARG(!ep->geglu, "af_conv3x3_bf16: geglu epilogue unsupported");
+// amode 1: stride 1, pad 1 (two sources); 2: stride 2, pad 1; 3: stride 2 after F.pad(0,1,0,1).  The entry points have
+// checked the arguments their mode needs.
+static int conv3x3_launch(const char* who, const void* X0, int C0, const void* X1, int C1, const void* Wt, int B, int H,
+                          int W, int Cout, int amode, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
+  const int stride = amode == 1 ? 1 : 2;
   GemmParams p;
   memset(&p, 0, sizeof(p));
   p.trace = ep->trace;
@@ -1140,7 +1158,7 @@ extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, c
     int rc = make_tmap_bf16(&p.tmA0, X0, 5, dims, str, box);
     if (rc) return rc;
     p.tmA1 = p.tmA0;
-    p.amode = 2;
+    p.amode = amode;
   }
   {
     const uint64_t K = 9ull * Cin;
@@ -1162,7 +1180,7 @@ extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, c
   if (p.rowbias && ep->rows_per_group <= 0) p.rows_per_group = Ho * Wo;
   if (p.gn_stats) {
     p.gn_slots = af_conv3x3_gn_slots(Ho, Wo);
-    AF_CHECK_ARG(p.gn_slots > 0, "af_conv3x3_bf16: gn_stats unsupported for %dx%d outputs (fewer than 32 pixels per tile row group)", Ho, Wo);
+    AF_CHECK_ARG(p.gn_slots > 0, "%s: gn_stats unsupported for %dx%d outputs (fewer than 32 pixels per tile row group)", who, Ho, Wo);
   }
 #ifndef AF_GEMM_NO_WIDE
   p.wide = p.out_bf16 && p.residual == nullptr && (bn == 128 || bn == 256);
@@ -1171,6 +1189,29 @@ extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, c
   if (rc) return rc;
   plan_split(p, bn, pair, ep);
   return dispatch_gemm(bn, p, pair, stream);
+}
+
+extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, const void* Wt, int B, int H, int W,
+                               int Cout, int stride, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
+  AF_CHECK_ARG(X0 && Wt && ep, "af_conv3x3_bf16: null pointer");
+  AF_CHECK_ARG(stride == 1 || stride == 2, "af_conv3x3_bf16: stride %d", stride);
+  AF_CHECK_ARG(C0 > 0 && C0 % 64 == 0 && C1 >= 0 && C1 % 64 == 0, "af_conv3x3_bf16: C0=%d C1=%d must be multiples of 64",
+               C0, C1);
+  AF_CHECK_ARG(Cout % 8 == 0, "af_conv3x3_bf16: Cout=%d must be a multiple of 8", Cout);
+  AF_CHECK_ARG(stride == 1 || (C1 == 0 && H % 2 == 0 && W % 2 == 0), "af_conv3x3_bf16: stride 2 needs single source, even H/W");
+  AF_CHECK_ARG(!ep->geglu, "af_conv3x3_bf16: geglu epilogue unsupported");
+  return conv3x3_launch("af_conv3x3_bf16", X0, C0, X1, C1, Wt, B, H, W, Cout, stride, ep, bn_hint, stream);
+}
+
+extern "C" int af_conv3x3_down01_bf16(const void* X, int C, const void* Wt, int B, int H, int W, int Cout,
+                                      const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
+  AF_CHECK_ARG(X && Wt && ep, "af_conv3x3_down01_bf16: null pointer");
+  AF_CHECK_ARG(B > 0 && H > 0 && W > 0, "af_conv3x3_down01_bf16: bad sizes B=%d H=%d W=%d", B, H, W);
+  AF_CHECK_ARG(C > 0 && C % 64 == 0, "af_conv3x3_down01_bf16: C=%d must be a multiple of 64", C);
+  AF_CHECK_ARG(Cout > 0 && Cout % 8 == 0, "af_conv3x3_down01_bf16: Cout=%d must be a multiple of 8", Cout);
+  AF_CHECK_ARG(H % 2 == 0 && W % 2 == 0, "af_conv3x3_down01_bf16: H=%d W=%d must be even", H, W);
+  AF_CHECK_ARG(!ep->geglu, "af_conv3x3_down01_bf16: geglu epilogue unsupported");
+  return conv3x3_launch("af_conv3x3_down01_bf16", X, C, nullptr, 0, Wt, B, H, W, Cout, 3, ep, bn_hint, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

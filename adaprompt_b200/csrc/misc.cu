@@ -6,8 +6,9 @@
 namespace af {
 
 // ---------------------------------------------------------------------------------------------
-// conv_in: NCHW fp32 [B,Cin,H,W] (Cin = 4) -> NHWC fp32 [B,H,W,Cout], 3x3 pad 1, fp32 math.
-// Reference: UNetModel.input_blocks[0] = conv_nd(2, 4, 320, 3, padding=1) (openaimodel.py:527-533).
+// conv_in: NCHW fp32 [B,Cin,H,W] (Cin = 4 or 3) -> NHWC fp32 [B,H,W,Cout], 3x3 pad 1, fp32 math.
+// Reference: UNetModel.input_blocks[0] = conv_nd(2, 4, 320, 3, padding=1) (openaimodel.py:527-533), the VAE's
+// Decoder.conv_in (4 -> 512) and Encoder.conv_in (3 -> 128, model.py:436-440).
 // Block = 32 consecutive pixels of one image row; the weights live in shared memory as [tap*Cin + ci][Cout] so a
 // thread reads the four output channels it owns with one 16-byte load per tap, and the input value of a (pixel,
 // tap) is one broadcast load shared by all channel quads.  Stores are 512 B contiguous per warp (NHWC).
@@ -344,21 +345,19 @@ static inline int grid_for(size_t work_items, int threads) {
   return static_cast<int>(g);
 }
 
-extern "C" int af_conv_in(const float* x_nchw, const float* w, const float* bias, float* y_nhwc, int B, int Cin, int H,
-                          int W, int Cout, cudaStream_t stream) {
-  AF_CHECK_ARG(x_nchw && w && y_nhwc, "af_conv_in: null pointer");
-  AF_CHECK_ARG(Cin == 4, "af_conv_in: Cin=%d unsupported (4)", Cin);
-  AF_CHECK_ARG(Cout % 4 == 0 && Cout >= 32 && Cout <= 1280, "af_conv_in: Cout=%d unsupported", Cout);
+template <int CIN>
+static int launch_conv_in(const float* x_nchw, const float* w, const float* bias, float* y_nhwc, int B, int H, int W,
+                          int Cout, cudaStream_t stream) {
   const int cq = Cout / 4;
   int groups = 320 / cq;                       // pixel groups per block; must divide 32 with >= 8 pixels each
   if (groups > 4) groups = 4;
   if (groups == 3) groups = 2;
   if (groups < 1) groups = 1;
   const int threads = ((groups * cq + 31) / 32) * 32;
-  const size_t smem = (static_cast<size_t>(36) * Cout + 4 * 3 * 34) * sizeof(float);
+  const size_t smem = (static_cast<size_t>(9 * CIN) * Cout + CIN * 3 * 34) * sizeof(float);
   static size_t configured = 0;
   if (smem > configured) {
-    AF_CUDA(cudaFuncSetAttribute(conv_in_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    AF_CUDA(cudaFuncSetAttribute(conv_in_kernel<CIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     configured = smem;
   }
   // rows per block: as many as keep >= 2 blocks per SM in flight
@@ -367,9 +366,20 @@ extern "C" int af_conv_in(const float* x_nchw, const float* w, const float* bias
   if (rows < 1) rows = 1;
   if (rows > 16) rows = 16;
   dim3 grid(col_blocks, (H + rows - 1) / rows, B);
-  conv_in_kernel<4><<<grid, threads, smem, stream>>>(x_nchw, w, bias, y_nhwc, B, H, W, Cout, rows);
+  conv_in_kernel<CIN><<<grid, threads, smem, stream>>>(x_nchw, w, bias, y_nhwc, B, H, W, Cout, rows);
   AF_LAUNCH_CHECK("conv_in_kernel");
   return 0;
+}
+
+// Cin 4: the UNet's and the VAE decoder's conv_in on latents; Cin 3: the VAE encoder's conv_in on RGB images
+// (model.py:436-440).
+extern "C" int af_conv_in(const float* x_nchw, const float* w, const float* bias, float* y_nhwc, int B, int Cin, int H,
+                          int W, int Cout, cudaStream_t stream) {
+  AF_CHECK_ARG(x_nchw && w && y_nhwc, "af_conv_in: null pointer");
+  AF_CHECK_ARG(Cin == 3 || Cin == 4, "af_conv_in: Cin=%d unsupported (3 or 4)", Cin);
+  AF_CHECK_ARG(Cout % 4 == 0 && Cout >= 32 && Cout <= 1280, "af_conv_in: Cout=%d unsupported", Cout);
+  if (Cin == 3) return launch_conv_in<3>(x_nchw, w, bias, y_nhwc, B, H, W, Cout, stream);
+  return launch_conv_in<4>(x_nchw, w, bias, y_nhwc, B, H, W, Cout, stream);
 }
 
 extern "C" int af_conv_out(const void* x_nhwc_bf16, const float* w_packed, const float* bias, float* y_nchw, int B,
@@ -544,6 +554,46 @@ extern "C" int af_channel_mix4(const float* x_nchw, const float* w, const float*
   channel_mix4_kernel<<<grid_for(static_cast<size_t>(total), 256), 256, 0, stream>>>(x_nchw, w, bias, in_scale, Cin, Cout,
                                                                                      HW, total, y_nchw);
   AF_LAUNCH_CHECK("channel_mix4_kernel");
+  return 0;
+}
+
+// DiagonalGaussianDistribution (ldm/modules/distributions/distributions.py:24-44) over the encoder's moments, fused with
+// get_first_stage_encoding's scale_factor * z (ddpm.py).  Same fp32 operations in the same order as the reference's torch
+// ops: clamp, 0.5 * lv, exp (expf, not the MUFU approximation), std * noise, mean + that, scale * that; no contraction.
+namespace af {
+__global__ void __launch_bounds__(256) vae_posterior_kernel(const float* __restrict__ moments, long long HW, int zc,
+                                                            long long total, const float* __restrict__ noise,
+                                                            float out_scale, float* __restrict__ z,
+                                                            float* __restrict__ mean_out, float* __restrict__ logvar_out) {
+  for (long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * 256) {
+    const long long pix = i % HW, bc = i / HW;                 // output index i = (b * zc + c) * HW + pix
+    const int c = static_cast<int>(bc % zc);
+    const long long b = bc / zc;
+    const float* m = moments + (b * HW + pix) * (2 * zc);
+    const float mean = m[c];
+    float lv = m[zc + c];
+    if (!isnan(lv)) lv = fminf(fmaxf(lv, -30.0f), 20.0f);    // torch.clamp(logvar, -30.0, 20.0)
+    float v = mean;
+    if (noise) {
+      const float stdv = expf(__fmul_rn(0.5f, lv));           // torch.exp(0.5 * self.logvar)
+      v = __fadd_rn(mean, __fmul_rn(stdv, noise[i]));         // self.mean + self.std * noise
+    }
+    z[i] = __fmul_rn(out_scale, v);
+    if (mean_out) mean_out[i] = mean;
+    if (logvar_out) logvar_out[i] = lv;
+  }
+}
+}  // namespace af
+
+extern "C" int af_vae_posterior(const float* moments_nhwc, int B, long long HW, int zc, const float* noise_nchw,
+                                float out_scale, float* z_nchw, float* mean_nchw, float* logvar_nchw, cudaStream_t stream) {
+  AF_CHECK_ARG(moments_nhwc && z_nchw, "af_vae_posterior: null pointer");
+  AF_CHECK_ARG(B > 0 && HW > 0 && zc > 0, "af_vae_posterior: bad sizes B=%d HW=%lld zc=%d", B, HW, zc);
+  const long long total = static_cast<long long>(B) * zc * HW;
+  vae_posterior_kernel<<<grid_for(static_cast<size_t>(total), 256), 256, 0, stream>>>(
+      moments_nhwc, HW, zc, total, noise_nchw, out_scale, z_nchw, mean_nchw, logvar_nchw);
+  AF_LAUNCH_CHECK("vae_posterior_kernel");
   return 0;
 }
 

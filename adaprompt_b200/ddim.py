@@ -24,6 +24,17 @@ from . import _lib, ops
 from .diffusion_util import make_ddim_sampling_parameters, make_ddim_timesteps, noise_like
 
 
+def img2img_t_enc(strength: float, ddim_steps: int) -> int:
+    """t_enc = int(strength * ddim_steps) (SD scripts/img2img.py), checked on the host before any device work:
+    stochastic_encode gathers ddim_alphas[t_enc] on the GPU (t_enc == ddim_steps is out of range there) and decode
+    divides by t_enc - 1 when it anneals the guidance scale, so t_enc must lie in [2, ddim_steps - 1]."""
+    t_enc = int(strength * ddim_steps)
+    if not 2 <= t_enc <= ddim_steps - 1:
+        raise ValueError(f"img2img: strength {strength} with {ddim_steps} DDIM steps gives t_enc = int(strength * steps) "
+                         f"= {t_enc}; it must lie in [2, {ddim_steps - 1}]")
+    return t_enc
+
+
 class DDIMSampler(object):
     def __init__(self, model, schedule="linear", **kwargs):
         super().__init__()

@@ -44,7 +44,7 @@ class LatentDiffusionLite(nn.Module):
         self.model = DiffusionWrapper(unet if unet is not None else UNetModel(**SD15_UNET_CONFIG))
         self.cond_stage_model = cond_stage_model      # clip_text.FrozenCLIPEmbedder (ddpm.py:756)
         self.embedding_manager = embedding_manager    # embedding_manager.EmbeddingManagerLite (ddpm.py:793)
-        self.first_stage_model = first_stage_model    # vae.AutoencoderKL, decode side (ddpm.py:744-751)
+        self.first_stage_model = first_stage_model    # vae.AutoencoderKL (ddpm.py:744-751); encodes if built with_encoder
         self.use_layerwise_embedding = True           # v1-inference-ada.yaml:19
         self.N_CA_LAYERS = 16                         # ddpm.py:150
         self.empty_context = None
@@ -120,6 +120,27 @@ class LatentDiffusionLite(nn.Module):
             raise RuntimeError("LatentDiffusionLite: first_stage_model is not set")
         from .vae import decode_first_stage
         return decode_first_stage(self.first_stage_model, z, self.scale_factor, max_batch=max_batch)
+
+    @torch.no_grad()
+    def encode_first_stage(self, x, max_batch=None):
+        """ddpm.py encode_first_stage, the plain branch (no split_input_params): NCHW images in [-1, 1] -> the posterior
+        (needs first_stage_model built with_encoder=True)."""
+        if hasattr(self, "split_input_params"):
+            raise NotImplementedError("encode_first_stage: patch-split encoding is not used by AdaFace sampling")
+        if self.first_stage_model is None:
+            raise RuntimeError("LatentDiffusionLite: first_stage_model is not set")
+        from .vae import encode_first_stage
+        return encode_first_stage(self.first_stage_model, x, max_batch=max_batch)
+
+    def get_first_stage_encoding(self, encoder_posterior):
+        """ddpm.py get_first_stage_encoding: scale_factor * posterior.sample() (one fused kernel), or scale_factor * a
+        tensor."""
+        from .vae import DiagonalGaussianDistribution
+        if isinstance(encoder_posterior, DiagonalGaussianDistribution):
+            return encoder_posterior.scaled_sample(self.scale_factor)
+        if isinstance(encoder_posterior, torch.Tensor):
+            return self.scale_factor * encoder_posterior
+        raise NotImplementedError(f"encoder_posterior of type '{type(encoder_posterior)}' not yet implemented")
 
     def refresh_conditioning(self, cond, batch: int):
         """Hook for the CUDA-graph sampler: (re)project the conditioning tuple's context through the 16

@@ -187,6 +187,23 @@ def conv3x3(x0: torch.Tensor, wt: torch.Tensor, out: torch.Tensor, *, x1: Option
     return out
 
 
+def conv3x3_down01(x: torch.Tensor, wt: torch.Tensor, out: torch.Tensor, *, bias=None, bn: int = 0,
+                   gn_stats: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """conv3x3 stride 2 of F.pad(x, (0,1,0,1)) (VAE encoder Downsample).  x: bf16 NHWC [B,H,W,C] (H, W even);
+    wt: bf16 [Cout, 3, 3, C]; out: [B,H/2,W/2,Cout] fp32|bf16."""
+    lib = _lib.load()
+    _chk(x, torch.bfloat16, "x")
+    _chk(wt, torch.bfloat16, "wt")
+    B, H, W, C = (int(s) for s in x.shape)
+    Cout = int(wt.shape[0])
+    if wt.numel() != Cout * 9 * C:
+        raise ValueError("conv3x3_down01 weight shape mismatch")
+    ep = _epilogue(out, bias, gn_stats=gn_stats)
+    rc = lib.af_conv3x3_down01_bf16(x.data_ptr(), C, wt.data_ptr(), B, H, W, Cout, byref(ep), bn, _stream())
+    _lib.check(rc, "af_conv3x3_down01_bf16")
+    return out
+
+
 def attention(q: torch.Tensor, k: torch.Tensor, vt: torch.Tensor, out: torch.Tensor, *, B: int, heads: int, Nq: int,
               Nk: int, d: int, ldq: int, ldk: int, ldvt: int, kv_stride: int,
               key_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -402,6 +419,27 @@ def channel_mix4(x_nchw: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Ten
                              out.data_ptr(), _stream())
     _lib.check(rc, "af_channel_mix4")
     return out
+
+
+def vae_posterior(moments_nhwc: torch.Tensor, noise: Optional[torch.Tensor], out_scale: float, z: torch.Tensor,
+                  mean: Optional[torch.Tensor] = None, logvar: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """DiagonalGaussianDistribution of the encoder moments fp32 NHWC [B,H,W,2*zc]: z = out_scale * (mean + std * noise)
+    (noise None: out_scale * mean), and optionally mean / clamped logvar; z, noise, mean, logvar fp32 NCHW [B,zc,H,W]."""
+    lib = _lib.load()
+    _chk(moments_nhwc, torch.float32, "moments")
+    _chk(z, torch.float32, "z")
+    B, H, W, C2 = (int(s) for s in moments_nhwc.shape)
+    zc = C2 // 2
+    shape = (B, zc, H, W)
+    for t, n in ((noise, "noise"), (z, "z"), (mean, "mean"), (logvar, "logvar")):
+        if t is not None:
+            _chk(t, torch.float32, n)
+            if tuple(t.shape) != shape:
+                raise ValueError(f"vae_posterior: {n} shape {tuple(t.shape)} != {shape}")
+    rc = lib.af_vae_posterior(moments_nhwc.data_ptr(), B, H * W, zc, _p(noise), float(out_scale), z.data_ptr(), _p(mean),
+                              _p(logvar), _stream())
+    _lib.check(rc, "af_vae_posterior")
+    return z
 
 
 def softmax_rows(x: torch.Tensor, scale: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -17,6 +17,10 @@ reference's nn.Module checkpoints (embedding_manager.py:1824-1838 stores module 
 state_dict of SubjBasisGenerator).  `--synthetic` runs the whole pipeline on random-init weights of the real
 architecture with a hashing stand-in tokenizer (no vocabulary or checkpoint files exist offline): that is what the
 GPU test drives end to end.
+
+img2img (SD scripts/img2img.py): with --init_img the image (--W x --H pixels) is encoded by the VAE encoder, its latent
+is noised to step t_enc = int(--strength * --ddim_steps) by DDIMSampler.stochastic_encode and denoised by
+DDIMSampler.decode, whose guidance scale anneals from the first --scale value towards min(2, scale).
 """
 from __future__ import annotations
 
@@ -93,7 +97,7 @@ def build_pipeline(args, device):
 
     with torch.device("meta"):
         unet = UNetModel(**SD15_UNET_CONFIG)
-        vae = AutoencoderKL()
+        vae = AutoencoderKL(with_encoder=bool(getattr(args, "init_img", None)))
     unet, vae = unet.to_empty(device=device), vae.to_empty(device=device)
     clip_cfg = CLIPTextConfigLite(num_hidden_layers=args.synthetic_clip_layers) if args.synthetic else CLIPTextConfigLite()
     frozen = FrozenCLIPEmbedder(tokenizer=tokenizer, config=clip_cfg,
@@ -199,7 +203,12 @@ def parse_args(argv=None):
     p.add_argument("--no_cuda_graph", action="store_true")
     p.add_argument("--save_latents", action="store_true", help="also torch.save the latents next to the images")
     p.add_argument("--save_conditioning", action="store_true",
-                   help="also torch.save the conditioning tensors (c, uc) and x_T of every batch (parity checks)")
+                   help="also torch.save the conditioning tensors (c, uc) and x_T of every batch (parity checks); "
+                        "img2img: the posterior noise, the stochastic_encode noise and z_enc instead of x_T")
+    p.add_argument("--init_img", type=str, default=None,
+                   help="img2img: start from this image (RGB, exactly --W x --H pixels) instead of noise")
+    p.add_argument("--strength", type=float, default=0.75,
+                   help="img2img: noise level of the init image; t_enc = int(strength * ddim_steps) in [2, ddim_steps - 1]")
     p.add_argument("--synthetic", action="store_true", help="random-init weights + hashing tokenizer (no files needed)")
     p.add_argument("--synthetic_clip_layers", type=int, default=12)
     p.add_argument("--seed_weights", type=int, default=1234)
@@ -212,7 +221,24 @@ def parse_args(argv=None):
         p.error("--H / --W must be multiples of 64 and --f 8 (the SD-1.5 VAE)")
     if not args.synthetic and not args.ckpt:
         p.error("--ckpt is required unless --synthetic is given")
+    if args.init_img:
+        from .ddim import img2img_t_enc
+        try:
+            img2img_t_enc(args.strength, args.ddim_steps)
+        except ValueError as e:
+            p.error(str(e))
     return args
+
+
+def load_init_image(path: str, H: int, W: int) -> torch.Tensor:
+    """SD scripts/img2img.py load_img: RGB -> [1, 3, H, W] fp32 in [-1, 1]; the size must already be W x H."""
+    import numpy as np
+    from PIL import Image
+    image = Image.open(path).convert("RGB")
+    if image.size != (W, H):
+        raise SystemExit(f"--init_img {path} is {image.size[0]}x{image.size[1]} pixels; --W x --H is {W}x{H}")
+    arr = np.array(image).astype(np.float32) / 255.0
+    return 2. * torch.from_numpy(arr[None].transpose(0, 3, 1, 2).copy()) - 1.
 
 
 @torch.no_grad()
@@ -251,6 +277,12 @@ def run(args) -> List[str]:
         id_embs = torch.randn(1, 512, generator=torch.Generator().manual_seed(args.seed)).to(device)
     id_embs = torch.nn.functional.normalize(id_embs, p=2, dim=-1)                                  # adaface/util.py:311
     shape = [args.C, args.H // args.f, args.W // args.f]
+    init_image = t_enc = None
+    if args.init_img:
+        from .ddim import img2img_t_enc
+        t_enc = img2img_t_enc(args.strength, args.ddim_steps)
+        init_image = load_init_image(args.init_img, args.H, args.W).to(device)
+        sampler.make_schedule(ddim_num_steps=args.ddim_steps, ddim_eta=args.ddim_eta, verbose=False)
     paths, all_imgs = [], []
     for start in range(0, len(mine), bs):
         chunk = mine[start:start + bs]
@@ -259,11 +291,26 @@ def run(args) -> List[str]:
         c = model.get_learned_conditioning(texts, zs_clip_features=None, zs_id_embs=id_embs,
                                            zs_out_id_embs_scale_range=tuple(args.zs_out_id_embs_scale_range))   # :606-613
         uc = model.get_learned_conditioning([args.neg_prompt] * n)                                              # :602
-        g = torch.Generator().manual_seed(args.seed + 1000 * rank + start)
-        x_T = torch.randn(n, *shape, generator=g).to(device)                                                    # :578
-        samples, _ = sampler.sample(S=args.ddim_steps, batch_size=n, shape=shape, conditioning=c,
-                                    unconditional_conditioning=uc, guidance_scale=tuple(args.scale),
-                                    eta=args.ddim_eta, x_T=x_T, verbose=False)                                  # :614-626
+        if init_image is None:
+            g = torch.Generator().manual_seed(args.seed + 1000 * rank + start)
+            x_T = torch.randn(n, *shape, generator=g).to(device)                                                # :578
+            samples, _ = sampler.sample(S=args.ddim_steps, batch_size=n, shape=shape, conditioning=c,
+                                        unconditional_conditioning=uc, guidance_scale=tuple(args.scale),
+                                        eta=args.ddim_eta, x_T=x_T, verbose=False)                              # :614-626
+            saved = {"x_T": x_T.cpu()}
+        else:
+            # img2img.py: encode the batch of init images, noise to t_enc, decode with CFG.  The two noises are drawn
+            # where the reference draws them (posterior: host generator; stochastic_encode: randn_like on the device)
+            torch.manual_seed(args.seed + 1000 * rank + start)
+            posterior = model.encode_first_stage(init_image.repeat(n, 1, 1, 1))
+            post_noise = torch.randn(posterior.mean.shape)
+            init_latent = posterior.scaled_sample(model.scale_factor, noise=post_noise)    # get_first_stage_encoding
+            se_noise = torch.randn_like(init_latent)
+            z_enc = sampler.stochastic_encode(init_latent, torch.full((n,), t_enc, dtype=torch.long, device=device),
+                                              noise=se_noise)
+            samples = sampler.decode(z_enc, c, t_enc, guidance_scale=args.scale[0], unconditional_conditioning=uc)
+            saved = {"posterior_noise": post_noise, "stochastic_encode_noise": se_noise.cpu(), "z_enc": z_enc.cpu(),
+                     "t_enc": t_enc}
         x = model.decode_first_stage(samples)                                                                   # :685
         x = torch.clamp((x + 1.0) / 2.0, min=0.0, max=1.0).cpu()                                                # :687
         paths += save_images(x, os.path.join(args.outdir, "samples"), b0 + start, f"r{rank}")
@@ -271,7 +318,7 @@ def run(args) -> List[str]:
         if args.save_latents:
             torch.save(samples.cpu(), os.path.join(args.outdir, "samples", f"r{rank}-{b0 + start:05d}-latents.pt"))
         if args.save_conditioning:
-            torch.save({"c": c[0].cpu(), "uc": uc[0].cpu(), "x_T": x_T.cpu(), "prompts": texts},
+            torch.save({"c": c[0].cpu(), "uc": uc[0].cpu(), "prompts": texts, **saved},
                        os.path.join(args.outdir, "samples", f"r{rank}-{b0 + start:05d}-cond.pt"))
     if all_imgs:
         save_grid(torch.cat(all_imgs), os.path.join(args.outdir, f"grid-r{rank}.png"), args.n_rows or args.n_samples)

@@ -1,14 +1,18 @@
-"""Host mirror of the first-stage DECODER: latents -> RGB (SURVEY.md section 8(f) row N1).
+"""Host mirror of the first stage: latents -> RGB (decoder) and, with `with_encoder=True`, RGB -> posterior over latents
+(encoder, for img2img) - SURVEY.md section 8(f) row N1.
 
 Reference: ldm/modules/diffusionmodules/model.py (ResnetBlock :83-142, AttnBlock :151-242, Upsample :43-58,
-Decoder :502-609), ldm/models/autoencoder.py (AutoencoderKL.decode :330-333) and
-LatentDiffusion.decode_first_stage (ldm/models/diffusion/ddpm.py:1260-1318, the `1/scale_factor` scaling :1267),
-configured by configs/stable-diffusion/v1-inference-ada.yaml:53-73 (ch 128, ch_mult [1,2,4,4], 2 res blocks,
-z_channels 4, no attention except the single-head 512-channel AttnBlock in the middle).
+Downsample :61-79, Encoder :408-500, Decoder :502-609), ldm/modules/distributions/distributions.py
+(DiagonalGaussianDistribution :24-44), ldm/models/autoencoder.py (AutoencoderKL :285-333) and
+LatentDiffusion.decode_first_stage / encode_first_stage / get_first_stage_encoding (ldm/models/diffusion/ddpm.py,
+the `1/scale_factor` scaling :1267), configured by configs/stable-diffusion/v1-inference-ada.yaml:53-73 (ch 128,
+ch_mult [1,2,4,4], 2 res blocks, z_channels 4, double_z, no attention except the single-head 512-channel AttnBlock in
+the middle).
 
-Same constructor arguments, forward signatures and state_dict key names as the reference (`decoder.*`,
-`post_quant_conv.*`), so an SD-1.5 VAE checkpoint loads unchanged (the encoder / quant_conv / loss keys of a full
-checkpoint are ignored: this is the sampling path).  The torch.nn layers only hold parameters; all arithmetic runs in
+Same constructor arguments, forward signatures and state_dict key names as the reference (`encoder.*`, `decoder.*`,
+`quant_conv.*`, `post_quant_conv.*`), so an SD-1.5 VAE checkpoint loads unchanged.  By default only the decode side is
+built (the sampling path): the encoder / quant_conv keys of a full checkpoint are then ignored, and the loss keys always
+are.  The torch.nn layers only hold parameters; all arithmetic runs in
 libadaface_b200.so with the same kernels as the UNet: NHWC fp32 residual stream, bf16 tensor-core operands, GroupNorm
 statistics produced by the conv epilogues.  The middle AttnBlock has ONE head of 512 channels over h*w tokens - too wide
 for the flash kernels' TMEM accumulators - so, like the reference, it materialises the scores: two tcgen05 GEMMs and a
@@ -57,6 +61,32 @@ class Upsample(PackedModule):
         ops.upsample2x_cast(x, up)
         out, st = _conv_out_act(B, 2 * H, 2 * W, C, x.device)
         ops.conv3x3(up, pk["w"], out, bias=pk["b"], gn_stats=st.buf if st else None)
+        return Act(out, st)
+
+    def forward(self, x):
+        return _nchw(self._run(Act(x.float().permute(0, 2, 3, 1).contiguous())).t)
+
+
+class Downsample(PackedModule):
+    """model.py:61-79: F.pad(x, (0, 1, 0, 1)) then conv3x3 stride 2 pad 0 - one kernel, the pad is TMA zero fill."""
+
+    def __init__(self, in_channels, with_conv):
+        super().__init__()
+        if not with_conv:
+            raise NotImplementedError("Downsample: resamp_with_conv=False (avg_pool2d) is not used by the SD-1.5 VAE")
+        self.with_conv = with_conv
+        self.conv = nn.Conv2d(in_channels, in_channels, kernel_size=3, stride=2, padding=0)
+
+    def _pack(self):
+        return {"w": pack_conv3x3(self.conv.weight.detach()), "b": _f(self.conv.bias)}
+
+    def _run(self, a: Act) -> Act:
+        pk = self.packed()
+        x = a.t
+        B, H, W, C = x.shape
+        xb = ops.cast_bf16(x)
+        out, st = _conv_out_act(B, H // 2, W // 2, C, x.device)
+        ops.conv3x3_down01(xb, pk["w"], out, bias=pk["b"], gn_stats=st.buf if st else None)
         return Act(out, st)
 
     def forward(self, x):
@@ -196,7 +226,8 @@ def make_attn(in_channels, attn_type="vanilla"):
 
 
 class _ConvIn(nn.Conv2d):
-    """Decoder.conv_in (4 -> 512): reads the public NCHW latent, writes the NHWC fp32 stream."""
+    """Decoder.conv_in (4 -> 512) / Encoder.conv_in (3 -> 128): reads the public NCHW input, writes the NHWC fp32
+    stream."""
 
     def _run(self, z_nchw: torch.Tensor) -> torch.Tensor:
         B, C, H, W = z_nchw.shape
@@ -299,37 +330,221 @@ class Decoder(PackedModule):
         return out
 
 
+class Encoder(PackedModule):
+    """model.py:408-500."""
+
+    def __init__(self, *, ch, out_ch, ch_mult=(1, 2, 4, 8), num_res_blocks, attn_resolutions, dropout=0.0,
+                 resamp_with_conv=True, in_channels, resolution, z_channels, double_z=True, use_linear_attn=False,
+                 attn_type="vanilla", **ignore_kwargs):
+        super().__init__()
+        if use_linear_attn:
+            attn_type = "linear"
+        self.ch = ch
+        self.temb_ch = 0
+        self.num_resolutions = len(ch_mult)
+        self.num_res_blocks = num_res_blocks
+        self.resolution = resolution
+        self.in_channels = in_channels
+        self.conv_in = _ConvIn(in_channels, self.ch, kernel_size=3, stride=1, padding=1)
+        curr_res = resolution
+        in_ch_mult = (1,) + tuple(ch_mult)
+        self.in_ch_mult = in_ch_mult
+        self.down = nn.ModuleList()
+        for i_level in range(self.num_resolutions):
+            block = nn.ModuleList()
+            attn = nn.ModuleList()
+            block_in = ch * in_ch_mult[i_level]
+            block_out = ch * ch_mult[i_level]
+            for _ in range(self.num_res_blocks):
+                block.append(ResnetBlock(in_channels=block_in, out_channels=block_out, temb_channels=self.temb_ch,
+                                         dropout=dropout))
+                block_in = block_out
+                if curr_res in attn_resolutions:
+                    attn.append(make_attn(block_in, attn_type=attn_type))
+            down = nn.Module()
+            down.block = block
+            down.attn = attn
+            if i_level != self.num_resolutions - 1:
+                down.downsample = Downsample(block_in, resamp_with_conv)
+                curr_res = curr_res // 2
+            self.down.append(down)
+        self.mid = nn.Module()
+        self.mid.block_1 = ResnetBlock(in_channels=block_in, out_channels=block_in, temb_channels=self.temb_ch,
+                                       dropout=dropout)
+        self.mid.attn_1 = make_attn(block_in, attn_type=attn_type)
+        self.mid.block_2 = ResnetBlock(in_channels=block_in, out_channels=block_in, temb_channels=self.temb_ch,
+                                       dropout=dropout)
+        self.norm_out = Normalize(block_in)
+        self.conv_out = nn.Conv2d(block_in, 2 * z_channels if double_z else z_channels, kernel_size=3, stride=1,
+                                  padding=1)
+        if self.conv_out.out_channels % 8:
+            raise NotImplementedError("Encoder: conv_out needs a multiple of 8 output channels (double_z, z_channels 4)")
+
+    def _pack(self):
+        return {"nw": _f(self.norm_out.weight), "nb": _f(self.norm_out.bias), "eps": float(self.norm_out.eps),
+                "w": pack_conv3x3(self.conv_out.weight.detach()), "b": _f(self.conv_out.bias)}
+
+    def _run(self, x: torch.Tensor, head=None) -> torch.Tensor:
+        """x NCHW [B, in_channels, H, W] -> conv_out output NHWC fp32 [B, H/8, W/8, Cout].  head = (packed weight, bias)
+        replaces conv_out's own (AutoencoderKL folds quant_conv into it)."""
+        if not x.is_cuda:
+            raise RuntimeError("Encoder: the B200 path has no CPU fallback - move the images to a CUDA device")
+        pk = self.packed()
+        h = Act(self.conv_in._run(x))                                        # :470
+        for i_level in range(self.num_resolutions):                          # :471-478
+            for i_block in range(self.num_res_blocks):
+                h = self.down[i_level].block[i_block]._run(h)
+                if len(self.down[i_level].attn) > 0:
+                    h = self.down[i_level].attn[i_block]._run(h)
+            if i_level != self.num_resolutions - 1:
+                h = self.down[i_level].downsample._run(h)
+        h = self.mid.block_1._run(h)                                         # :482
+        if isinstance(self.mid.attn_1, AttnBlock):
+            h = self.mid.attn_1._run(h)                                      # :483
+        h = self.mid.block_2._run(h)                                         # :484
+        B, H, W, C = h.t.shape
+        dev = h.t.device
+        y = torch.empty(B, H, W, C, dtype=torch.bfloat16, device=dev)
+        ops.groupnorm_apply(h.t, h.stats(), pk["nw"], pk["nb"], pk["eps"], True, y)    # :487-488
+        del h
+        w, b = head if head is not None else (pk["w"], pk["b"])
+        out = torch.empty(B, H, W, int(w.shape[0]), dtype=torch.float32, device=dev)
+        ops.conv3x3(y, w, out, bias=b, bn=64)                                            # :489
+        return out
+
+    def forward(self, x, mask=None):
+        """x: [B, in_channels, H, W] -> [B, Cout, H/8, W/8] fp32 NCHW."""
+        if mask is not None:
+            raise NotImplementedError("Encoder: the fg/bg mask input belongs to the fork's training path")
+        return _nchw(self._run(x.float().contiguous()))
+
+
+class DiagonalGaussianDistribution(object):
+    """distributions.py:24-44 over the encoder's moments.  mean and the clamped logvar come out of one kernel
+    (af_vae_posterior), which also draws sample() = mean + std * noise - with the noise taken from the host generator
+    like the reference (`torch.randn(self.mean.shape)`), so the global CPU RNG stream advances as there.  std, var and
+    the NCHW `parameters` are formed on first use.  kl() / nll() are training losses and not mirrored."""
+
+    def __init__(self, parameters=None, deterministic=False, *, moments_nhwc=None):
+        if moments_nhwc is None:
+            moments_nhwc = parameters.float().permute(0, 2, 3, 1).contiguous()
+        self._moments = moments_nhwc
+        self._parameters = parameters
+        self.deterministic = deterministic
+        B, H, W, C2 = moments_nhwc.shape
+        zc = C2 // 2
+        dev = moments_nhwc.device
+        self.mean = torch.empty(B, zc, H, W, dtype=torch.float32, device=dev)
+        self.logvar = torch.empty_like(self.mean)
+        ops.vae_posterior(moments_nhwc, None, 1.0, self.mean, logvar=self.logvar)
+        self._std = self._var = None
+
+    @property
+    def parameters(self):
+        if self._parameters is None:
+            self._parameters = self._moments.permute(0, 3, 1, 2).contiguous()
+        return self._parameters
+
+    @property
+    def std(self):
+        if self._std is None:
+            self._std = torch.zeros_like(self.mean) if self.deterministic else torch.exp(0.5 * self.logvar)
+        return self._std
+
+    @property
+    def var(self):
+        if self._var is None:
+            self._var = torch.zeros_like(self.mean) if self.deterministic else torch.exp(self.logvar)
+        return self._var
+
+    def scaled_sample(self, scale: float = 1.0, noise: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """scale * sample() in one kernel: get_first_stage_encoding's scale_factor * z.  noise (NCHW like mean) replaces
+        the draw from the host generator."""
+        if noise is None:
+            noise = torch.randn(self.mean.shape)
+        noise = noise.to(device=self.mean.device, dtype=torch.float32).contiguous()
+        z = torch.empty_like(self.mean)
+        # deterministic: std is 0, so mean + 0 * noise == mean (the reference still draws the noise)
+        ops.vae_posterior(self._moments, None if self.deterministic else noise, float(scale), z)
+        return z
+
+    def sample(self):
+        return self.scaled_sample(1.0)
+
+    def mode(self):
+        return self.mean
+
+
 SD15_VAE_DDCONFIG = dict(  # configs/stable-diffusion/v1-inference-ada.yaml:58-72
     double_z=True, z_channels=4, resolution=256, in_channels=3, out_ch=3, ch=128, ch_mult=[1, 2, 4, 4],
     num_res_blocks=2, attn_resolutions=[], dropout=0.0)
 
 
 class AutoencoderKL(nn.Module):
-    """ldm/models/autoencoder.py:285-333, decode side.  `post_quant_conv` (1x1, embed_dim -> z_channels) is a tiny fp32
+    """ldm/models/autoencoder.py:285-333.  Decode side: `post_quant_conv` (1x1, embed_dim -> z_channels) is a tiny fp32
     channel-mix kernel on the NCHW latent (16 MACs per pixel) in front of the decoder's conv_in kernel; the
-    `1 / scale_factor` of decode_first_stage rides along as its input scale."""
+    `1 / scale_factor` of decode_first_stage rides along as its input scale.  with_encoder=True also builds the encoder
+    side: `quant_conv` (1x1, 2*z_channels -> 2*embed_dim) is linear and directly follows the encoder's 3x3 conv_out, so
+    it is folded into that convolution's weights (fp32 product, one bf16 rounding) and the moments leave one
+    tensor-core conv."""
 
     def __init__(self, ddconfig=None, lossconfig=None, embed_dim=4, ckpt_path=None, ignore_keys=(), image_key="image",
-                 colorize_nlabels=None, monitor=None):
+                 colorize_nlabels=None, monitor=None, with_encoder=False):
         super().__init__()
         ddconfig = dict(SD15_VAE_DDCONFIG if ddconfig is None else ddconfig)
         self.image_key = image_key
         self.embed_dim = embed_dim
+        self.with_encoder = with_encoder
+        if with_encoder:
+            if not ddconfig.get("double_z", True):
+                raise NotImplementedError("AutoencoderKL: the encoder needs double_z (autoencoder.py:299)")
+            self.encoder = Encoder(**ddconfig)
         self.decoder = Decoder(**ddconfig)
+        if with_encoder:
+            self.quant_conv = nn.Conv2d(2 * ddconfig["z_channels"], 2 * embed_dim, 1)
         self.post_quant_conv = nn.Conv2d(embed_dim, ddconfig["z_channels"], 1)
         if ckpt_path is not None:
             sd = torch.load(ckpt_path, map_location="cpu")
             self.load_state_dict(sd.get("state_dict", sd))
 
     def load_state_dict(self, state_dict, strict: bool = True, **kw):
-        """Full AutoencoderKL checkpoints also carry encoder.*, quant_conv.* and loss.* tensors: the sampling path has no
-        use for them, so they are dropped instead of failing a strict load."""
-        keep = {k: v for k, v in state_dict.items()
-                if k.startswith("decoder.") or k.startswith("post_quant_conv.")}
+        """Full AutoencoderKL checkpoints also carry loss.* tensors (and encoder.* / quant_conv.*, which only a module
+        built with_encoder uses): what this module has no parameter for is dropped instead of failing a strict load."""
+        prefixes = ("decoder.", "post_quant_conv.") + (("encoder.", "quant_conv.") if self.with_encoder else ())
+        keep = {k: v for k, v in state_dict.items() if k.startswith(prefixes)}
         return super().load_state_dict(keep, strict=strict, **kw)
 
+    def _moments_head(self):
+        """conv_out with quant_conv folded in: W' = Wq . Wc, b' = Wq . bc + bq in fp32, then the bf16 pack."""
+        co, qc = self.encoder.conv_out, self.quant_conv
+        params = (co.weight, co.bias, qc.weight, qc.bias)
+        key = tuple((p.data_ptr(), p._version) for p in params)
+        ent = self.__dict__.get("_head")
+        if ent is None or ent[0] != key:
+            with torch.no_grad():
+                wq = qc.weight.detach().float().reshape(qc.out_channels, qc.in_channels)
+                wc = co.weight.detach().float()
+                w = (wq @ wc.reshape(wc.shape[0], -1)).reshape(qc.out_channels, *wc.shape[1:])
+                b = wq @ co.bias.detach().float() + qc.bias.detach().float()
+            ent = (key, (pack_conv3x3(w), b.contiguous()))
+            self.__dict__["_head"] = ent
+        return ent[1]
+
+    @torch.no_grad()
+    def _moments(self, x) -> torch.Tensor:
+        """x NCHW images -> quant_conv(encoder(x)) as NHWC fp32 [B, H/8, W/8, 2*embed_dim]."""
+        if not self.with_encoder:
+            raise NotImplementedError("AutoencoderKL.encode: build the module with with_encoder=True (the default is the "
+                                      "decode side only)")
+        if not x.is_cuda:
+            raise RuntimeError("AutoencoderKL.encode: the B200 path has no CPU fallback - move the images to a CUDA device")
+        return self.encoder._run(x.float().contiguous(), head=self._moments_head())
+
     def encode(self, x, mask=None):
-        raise NotImplementedError("AutoencoderKL.encode: only the sampling direction (decode) is on the B200 path")
+        """autoencoder.py:316-320: NCHW images in [-1, 1] -> DiagonalGaussianDistribution over the latents."""
+        if mask is not None:
+            raise NotImplementedError("AutoencoderKL.encode: the fg/bg mask input belongs to the fork's training path")
+        return DiagonalGaussianDistribution(moments_nhwc=self._moments(x))
 
     @torch.no_grad()
     def decode(self, z, in_scale: float = 1.0):
@@ -342,6 +557,16 @@ class AutoencoderKL(nn.Module):
 
     def forward(self, z):
         return self.decode(z)
+
+
+def encode_first_stage(first_stage_model: AutoencoderKL, x: torch.Tensor, max_batch: Optional[int] = None
+                       ) -> DiagonalGaussianDistribution:
+    """LatentDiffusion.encode_first_stage (ddpm.py, the non-split branch): first_stage_model.encode(x).  max_batch bounds
+    the images encoded per pass (a 512^2 activation with 128 channels is 134 MB per image and tensor)."""
+    if max_batch is None or x.shape[0] <= max_batch:
+        return first_stage_model.encode(x)
+    return DiagonalGaussianDistribution(moments_nhwc=torch.cat(
+        [first_stage_model._moments(x[i:i + max_batch]) for i in range(0, x.shape[0], max_batch)], 0))
 
 
 def decode_first_stage(first_stage_model: AutoencoderKL, z: torch.Tensor, scale_factor: float = 0.18215,

@@ -102,6 +102,13 @@ int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, const void* 
                     int stride, const af_epilogue* ep, int bn_hint, af_stream_t stream);
 /* statistic slots per sample that af_conv3x3_bf16 writes for an Ho x Wo output (0: unsupported geometry). */
 int af_conv3x3_gn_slots(int Ho, int Wo);
+/* 3x3 convolution, stride 2, on the input padded by one zero row at the bottom and one zero column at the right
+ * (F.pad(x, (0,1,0,1)) then padding 0: the VAE encoder's Downsample, ldm/modules/diffusionmodules/model.py:61-79).
+ * Output pixel (oh, ow) reads input rows 2*oh .. 2*oh+2 and columns 2*ow .. 2*ow+2.  X NHWC bf16 [B,H,W,C], H and W
+ * even, C % 64 == 0; Wt[Cout][ky][kx][C] bf16, Cout % 8 == 0; output [B,H/2,W/2,Cout] through the epilogue as in
+ * af_conv3x3_bf16 (GroupNorm statistics: af_conv3x3_gn_slots(H/2, W/2)). */
+int af_conv3x3_down01_bf16(const void* X, int C, const void* Wt, int B, int H, int W, int Cout, const af_epilogue* ep,
+                           int bn_hint, af_stream_t stream);
 
 /* Flash attention, 8-head SD-1.5 geometry (d in {40,80,160}); replaces attention.py:198-242.
  * Q [B,Nq,ldq], K [B,Nk,ldk] bf16 with head h at column h*DP (DP = 48 for d = 40, zero padded, else d);
@@ -187,7 +194,8 @@ int af_layernorm_f32(const float* x, long long rows, int C, const float* gamma, 
                      af_stream_t stream);
 
 /* First / last convolutions of the UNet (4 latent channels), fp32 CUDA-core kernels that also convert
- * between the public NCHW layout and the internal NHWC one (openaimodel.py:527-533, :693-697). */
+ * between the public NCHW layout and the internal NHWC one (openaimodel.py:527-533, :693-697).  af_conv_in also takes
+ * Cin = 3: the VAE encoder's conv_in on RGB images (model.py:436-440). */
 int af_conv_in(const float* x_nchw, const float* w /*[Cout,Cin,3,3]*/, const float* bias, float* y_nhwc, int B, int Cin,
                int H, int W, int Cout, af_stream_t stream);
 int af_conv_out(const void* x_nhwc_bf16, const float* w_packed /*[Cout,3,3,C]*/, const float* bias, float* y_nchw,
@@ -209,6 +217,13 @@ int af_cast_bf16(const float* x, void* y_bf16, long long n, af_stream_t stream);
  * post_quant_conv applied to z / scale_factor (ldm/models/autoencoder.py:331, ldm/models/diffusion/ddpm.py:1267). */
 int af_channel_mix4(const float* x_nchw, const float* w, const float* bias, float in_scale, int B, int Cin, int Cout,
                     long long HW, float* y_nchw, af_stream_t stream);
+/* Posterior of the VAE encoder (DiagonalGaussianDistribution, ldm/modules/distributions/distributions.py:24-44) fused
+ * with get_first_stage_encoding's scale (ddpm.py): moments NHWC fp32 [B,HW,2*zc] = (mean | logvar) per pixel.
+ * lv = clamp(logvar, -30, 20); z = out_scale * (mean + exp(0.5*lv) * noise), or out_scale * mean (the mode) when noise
+ * is NULL; fp32 in the reference's operation order (no contraction, full-precision exp).  noise, z, mean and logvar
+ * (= lv) are NCHW fp32 [B,zc,HW]; mean / logvar may be NULL. */
+int af_vae_posterior(const float* moments_nhwc, int B, long long HW, int zc, const float* noise_nchw, float out_scale,
+                     float* z_nchw, float* mean_nchw, float* logvar_nchw, af_stream_t stream);
 /* Row softmax of materialised scores for the VAE's single-head AttnBlock (ldm/modules/diffusionmodules/model.py:
  * 188-193: softmax(q.k^T * c^-1/2, dim=2)): y[r][0..n) = softmax(scale * x[r][0..n)), fp32 in, bf16 out, n <= 16384. */
 int af_softmax_rows(const float* x, long long ldx, long long rows, int n, float scale, void* y_bf16, long long ldo,
