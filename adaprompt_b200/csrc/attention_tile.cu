@@ -394,10 +394,7 @@ __global__ void __launch_bounds__(256, 2) attention_tile_kernel(const __grid_con
         // The first kLate x 32 exponentials go to REGISTERS before the wait for the P buffer (PV_{j-1} may still be reading
         // it): the wait - 360 cycles at the head of the chain before - hides behind them; every later chunk is stored as soon
         // as it is computed (storing everything late was slower: the stores then drain at the tail of the block).
-#ifndef AF_TILE_LATE_CHUNKS
-#define AF_TILE_LATE_CHUNKS 2
-#endif
-        constexpr int kLate = AF_TILE_LATE_CHUNKS * 32 < BN ? AF_TILE_LATE_CHUNKS * 32 : BN / 2;
+        constexpr int kLate = BN > 64 ? 64 : BN / 2;   // two 32-column chunks (one when BN = 64)
         uint32_t pk0[kLate / 2];
 #pragma unroll
         for (int c = 0; c < kLate; c += 32) {
@@ -601,13 +598,7 @@ int attention_tile_dispatch(const void* Q, long long ldq, const void* K, long lo
   p.out = static_cast<__nv_bfloat16*>(O);
   p.ldo = static_cast<long long>(heads) * d;
   // d = 40: every third exponential on the FMA pipe (0.764 -> 0.688 ms at N = 4096, profiles/r02_attention.md)
-#ifndef AF_TILE_POLY40
-#define AF_TILE_POLY40 3
-#endif
-#ifndef AF_TILE_POLY80
-#define AF_TILE_POLY80 0
-#endif
-  return d == 40 ? launch_tile<40, AF_TILE_POLY40>(p, stream) : launch_tile<80, AF_TILE_POLY80>(p, stream);
+  return d == 40 ? launch_tile<40, 3>(p, stream) : launch_tile<80, 0>(p, stream);
 }
 
 }  // namespace af

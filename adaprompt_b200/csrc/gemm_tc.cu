@@ -818,7 +818,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
 // host side
 // ---------------------------------------------------------------------------------------------
 // No process-global switches: the tile schedule (af_epilogue.pair_mode) and the timeline probe (af_epilogue.trace) are
-// per-call options.
+// per-call options.  plan_linear / plan_conv make every argument check that needs no buffer and every schedule decision;
+// the launches and the introspection calls (af_gemm_plan / af_conv3x3_plan) share them.
 
 template <int BN, bool GEGLU, int SLOTS, bool CTA2, bool DOWN01 = false>
 static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
@@ -861,16 +862,11 @@ static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
 // any tile width >= 128 from 512 row tiles (the VAE decoder's 128^2 .. 512^2 layers: -5 .. -10 %); it
 // loses where the tile count is small (16x16 / 8x8: those go to split-K, which the pair schedule does not do).
 // Mode 1 ("auto") applies that; mode 2 forces pairs wherever they are legal (tests).
-static bool want_pair(int pair_mode, int m_tiles, int n_tiles, int bn, int amode) {
-  (void)n_tiles;
+static bool want_pair(int pair_mode, int m_tiles, int bn, bool conv) {
   if (pair_mode == AF_PAIR_NEVER || m_tiles < 2) return false;
   if (pair_mode == AF_PAIR_ALWAYS) return true;
-#ifdef AF_PAIR_R1_RULE
-  return amode == 0 && bn >= 160 && ((m_tiles + 1) / 2) * n_tiles >= num_sms();
-#endif
-  if (amode == 0) return bn >= 160 && m_tiles >= 16;
-  if (amode == 1) return (bn == 160 && m_tiles >= 128) || (bn >= 128 && m_tiles >= 512);   // the second clause: VAE decoder layers
-  return false;
+  if (!conv) return bn >= 160 && m_tiles >= 16;
+  return (bn == 160 && m_tiles >= 128) || (bn >= 128 && m_tiles >= 512);   // the second clause: VAE decoder layers
 }
 
 template <int BN, bool GEGLU, int SLOTS, bool DOWN01 = false>
@@ -922,27 +918,40 @@ static void plan_split(GemmParams& p, int bn, bool pair, const af_epilogue* ep) 
   p.ws = reinterpret_cast<float*>(static_cast<char*>(ep->splitk_ws) + static_cast<size_t>(kSplitFlagInts) * 4);
 }
 
-static int dispatch_gemm(int bn, const GemmParams& p, bool pair, cudaStream_t stream) {
-  if (p.geglu) return launch_gemm_mode<256, true, 2>(p, pair, stream);
+// The kernel instantiation a planner chose; the rest of the schedule is in GemmParams.
+struct GemmPlan {
+  int bn;      // N-tile width
+  bool pair;   // CTA pairs
+  int slots;   // epilogue slots per warp
+};
+
+constexpr int tile_key(int bn, int slots) { return bn * 4 + slots; }   // (tile width, epilogue slots) as one case label
+
+static int dispatch_gemm(const GemmParams& p, const GemmPlan& s, cudaStream_t stream) {
+  if (p.geglu) return launch_gemm_mode<256, true, 2>(p, s.pair, stream);
   if (p.amode == 3) {
-    switch (bn) {
-      case 64: return launch_gemm_mode<64, false, 1, true>(p, pair, stream);
-      case 128: return launch_gemm_mode<128, false, 1, true>(p, pair, stream);
-      case 160: return launch_gemm_mode<160, false, 1, true>(p, pair, stream);
-      case 256: return launch_gemm_mode<256, false, 1, true>(p, pair, stream);
-      default: set_error("unsupported BN %d (64/128/160/256)", bn); return -1;
+    switch (tile_key(s.bn, s.slots)) {
+      case tile_key(64, 1): return launch_gemm_mode<64, false, 1, true>(p, s.pair, stream);
+      case tile_key(128, 1): return launch_gemm_mode<128, false, 1, true>(p, s.pair, stream);
+      case tile_key(160, 1): return launch_gemm_mode<160, false, 1, true>(p, s.pair, stream);
+      case tile_key(256, 1): return launch_gemm_mode<256, false, 1, true>(p, s.pair, stream);
+    }
+  } else {
+    switch (tile_key(s.bn, s.slots)) {
+      case tile_key(64, 1): return launch_gemm_mode<64, false, 1>(p, s.pair, stream);
+      case tile_key(64, 2): return launch_gemm_mode<64, false, 2>(p, s.pair, stream);
+      case tile_key(64, 3): return launch_gemm_mode<64, false, 3>(p, s.pair, stream);
+      case tile_key(128, 1): return launch_gemm_mode<128, false, 1>(p, s.pair, stream);
+      case tile_key(128, 2): return launch_gemm_mode<128, false, 2>(p, s.pair, stream);
+      case tile_key(128, 3): return launch_gemm_mode<128, false, 3>(p, s.pair, stream);
+      case tile_key(160, 1): return launch_gemm_mode<160, false, 1>(p, s.pair, stream);
+      case tile_key(160, 2): return launch_gemm_mode<160, false, 2>(p, s.pair, stream);
+      case tile_key(160, 3): return launch_gemm_mode<160, false, 3>(p, s.pair, stream);
+      case tile_key(256, 1): return launch_gemm_mode<256, false, 1>(p, s.pair, stream);
     }
   }
-  // epilogue slots per warp: 3 (two residual chunks in flight) for the memory-bound linear GEMMs with a residual,
-  // 1 for the K-deep convolutions (their epilogue has slack; the shared memory goes to the operand ring), else 2
-  const int slots = p.amode != 0 ? 1 : (p.residual != nullptr ? 3 : 2);
-  switch (bn) {
-    case 64: return slots == 1 ? launch_gemm_mode<64, false, 1>(p, pair, stream) : slots == 3 ? launch_gemm_mode<64, false, 3>(p, pair, stream) : launch_gemm_mode<64, false, 2>(p, pair, stream);
-    case 128: return slots == 1 ? launch_gemm_mode<128, false, 1>(p, pair, stream) : slots == 3 ? launch_gemm_mode<128, false, 3>(p, pair, stream) : launch_gemm_mode<128, false, 2>(p, pair, stream);
-    case 160: return slots == 1 ? launch_gemm_mode<160, false, 1>(p, pair, stream) : slots == 3 ? launch_gemm_mode<160, false, 3>(p, pair, stream) : launch_gemm_mode<160, false, 2>(p, pair, stream);
-    case 256: return launch_gemm_mode<256, false, 1>(p, pair, stream);
-    default: set_error("unsupported BN %d (64/128/160/256)", bn); return -1;
-  }
+  set_error("no kernel for BN %d with %d epilogue slots (amode %d)", s.bn, s.slots, p.amode);
+  return -1;
 }
 
 // Output / residual tensor maps: 4-D {cols, w, h, n} with one warp's 32 rows x 32 columns as the box.
@@ -977,6 +986,14 @@ static int make_epilogue_maps(GemmParams& p, int out_cols, bool conv) {
   return rc;
 }
 
+// 2-D bf16 operand [rows][cols], cols contiguous with a row pitch of ld elements, read in boxes of 64 columns x box_rows.
+static int make_operand_map(CUtensorMap* m, const void* base, long long cols, long long rows, long long ld, int box_rows) {
+  uint64_t dims[2] = {static_cast<uint64_t>(cols), static_cast<uint64_t>(rows)};
+  uint64_t str[1] = {static_cast<uint64_t>(ld) * 2};
+  uint32_t box[2] = {64, static_cast<uint32_t>(box_rows)};
+  return make_tmap_bf16(m, base, 2, dims, str, box);
+}
+
 // N-tile width.  160 divides every channel count of the UNet (320 .. 2560) without padding and is the default for
 // those; the 256-wide tile (the most efficient tcgen05 shape: one A tile feeds 256 output columns) wins once the K loop
 // dominates the tile - measured with scripts/bench_bn.py on B200 (profiles/r02_splitk.md): linear GEMMs without a
@@ -987,9 +1004,6 @@ static int pick_bn(int N, int geglu, int bn_hint, int K, bool residual, bool con
   if (geglu) return 256;
   if (bn_hint == 64 || bn_hint == 128 || bn_hint == 160 || bn_hint == 256) return bn_hint;
   if (N % 160 == 0) {
-#ifdef AF_BN160_ONLY   // A/B builds (scripts/build_alt.sh): the round-1 rule
-    return 160;
-#endif
     if (conv) return (N % 256 == 0 && N >= 1024 && m_tiles >= 32) ? 256 : 160;
     if (K >= 2560) return 256;
     if (!residual && N >= 1280 && K >= 640) return 256;
@@ -1002,80 +1016,66 @@ static int pick_bn(int N, int geglu, int bn_hint, int K, bool residual, bool con
   return 160;
 }
 
-static int fill_epilogue(GemmParams& p, const af_epilogue* ep, long long default_ldo) {
-  p.bias = ep->bias;
-  p.rowbias = ep->rowbias;
-  p.rows_per_group = ep->rows_per_group > 0 ? ep->rows_per_group : 1;
-  p.ld_rowbias = ep->ld_rowbias > 0 ? ep->ld_rowbias : p.N;
-  p.residual = ep->residual;
-  p.ldr = ep->ldr > 0 ? ep->ldr : default_ldo;
-  p.out = ep->out;
-  p.ldo = ep->ldo > 0 ? ep->ldo : default_ldo;
-  p.out_bf16 = ep->out_dtype == AF_DTYPE_BF16;
-  p.geglu = ep->geglu;
-  p.gn_stats = ep->gn_stats;
-  p.act = ep->act;
+// Epilogue options: the checks that need no buffer, and the row pitches (default_ldo: the output width; p.N is set).
+static int plan_epilogue(GemmParams& p, const af_epilogue* ep, long long default_ldo) {
   AF_CHECK_ARG(ep->act == 0 || (ep->act == 1 && !ep->geglu), "epilogue: act %d unsupported", ep->act);
-  AF_CHECK_ARG(!ep->gn_stats || (!ep->geglu && (reinterpret_cast<uintptr_t>(ep->gn_stats) & 15) == 0),
-               "epilogue: gn_stats needs the generic epilogue and a 16-byte aligned buffer");
-  AF_CHECK_ARG(ep->out != nullptr, "epilogue: out is null");
+  AF_CHECK_ARG(!ep->gn_stats || !ep->geglu, "epilogue: gn_stats needs the generic epilogue");
   AF_CHECK_ARG(ep->out_dtype == AF_DTYPE_BF16 || ep->out_dtype == AF_DTYPE_F32, "epilogue: bad out dtype %d",
                ep->out_dtype);
   AF_CHECK_ARG(!ep->geglu || ep->out_dtype == AF_DTYPE_BF16, "geglu epilogue writes bf16 only");
   AF_CHECK_ARG(!ep->geglu || (!ep->residual && !ep->rowbias), "geglu epilogue: residual / rowbias unsupported");
-  AF_CHECK_ARG((reinterpret_cast<uintptr_t>(ep->out) & 15) == 0, "epilogue: out not 16B aligned");
-  {
-    const long long lim = 1ll << 31, rows = p.M;
-    const long long groups = ep->rows_per_group > 0 ? rows / p.rows_per_group + 1 : 4096;  // conv: one group per image
-    AF_CHECK_ARG(rows * p.ldo < lim && rows * p.ldr < lim && (!p.rowbias || groups * p.ld_rowbias < lim),
-                 "epilogue: output / residual / rowbias larger than 2^31 elements");
-  }
+  p.rows_per_group = ep->rows_per_group > 0 ? ep->rows_per_group : 1;
+  p.ld_rowbias = ep->ld_rowbias > 0 ? ep->ld_rowbias : p.N;
+  p.ldr = ep->ldr > 0 ? ep->ldr : default_ldo;
+  p.ldo = ep->ldo > 0 ? ep->ldo : default_ldo;
+  p.out_bf16 = ep->out_dtype == AF_DTYPE_BF16;
+  p.geglu = ep->geglu;
+  p.act = ep->act;
   AF_CHECK_ARG(p.ldo % 8 == 0 && p.ldr % 4 == 0 && p.ld_rowbias % 4 == 0, "epilogue: ldo %lld / ldr %lld / ld_rowbias %lld misaligned", p.ldo, p.ldr, p.ld_rowbias);
   return 0;
 }
 
-}  // namespace af
+// The caller's epilogue buffers, after planning: the extent check needs the row pitches plan_epilogue chose.
+static int fill_epilogue_buffers(GemmParams& p, const af_epilogue* ep) {
+  AF_CHECK_ARG(ep->out != nullptr, "epilogue: out is null");
+  AF_CHECK_ARG((reinterpret_cast<uintptr_t>(ep->out) & 15) == 0, "epilogue: out not 16B aligned");
+  AF_CHECK_ARG((reinterpret_cast<uintptr_t>(ep->gn_stats) & 15) == 0, "epilogue: gn_stats not 16B aligned");
+  const long long lim = 1ll << 31, rows = p.M;
+  const long long groups = ep->rows_per_group > 0 ? rows / p.rows_per_group + 1 : 4096;  // conv: one group per image
+  AF_CHECK_ARG(rows * p.ldo < lim && rows * p.ldr < lim && (!ep->rowbias || groups * p.ld_rowbias < lim),
+               "epilogue: output / residual / rowbias larger than 2^31 elements");
+  p.bias = ep->bias;
+  p.rowbias = ep->rowbias;
+  p.residual = ep->residual;
+  p.out = ep->out;
+  p.gn_stats = ep->gn_stats;
+  p.trace = ep->trace;
+  return 0;
+}
 
-using namespace af;
+// Tile width, CTA pairs, epilogue form and split-K, once the operand geometry in p is set (K: the contraction length).
+// Every convolution mode, the VAE encoder's amode 3 included, takes the convolution rules of pick_bn and want_pair.
+static void plan_schedule(GemmParams& p, GemmPlan& s, const af_epilogue* ep, int bn_hint, int K) {
+  const bool conv = p.amode != 0, residual = ep->residual != nullptr;
+  s.bn = pick_bn(p.N, p.geglu, bn_hint, K, residual, conv, p.m_tiles);
+  s.pair = want_pair(ep->pair_mode, p.m_tiles, s.bn, conv);
+  p.n_tiles = (p.N + s.bn - 1) / s.bn;
+  p.wide = p.out_bf16 && !p.geglu && !residual && (s.bn == 128 || s.bn == 256);
+  // epilogue slots per warp: 3 (two residual chunks in flight) for the memory-bound linear GEMMs with a residual; 1 for
+  // the K-deep convolutions (their epilogue has slack) and for 256-wide tiles, where the shared memory goes to the
+  // operand ring; 2 for the GEGLU epilogue and everything else
+  s.slots = p.geglu ? 2 : (conv || s.bn == 256) ? 1 : residual ? 3 : 2;
+  plan_split(p, s.bn, s.pair, ep);
+}
 
-extern "C" int af_gemm_bf16(const void* A0, long long lda0, int K0, const void* A1, long long lda1, int K1,
-                            const void* Wt, int M, int N, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
-  AF_CHECK_ARG(A0 && Wt && ep, "af_gemm_bf16: null pointer");
+// Linear / 1x1 GEMM: D[M, N] over the K0 + K1 columns of [A0 | A1].
+static int plan_linear(GemmParams& p, GemmPlan& s, int M, int N, int K0, int K1, const af_epilogue* ep, int bn_hint) {
   AF_CHECK_ARG(M > 0 && N > 0 && K0 > 0 && K1 >= 0, "af_gemm_bf16: bad sizes M=%d N=%d K0=%d K1=%d", M, N, K0, K1);
   AF_CHECK_ARG(N % 8 == 0, "af_gemm_bf16: N=%d must be a multiple of 8", N);
   AF_CHECK_ARG(K1 == 0 || K0 % 64 == 0, "af_gemm_bf16: K0=%d must be a multiple of 64 for a dual-source A", K0);
-  AF_CHECK_ARG((K0 + K1) % 8 == 0 && lda0 % 8 == 0 && (K1 == 0 || lda1 % 8 == 0),
-               "af_gemm_bf16: K / lda must be multiples of 8 (16-byte TMA strides)");
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.trace = ep->trace;
-  const int K = K0 + K1;
-  const int bn = pick_bn(N, ep->geglu, bn_hint, K, ep->residual != nullptr, false, (M + 127) / 128);
-  const bool pair = want_pair(ep->pair_mode, (M + 127) / 128, (N + bn - 1) / bn, bn, 0);
+  AF_CHECK_ARG((K0 + K1) % 8 == 0, "af_gemm_bf16: K / lda must be multiples of 8 (16-byte TMA strides)");
   AF_CHECK_ARG(!ep->geglu || N % 256 == 0, "geglu: packed N=%d must be a multiple of 256", N);
-  {
-    uint64_t dims[2] = {static_cast<uint64_t>(K0), static_cast<uint64_t>(M)};
-    uint64_t str[1] = {static_cast<uint64_t>(lda0) * 2};
-    uint32_t box[2] = {64, 128};
-    int rc = make_tmap_bf16(&p.tmA0, A0, 2, dims, str, box);
-    if (rc) return rc;
-    p.tmA1 = p.tmA0;
-  }
-  if (K1 > 0) {
-    AF_CHECK_ARG(A1 != nullptr, "af_gemm_bf16: A1 null with K1=%d", K1);
-    uint64_t dims[2] = {static_cast<uint64_t>(K1), static_cast<uint64_t>(M)};
-    uint64_t str[1] = {static_cast<uint64_t>(lda1) * 2};
-    uint32_t box[2] = {64, 128};
-    int rc = make_tmap_bf16(&p.tmA1, A1, 2, dims, str, box);
-    if (rc) return rc;
-  }
-  {
-    uint64_t dims[2] = {static_cast<uint64_t>(K), static_cast<uint64_t>(N)};
-    uint64_t str[1] = {static_cast<uint64_t>(K) * 2};
-    uint32_t box[2] = {64, static_cast<uint32_t>(pair ? bn / 2 : bn)};
-    int rc = make_tmap_bf16(&p.tmB, Wt, 2, dims, str, box);
-    if (rc) return rc;
-  }
+  memset(&p, 0, sizeof(p));
   p.M = M;
   p.N = N;
   p.num_kb = (K0 + 63) / 64 + (K1 + 63) / 64;
@@ -1083,16 +1083,10 @@ extern "C" int af_gemm_bf16(const void* A0, long long lda0, int K0, const void* 
   p.kb_split = (K0 + 63) / 64;
   p.amode = 0;
   p.m_tiles = (M + 127) / 128;
-  p.n_tiles = (N + bn - 1) / bn;
-  int rc = fill_epilogue(p, ep, ep->geglu ? N / 2 : N);
+  int rc = plan_epilogue(p, ep, ep->geglu ? N / 2 : N);
   if (rc) return rc;
-#ifndef AF_GEMM_NO_WIDE
-  p.wide = p.out_bf16 && !p.geglu && p.residual == nullptr && (bn == 128 || bn == 256);
-#endif
-  rc = make_epilogue_maps(p, ep->geglu ? N / 2 : N, false);
-  if (rc) return rc;
-  plan_split(p, bn, pair, ep);
-  return dispatch_gemm(bn, p, pair, stream);
+  plan_schedule(p, s, ep, bn_hint, K0 + K1);
+  return 0;
 }
 
 // output-pixel box of one 128-row conv tile: bw = largest power of two <= min(64, next_pow2(Wo)); rows / images
@@ -1105,6 +1099,72 @@ static void conv_tile_box(int Ho, int Wo, int* bw_, int* bh_, int* nb_) {
   *bw_ = bw; *bh_ = bh; *nb_ = 128 / (bw * bh);
 }
 
+// 3x3 convolution over [X0 | X1]: pad 1 with stride 1 (amode 1) or 2 (amode 2), or, with pad01, stride 2 after
+// F.pad(0,1,0,1) (amode 3).  who: the entry point the messages name.
+static int plan_conv(GemmParams& p, GemmPlan& s, const char* who, int C0, int C1, int B, int H, int W, int Cout,
+                     int stride, bool pad01, const af_epilogue* ep, int bn_hint) {
+  AF_CHECK_ARG(stride == 1 || stride == 2, "%s: stride %d", who, stride);
+  AF_CHECK_ARG(B > 0 && H > 0 && W > 0, "%s: bad sizes B=%d H=%d W=%d", who, B, H, W);
+  AF_CHECK_ARG(C0 > 0 && C0 % 64 == 0 && C1 >= 0 && C1 % 64 == 0, "%s: C0=%d C1=%d must each be a multiple of 64", who,
+               C0, C1);
+  AF_CHECK_ARG(Cout > 0 && Cout % 8 == 0, "%s: Cout=%d must be a multiple of 8", who, Cout);
+  AF_CHECK_ARG(stride == 1 || (C1 == 0 && H % 2 == 0 && W % 2 == 0),
+               "%s: stride 2 needs a single source and even H=%d W=%d", who, H, W);
+  AF_CHECK_ARG(!ep->geglu, "%s: geglu epilogue unsupported", who);
+  const int Cin = C0 + C1, Ho = H / stride, Wo = W / stride;
+  memset(&p, 0, sizeof(p));
+  p.amode = pad01 ? 3 : stride;
+  p.B = B; p.H = Ho; p.W = Wo; p.C0 = C0;
+  conv_tile_box(Ho, Wo, &p.bw, &p.bh, &p.nb);
+  p.tiles_w = (Wo + p.bw - 1) / p.bw;
+  p.tiles_h = (Ho + p.bh - 1) / p.bh;
+  p.M = B * Ho * Wo;
+  p.N = Cout;
+  p.cpb = Cin / 64;
+  p.kb_split = C0 / 64;
+  p.num_kb = 9 * p.cpb;
+  p.m_tiles = p.tiles_w * p.tiles_h * ((B + p.nb - 1) / p.nb);
+  int rc = plan_epilogue(p, ep, Cout);
+  if (rc) return rc;
+  if (ep->rowbias && ep->rows_per_group <= 0) p.rows_per_group = Ho * Wo;
+  if (ep->gn_stats) {
+    p.gn_slots = af_conv3x3_gn_slots(Ho, Wo);
+    AF_CHECK_ARG(p.gn_slots > 0, "%s: gn_stats unsupported for %dx%d outputs (fewer than 32 pixels per tile row group)", who, Ho, Wo);
+  }
+  plan_schedule(p, s, ep, bn_hint, 9 * Cin);
+  return 0;
+}
+
+}  // namespace af
+
+using namespace af;
+
+extern "C" int af_gemm_bf16(const void* A0, long long lda0, int K0, const void* A1, long long lda1, int K1,
+                            const void* Wt, int M, int N, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
+  AF_CHECK_ARG(A0 && Wt && ep, "af_gemm_bf16: null pointer");
+  GemmParams p;
+  GemmPlan s;
+  int rc = plan_linear(p, s, M, N, K0, K1, ep, bn_hint);
+  if (rc) return rc;
+  AF_CHECK_ARG(lda0 % 8 == 0 && (K1 == 0 || lda1 % 8 == 0),
+               "af_gemm_bf16: K / lda must be multiples of 8 (16-byte TMA strides)");
+  AF_CHECK_ARG(K1 == 0 || A1 != nullptr, "af_gemm_bf16: A1 null with K1=%d", K1);
+  rc = fill_epilogue_buffers(p, ep);
+  if (rc) return rc;
+  rc = make_operand_map(&p.tmA0, A0, K0, M, lda0, 128);
+  if (rc) return rc;
+  p.tmA1 = p.tmA0;
+  if (K1 > 0) {
+    rc = make_operand_map(&p.tmA1, A1, K1, M, lda1, 128);
+    if (rc) return rc;
+  }
+  rc = make_operand_map(&p.tmB, Wt, K0 + K1, N, K0 + K1, s.pair ? s.bn / 2 : s.bn);
+  if (rc) return rc;
+  rc = make_epilogue_maps(p, p.geglu ? N / 2 : N, false);
+  if (rc) return rc;
+  return dispatch_gemm(p, s, stream);
+}
+
 extern "C" int af_conv3x3_gn_slots(int Ho, int Wo) {
   int bw, bh, nb;
   conv_tile_box(Ho, Wo, &bw, &bh, &nb);
@@ -1112,117 +1172,71 @@ extern "C" int af_conv3x3_gn_slots(int Ho, int Wo) {
   return ((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh) * (bw * bh / 32);
 }
 
-// amode 1: stride 1, pad 1 (two sources); 2: stride 2, pad 1; 3: stride 2 after F.pad(0,1,0,1).  The entry points have
-// checked the arguments their mode needs.
-static int conv3x3_launch(const char* who, const void* X0, int C0, const void* X1, int C1, const void* Wt, int B, int H,
-                          int W, int Cout, int amode, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
-  const int stride = amode == 1 ? 1 : 2;
+// The convolution entry points; pad01: af_conv3x3_down01_bf16 (stride 2).
+static int conv3x3_launch(const char* who, bool pad01, const void* X0, int C0, const void* X1, int C1, const void* Wt,
+                          int B, int H, int W, int Cout, int stride, const af_epilogue* ep, int bn_hint,
+                          cudaStream_t stream) {
+  AF_CHECK_ARG(X0 && Wt && ep, "%s: null pointer", who);
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.trace = ep->trace;
-  const int Cin = C0 + C1;
-  const int Ho = stride == 1 ? H : H / 2, Wo = stride == 1 ? W : W / 2;
-  int bw, bh, nb;
-  conv_tile_box(Ho, Wo, &bw, &bh, &nb);
-  const int bn = pick_bn(Cout, 0, bn_hint, 9 * Cin, ep->residual != nullptr, true,
-                         ((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh) * ((B + nb - 1) / nb));
-  const bool pair = want_pair(ep->pair_mode, ((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh) * ((B + nb - 1) / nb), (Cout + bn - 1) / bn, bn, 1);
-  p.bw = bw; p.bh = bh; p.nb = nb;
-  p.tiles_w = (Wo + bw - 1) / bw;
-  p.tiles_h = (Ho + bh - 1) / bh;
-  p.B = B; p.H = Ho; p.W = Wo; p.C0 = C0;
+  GemmPlan s;
+  int rc = plan_conv(p, s, who, C0, C1, B, H, W, Cout, stride, pad01, ep, bn_hint);
+  if (rc) return rc;
+  AF_CHECK_ARG(C1 == 0 || X1 != nullptr, "%s: X1 null with C1=%d", who, C1);
+  rc = fill_epilogue_buffers(p, ep);
+  if (rc) return rc;
   const uint64_t es = 2;
+  const uint32_t bw = p.bw, bh = p.bh, nb = p.nb;
   if (stride == 1) {
-    uint32_t box[4] = {64, static_cast<uint32_t>(bw), static_cast<uint32_t>(bh), static_cast<uint32_t>(nb)};
+    uint32_t box[4] = {64, bw, bh, nb};
     {
       uint64_t dims[4] = {static_cast<uint64_t>(C0), static_cast<uint64_t>(W), static_cast<uint64_t>(H), static_cast<uint64_t>(B)};
       uint64_t str[3] = {C0 * es, static_cast<uint64_t>(W) * C0 * es, static_cast<uint64_t>(H) * W * C0 * es};
-      int rc = make_tmap_bf16(&p.tmA0, X0, 4, dims, str, box);
+      rc = make_tmap_bf16(&p.tmA0, X0, 4, dims, str, box);
       if (rc) return rc;
       p.tmA1 = p.tmA0;
     }
     if (C1 > 0) {
-      AF_CHECK_ARG(X1 != nullptr, "af_conv3x3_bf16: X1 null with C1=%d", C1);
       uint64_t dims[4] = {static_cast<uint64_t>(C1), static_cast<uint64_t>(W), static_cast<uint64_t>(H), static_cast<uint64_t>(B)};
       uint64_t str[3] = {C1 * es, static_cast<uint64_t>(W) * C1 * es, static_cast<uint64_t>(H) * W * C1 * es};
-      int rc = make_tmap_bf16(&p.tmA1, X1, 4, dims, str, box);
+      rc = make_tmap_bf16(&p.tmA1, X1, 4, dims, str, box);
       if (rc) return rc;
     }
-    p.amode = 1;
   } else {
-    uint32_t box[5] = {64, static_cast<uint32_t>(bw), 1, static_cast<uint32_t>(bh), static_cast<uint32_t>(nb)};
+    uint32_t box[5] = {64, bw, 1, bh, nb};
     uint64_t dims[5] = {static_cast<uint64_t>(2 * C0), static_cast<uint64_t>(W / 2), 2, static_cast<uint64_t>(H / 2),
                         static_cast<uint64_t>(B)};
     uint64_t str[4] = {2 * C0 * es, static_cast<uint64_t>(W) * C0 * es, 2 * static_cast<uint64_t>(W) * C0 * es,
                        static_cast<uint64_t>(H) * W * C0 * es};
-    int rc = make_tmap_bf16(&p.tmA0, X0, 5, dims, str, box);
+    rc = make_tmap_bf16(&p.tmA0, X0, 5, dims, str, box);
     if (rc) return rc;
     p.tmA1 = p.tmA0;
-    p.amode = amode;
   }
-  {
-    const uint64_t K = 9ull * Cin;
-    uint64_t dims[2] = {K, static_cast<uint64_t>(Cout)};
-    uint64_t str[1] = {K * 2};
-    uint32_t box[2] = {64, static_cast<uint32_t>(pair ? bn / 2 : bn)};
-    int rc = make_tmap_bf16(&p.tmB, Wt, 2, dims, str, box);
-    if (rc) return rc;
-  }
-  p.M = B * Ho * Wo;
-  p.N = Cout;
-  p.cpb = Cin / 64;
-  p.kb_split = C0 / 64;
-  p.num_kb = 9 * p.cpb;
-  p.m_tiles = p.tiles_w * p.tiles_h * ((B + nb - 1) / nb);
-  p.n_tiles = (Cout + bn - 1) / bn;
-  int rc = fill_epilogue(p, ep, Cout);
+  rc = make_operand_map(&p.tmB, Wt, 9ll * (C0 + C1), Cout, 9ll * (C0 + C1), s.pair ? s.bn / 2 : s.bn);
   if (rc) return rc;
-  if (p.rowbias && ep->rows_per_group <= 0) p.rows_per_group = Ho * Wo;
-  if (p.gn_stats) {
-    p.gn_slots = af_conv3x3_gn_slots(Ho, Wo);
-    AF_CHECK_ARG(p.gn_slots > 0, "%s: gn_stats unsupported for %dx%d outputs (fewer than 32 pixels per tile row group)", who, Ho, Wo);
-  }
-#ifndef AF_GEMM_NO_WIDE
-  p.wide = p.out_bf16 && p.residual == nullptr && (bn == 128 || bn == 256);
-#endif
   rc = make_epilogue_maps(p, Cout, true);
   if (rc) return rc;
-  plan_split(p, bn, pair, ep);
-  return dispatch_gemm(bn, p, pair, stream);
+  return dispatch_gemm(p, s, stream);
 }
 
 extern "C" int af_conv3x3_bf16(const void* X0, int C0, const void* X1, int C1, const void* Wt, int B, int H, int W,
                                int Cout, int stride, const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
-  AF_CHECK_ARG(X0 && Wt && ep, "af_conv3x3_bf16: null pointer");
-  AF_CHECK_ARG(stride == 1 || stride == 2, "af_conv3x3_bf16: stride %d", stride);
-  AF_CHECK_ARG(C0 > 0 && C0 % 64 == 0 && C1 >= 0 && C1 % 64 == 0, "af_conv3x3_bf16: C0=%d C1=%d must be multiples of 64",
-               C0, C1);
-  AF_CHECK_ARG(Cout % 8 == 0, "af_conv3x3_bf16: Cout=%d must be a multiple of 8", Cout);
-  AF_CHECK_ARG(stride == 1 || (C1 == 0 && H % 2 == 0 && W % 2 == 0), "af_conv3x3_bf16: stride 2 needs single source, even H/W");
-  AF_CHECK_ARG(!ep->geglu, "af_conv3x3_bf16: geglu epilogue unsupported");
-  return conv3x3_launch("af_conv3x3_bf16", X0, C0, X1, C1, Wt, B, H, W, Cout, stride, ep, bn_hint, stream);
+  return conv3x3_launch("af_conv3x3_bf16", false, X0, C0, X1, C1, Wt, B, H, W, Cout, stride, ep, bn_hint, stream);
 }
 
 extern "C" int af_conv3x3_down01_bf16(const void* X, int C, const void* Wt, int B, int H, int W, int Cout,
                                       const af_epilogue* ep, int bn_hint, cudaStream_t stream) {
-  AF_CHECK_ARG(X && Wt && ep, "af_conv3x3_down01_bf16: null pointer");
-  AF_CHECK_ARG(B > 0 && H > 0 && W > 0, "af_conv3x3_down01_bf16: bad sizes B=%d H=%d W=%d", B, H, W);
-  AF_CHECK_ARG(C > 0 && C % 64 == 0, "af_conv3x3_down01_bf16: C=%d must be a multiple of 64", C);
-  AF_CHECK_ARG(Cout > 0 && Cout % 8 == 0, "af_conv3x3_down01_bf16: Cout=%d must be a multiple of 8", Cout);
-  AF_CHECK_ARG(H % 2 == 0 && W % 2 == 0, "af_conv3x3_down01_bf16: H=%d W=%d must be even", H, W);
-  AF_CHECK_ARG(!ep->geglu, "af_conv3x3_down01_bf16: geglu epilogue unsupported");
-  return conv3x3_launch("af_conv3x3_down01_bf16", X, C, nullptr, 0, Wt, B, H, W, Cout, 3, ep, bn_hint, stream);
+  return conv3x3_launch("af_conv3x3_down01_bf16", true, X, C, nullptr, 0, Wt, B, H, W, Cout, 2, ep, bn_hint, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
 // Schedule introspection (no launch, no device needed: 148 SMs are assumed without one): the tile width, tile schedule
-// and split-K plan af_gemm_bf16 / af_conv3x3_bf16 would use - the same pick_bn / want_pair / plan_split calls.
+// and split-K plan af_gemm_bf16 / af_conv3x3_bf16 would use - the same planners, so the same argument checks.
 // out[0] = N-tile width, out[1] = 1 if CTA pairs, out[2] = K ranges per remainder tile (1 = whole tiles),
 // out[3] = work units, out[4] = whole-K tiles before the split ones, out[5] = 1 if 64-column bf16 epilogue items.
 // ---------------------------------------------------------------------------------------------
-static void fill_plan(const GemmParams& p, int bn, bool pair, int* out) {
-  out[0] = bn;
-  out[1] = pair ? 1 : 0;
+static void fill_plan(const GemmParams& p, const GemmPlan& s, int* out) {
+  out[0] = s.bn;
+  out[1] = s.pair ? 1 : 0;
   out[2] = p.split;
   out[3] = p.num_units;
   out[4] = p.dp_tiles;
@@ -1230,49 +1244,22 @@ static void fill_plan(const GemmParams& p, int bn, bool pair, int* out) {
 }
 
 extern "C" int af_gemm_plan(int M, int N, int K, const af_epilogue* ep, int bn_hint, int* out) {
-  AF_CHECK_ARG(ep && out && M > 0 && N > 0 && K > 0, "af_gemm_plan: bad arguments");
+  AF_CHECK_ARG(ep && out, "af_gemm_plan: null pointer");
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  const int bn = pick_bn(N, ep->geglu, bn_hint, K, ep->residual != nullptr, false, (M + 127) / 128);
-  const bool pair = want_pair(ep->pair_mode, (M + 127) / 128, (N + bn - 1) / bn, bn, 0);
-  p.num_kb = (K + 63) / 64;
-  p.m_tiles = (M + 127) / 128;
-  p.n_tiles = (N + bn - 1) / bn;
-  p.geglu = ep->geglu;
-  p.residual = ep->residual;
-  p.out_bf16 = ep->out_dtype == AF_DTYPE_BF16;
-#ifndef AF_GEMM_NO_WIDE
-  p.wide = p.out_bf16 && !p.geglu && p.residual == nullptr && (bn == 128 || bn == 256);
-#endif
-  plan_split(p, bn, pair, ep);
-  fill_plan(p, bn, pair, out);
+  GemmPlan s;
+  int rc = plan_linear(p, s, M, N, K, 0, ep, bn_hint);
+  if (rc) return rc;
+  fill_plan(p, s, out);
   return 0;
 }
 
 extern "C" int af_conv3x3_plan(int C0, int C1, int B, int H, int W, int Cout, int stride, const af_epilogue* ep,
                                int bn_hint, int* out) {
-  AF_CHECK_ARG(ep && out && B > 0 && H > 0 && W > 0 && Cout > 0 && C0 > 0 && (stride == 1 || stride == 2),
-               "af_conv3x3_plan: bad arguments");
+  AF_CHECK_ARG(ep && out, "af_conv3x3_plan: null pointer");
   GemmParams p;
-  memset(&p, 0, sizeof(p));
-  const int Cin = C0 + C1;
-  const int Ho = stride == 1 ? H : H / 2, Wo = stride == 1 ? W : W / 2;
-  int bw, bh, nb;
-  conv_tile_box(Ho, Wo, &bw, &bh, &nb);
-  const int m_tiles = ((Wo + bw - 1) / bw) * ((Ho + bh - 1) / bh) * ((B + nb - 1) / nb);
-  const int bn = pick_bn(Cout, 0, bn_hint, 9 * Cin, ep->residual != nullptr, true, m_tiles);
-  const bool pair = want_pair(ep->pair_mode, m_tiles, (Cout + bn - 1) / bn, bn, 1);
-  p.amode = stride == 1 ? 1 : 2;
-  p.num_kb = 9 * (Cin / 64);
-  p.m_tiles = m_tiles;
-  p.n_tiles = (Cout + bn - 1) / bn;
-  p.residual = ep->residual;
-  p.out_bf16 = ep->out_dtype == AF_DTYPE_BF16;
-#ifndef AF_GEMM_NO_WIDE
-  p.wide = p.out_bf16 && p.residual == nullptr && (bn == 128 || bn == 256);
-#endif
-  plan_split(p, bn, pair, ep);
-  fill_plan(p, bn, pair, out);
+  GemmPlan s;
+  int rc = plan_conv(p, s, "af_conv3x3_bf16", C0, C1, B, H, W, Cout, stride, false, ep, bn_hint);
+  if (rc) return rc;
+  fill_plan(p, s, out);
   return 0;
 }
-

@@ -88,7 +88,9 @@ int af_gemm_bf16(const void* A0, long long lda0, int K0, const void* A1, long lo
                  int M, int N, const af_epilogue* ep, int bn_hint, af_stream_t stream);
 
 /* Schedule introspection (no launch, no device needed - 148 SMs are assumed without one): what af_gemm_bf16 /
- * af_conv3x3_bf16 would choose for these sizes and this epilogue.  out[0] = N-tile width, out[1] = 1 if CTA pairs,
+ * af_conv3x3_bf16 would choose for these sizes and this epilogue.  They apply the launch's own checks of sizes and
+ * epilogue options (not those of pointers, operand pitches and buffer extents): sizes or options the launch refuses
+ * return its negative code and message (af_last_error).  out[0] = N-tile width, out[1] = 1 if CTA pairs,
  * out[2] = K ranges per remainder tile (1 = whole tiles only), out[3] = work units, out[4] = whole-K tiles in front of the
  * split ones, out[5] = 1 if the bf16 output leaves in 64-column epilogue items.  Host-side logic tests use these. */
 int af_gemm_plan(int M, int N, int K, const af_epilogue* ep, int bn_hint, int* out);

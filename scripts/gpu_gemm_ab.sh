@@ -1,3 +1,2 @@
-# GEMM / conv kernel tests, then the sampler A/B against the alternative builds in adaprompt_b200/_alt
+# GEMM / conv kernel tests
 timeout 900 python -m pytest tests/test_kernels_gpu.py tests/test_unet_gpu.py -x -q -m gpu -p no:cacheprovider 2>&1 | tail -4
-bash scripts/gpu_alt_ab.sh

@@ -150,3 +150,32 @@ def test_gemm_and_conv_schedule_plans():
     assert (p["bn"], p["wide"]) == (256, 1)
     assert gemm(65536, 320, 320, bf16=True)["wide"] == 0                        # 160-wide tiles keep 32-column items
     assert gemm(4096, 10240, 1280, geglu=True, bf16=True)["bn"] == 256
+
+
+@pytest.mark.parametrize("call,message", [
+    (("gemm", 4096, 324, 320, {}), b"af_gemm_bf16: N=324 must be a multiple of 8"),
+    (("gemm", 4096, 10240, 1280, dict(geglu=1, residual=16)), b"geglu epilogue: residual / rowbias unsupported"),
+    (("gemm", 4096, 10112, 1280, dict(geglu=1)), b"geglu: packed N=10112 must be a multiple of 256"),
+    (("gemm", 4096, 10240, 1280, dict(geglu=1, act=1)), b"epilogue: act 1 unsupported"),
+    (("conv", 100, 0, 16, 32, 32, 320, 1), b"af_conv3x3_bf16: C0=100 C1=0 must each be a multiple of 64"),
+    (("conv", 320, 0, 16, 32, 32, 320, 3), b"af_conv3x3_bf16: stride 3"),
+    (("conv", 320, 0, 16, 33, 32, 320, 2), b"af_conv3x3_bf16: stride 2 needs a single source and even H=33 W=32"),
+], ids=["gemm-N%8", "geglu-residual", "geglu-N%256", "geglu-act", "conv-C0=100", "conv-stride3", "conv-s2-oddH"])
+def test_schedule_plans_refuse_what_the_launch_refuses(call, message):
+    """af_gemm_plan / af_conv3x3_plan run the argument checks of af_gemm_bf16 / af_conv3x3_bf16: sizes or epilogue
+    options the launch refuses get no schedule, but the launch's negative code and message."""
+    import ctypes
+    from adaprompt_b200 import _lib
+    lib = _lib.load()
+    out = (ctypes.c_int * 6)()
+    e = _lib.AfEpilogue()
+    e.out_dtype = 1                     # bf16, as GEGLU needs
+    if call[0] == "gemm":
+        M, N, K, fields = call[1:]
+        for k, v in fields.items():
+            setattr(e, k, v)            # residual: only tested for NULL by the planner
+        rc = lib.af_gemm_plan(M, N, K, ctypes.byref(e), 0, out)
+    else:
+        rc = lib.af_conv3x3_plan(*call[1:], ctypes.byref(e), 0, out)
+    assert rc < 0
+    assert lib.af_last_error() == message
