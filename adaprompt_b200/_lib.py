@@ -111,6 +111,11 @@ SIGNATURES = {
     "af_attention_bf16_lse": (c_int, [c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_longlong, c_int,
                                       c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "af_bgemm_bf16": (c_int, [POINTER(AfBgemm), c_void_p]),
+    "af_bgemm_masked_bf16": (c_int, [POINTER(AfBgemm), c_void_p, c_longlong, c_longlong, c_void_p]),
+    "af_attention_bwd_masked_bf16": (c_int, [c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_longlong, c_void_p,
+                                             c_longlong, c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_longlong,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_longlong,
+                                             c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_void_p]),
     "af_groupnorm_bwd_workspace_floats": (c_size_t, [c_int, c_int, c_int]),
     "af_groupnorm_bwd": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -183,6 +188,7 @@ KERNELS_PER_CALL = {
     "af_geglu_bwd": 1, "af_quick_gelu": 1, "af_rowdot_heads": 1, "af_attention_small_bwd": 1, "af_conv_out_dgrad": 1,
     "af_sumpool2x2": 1, "af_zero_insert2x": 1, "af_transpose_to_bf16": 1, "af_prodigy_moments": 1, "af_prodigy_apply": 1,
     "af_softmax_rows": 1, "af_channel_mix4": 1, "af_conv3x3_down01_bf16": 1, "af_vae_posterior": 1,
+    "af_bgemm_masked_bf16": 1, "af_attention_bwd_masked_bf16": 2,
 }
 
 

@@ -43,6 +43,7 @@ struct AttnBwdParams {
   __nv_bfloat16* out1;       // dK [B*N, ld1] (DKV only)
   long long ld0, ld1;
   int B, heads, N, d;
+  const uint8_t* kmask;      // [B][N] key mask, 1 = attend (masked instantiations only)
 };
 
 template <int D>
@@ -78,11 +79,21 @@ __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_
                : "memory");
 }
 
-template <int D, bool DKV>
-__global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(const __grid_constant__ AttnBwdParams p) {
+// MASKED: the key mask of attention.py:223-232 (scores of masked keys filled with -finfo.max before the softmax), as the
+// exact derivative of af_attention_bf16_lse with a key mask:
+//   a sample with a kept key:  P_ij = m_j ? exp2(S_ij - lse_i) : 0,   dS_ij = m_j ? ln2 P_ij (dP_ij - delta_i) : 0;
+//   a sample that keeps no key (lse = +inf in every row, the forward output is the mean of V):  P_ij = 1 / N, dS = 0.
+// The mask enters through selects only, so whatever masked K / V rows hold never reaches a gradient, and the kept
+// keys take the operation order of the unmasked instantiation (an all-ones mask gives bit-identical results).
+//   dQ kernel:     the 64 mask bytes of key block c ride in the stage, next to where the DKV kernel keeps lse / delta.
+//   dK/dV kernel:  the mask is a per-row scalar; the row's own lse (queries and keys are the same tokens) tells whether
+//                  the sample keeps no key.  Then P^T is 1 in every entry and the dV accumulator is scaled by 1/N.
+template <int D, bool DKV, bool MASKED>
+__device__ __forceinline__ void attention_bwd_body(const AttnBwdParams& p) {
   using C = BwdCfg<D>;
   using S = BwdSmem<D, DKV>;
   constexpr int DP = C::DP, KA = S::KA, NST = C::STAGES;
+  constexpr int kStageTx = S::kStageTx + (MASKED && !DKV ? 64 : 0);
   constexpr uint32_t kTmS = 0, kTmT = 64, kTmA0 = 128, kTmA1 = 128 + DP;
   constexpr uint32_t kTmemCols = (128 + (DKV ? 2 : 1) * DP) <= 256 ? 256 : 512;
   constexpr float kLn2 = 0.69314718055994530942f;
@@ -148,7 +159,7 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
         for (int c = 0; c < n_blocks; ++c) {
           mbar_wait_lean(&st_empty[st], ph ^ 1);
           uint8_t* base = smem + S::kStageOff + st * S::kStageBytes;
-          mbar_arrive_expect_tx(&st_full[st], S::kStageTx);
+          mbar_arrive_expect_tx(&st_full[st], kStageTx);
 #pragma unroll
           for (int a = 0; a < KA; ++a) {
             tma_load_3d(base + a * 64 * 128, &p.tmU, &st_full[st], h * DP + a * 64, c * 64, b);
@@ -161,6 +172,8 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
             uint8_t* vec = base + S::kStageBytes - 1024;
             bulk_load_1d(vec, p.lse + voff, 256, &st_full[st]);
             bulk_load_1d(vec + 256, p.delta + voff, 256, &st_full[st]);
+          } else if (MASKED) {
+            bulk_load_1d(base + S::kStageBytes - 1024, p.kmask + static_cast<size_t>(b) * p.N + c * 64, 64, &st_full[st]);
           }
           if (++st == NST) { st = 0; ph ^= 1; }
         }
@@ -239,6 +252,12 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
       lse_r = __ldg(p.lse + voff);
       dl_r = __ldg(p.delta + voff) * kLn2;
     }
+    bool keep = true, empty = false;      // MASKED && DKV: this key row is attended / its sample keeps no key
+    if (MASKED && DKV) {
+      keep = __ldg(p.kmask + static_cast<size_t>(b) * p.N + row0 + r) != 0;
+      empty = isinf(__ldg(p.lse + (static_cast<size_t>(b) * p.heads + h) * p.N + row0 + r));
+    }
+    const uint32_t p_drop = empty ? pack_bf16x2(1.f, 1.f) : 0u;
     int st = 0;
     for (int c = 0; c < n_blocks; ++c) {
       mbar_wait_lean(a_s_full, c & 1);
@@ -262,9 +281,28 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
           pkp[(e >> 1) + 1] = pack_bf16x2(p2, p3);
           pkg[e >> 1] = pack_bf16x2(p0 * ((tv[e] - d4.x) * kLn2), p1 * ((tv[e + 1] - d4.y) * kLn2));
           pkg[(e >> 1) + 1] = pack_bf16x2(p2 * ((tv[e + 2] - d4.z) * kLn2), p3 * ((tv[e + 3] - d4.w) * kLn2));
+          if (MASKED) {
+            pkp[e >> 1] = keep ? pkp[e >> 1] : p_drop;
+            pkp[(e >> 1) + 1] = keep ? pkp[(e >> 1) + 1] : p_drop;
+            pkg[e >> 1] = keep ? pkg[e >> 1] : 0u;
+            pkg[(e >> 1) + 1] = keep ? pkg[(e >> 1) + 1] : 0u;
+          }
         }
         tile_st32(s_addr, pkp);          // P^T over the head of S
         tile_st32(t_addr, pkg);          // dS^T over the head of T
+      } else if (MASKED) {
+        const uint32_t mvec = smem_base + S::kStageOff + st * S::kStageBytes + S::kStageBytes - 1024;
+#pragma unroll
+        for (int e = 0; e < 64; e += 4) {
+          const uint32_t m4 = __float_as_uint(lds32f(mvec + e));     // mask bytes of keys e .. e+3 (broadcast)
+#pragma unroll
+          for (int u = 0; u < 4; u += 2) {
+            const float p0 = fast_exp2(sv[e + u] - lse_r), p1 = fast_exp2(sv[e + u + 1] - lse_r);
+            const float g0 = p0 * fmaf(tv[e + u], kLn2, -dl_r), g1 = p1 * fmaf(tv[e + u + 1], kLn2, -dl_r);
+            pkg[(e + u) >> 1] = pack_bf16x2((m4 >> (8 * u)) & 0xffu ? g0 : 0.f, (m4 >> (8 * u + 8)) & 0xffu ? g1 : 0.f);
+          }
+        }
+        tile_st32(t_addr, pkg);          // dS over the head of T
       } else {
 #pragma unroll
         for (int e = 0; e < 64; e += 2) {
@@ -283,13 +321,18 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
     mbar_wait_lean(done, 0);
     tc_fence_after();
     const size_t grow = static_cast<size_t>(b) * p.N + row0 + r;
-    auto store_acc = [&](uint32_t tm_col, __nv_bfloat16* out, long long ld, int col0, int ncols) {
+    auto store_acc = [&](uint32_t tm_col, __nv_bfloat16* out, long long ld, int col0, int ncols, bool mean) {
       __nv_bfloat16* orow = out + grow * ld + col0;
+      const float inv_n = 1.f / static_cast<float>(p.N);
 #pragma unroll 1
       for (int cc = 0; cc < DP; cc += 16) {
         uint32_t o[16];
         tmem_ld16(tmem_base + tm_col + lane_off + cc, o);
         tmem_ld_wait();
+        if (MASKED && mean) {            // dV of a sample that keeps no key: (sum_i dO_i) / N
+#pragma unroll
+          for (int i = 0; i < 16; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * inv_n);
+        }
 #pragma unroll
         for (int g = 0; g < 2; ++g) {
           if (cc + g * 8 < ncols) {
@@ -304,10 +347,10 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
       }
     };
     if (DKV) {
-      store_acc(kTmA0, p.out0, p.ld0, h * p.d, p.d);     // dV: d columns
-      store_acc(kTmA1, p.out1, p.ld1, h * DP, DP);       // dK: DP columns (pads are exact zeros)
+      store_acc(kTmA0, p.out0, p.ld0, h * p.d, p.d, empty);     // dV: d columns
+      store_acc(kTmA1, p.out1, p.ld1, h * DP, DP, false);       // dK: DP columns (pads are exact zeros)
     } else {
-      store_acc(kTmA0, p.out0, p.ld0, h * DP, DP);       // dQ
+      store_acc(kTmA0, p.out0, p.ld0, h * DP, DP, false);       // dQ
     }
   }
 
@@ -320,18 +363,27 @@ __global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(con
 }
 
 template <int D, bool DKV>
+__global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_kernel(const __grid_constant__ AttnBwdParams p) {
+  attention_bwd_body<D, DKV, false>(p);
+}
+template <int D, bool DKV>
+__global__ void __launch_bounds__(256, BwdCfg<D>::CTAS) attention_bwd_masked_kernel(const __grid_constant__ AttnBwdParams p) {
+  attention_bwd_body<D, DKV, true>(p);
+}
+
+template <int D, bool DKV, bool MASKED>
 static int launch_bwd(const AttnBwdParams& p, cudaStream_t stream) {
   using S = BwdSmem<D, DKV>;
+  const auto kernel = MASKED ? attention_bwd_masked_kernel<D, DKV> : attention_bwd_kernel<D, DKV>;
   static bool configured = false;
   if (!configured) {
-    AF_CUDA(cudaFuncSetAttribute(attention_bwd_kernel<D, DKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-    AF_CUDA(cudaFuncSetAttribute(attention_bwd_kernel<D, DKV>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared));
+    AF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
+    AF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     configured = true;
   }
   dim3 grid(p.N / 128, p.heads, p.B);
-  attention_bwd_kernel<D, DKV><<<grid, 256, S::kTotal, stream>>>(p);
-  AF_LAUNCH_CHECK("attention_bwd_kernel");
+  kernel<<<grid, 256, S::kTotal, stream>>>(p);
+  AF_LAUNCH_CHECK(MASKED ? "attention_bwd_masked_kernel" : "attention_bwd_kernel");
   return 0;
 }
 
@@ -352,20 +404,15 @@ static int make_t_map(CUtensorMap* m, const void* base, long long ld, int heads,
 
 using namespace af;
 
-extern "C" int af_attention_bwd_bf16(const void* Q, long long ldq, const void* K, long long ldk, const void* Vp,
-                                     long long ldv, const void* dOp, long long lddo, const void* QT, long long ldqt,
-                                     const void* KT, long long ldkt, const void* dOT, long long lddot, const float* lse,
-                                     const float* delta, void* dQ, long long lddq, void* dK, long long lddk, void* dV,
-                                     long long lddv, int B, int heads, int N, int d, cudaStream_t stream) {
-  AF_CHECK_ARG(Q && K && Vp && dOp && QT && KT && dOT && lse && delta && dQ && dK && dV, "af_attention_bwd_bf16: null pointer");
-  AF_CHECK_ARG(d == 40 || d == 80, "af_attention_bwd_bf16: head dim %d unsupported (40 / 80)", d);
-  AF_CHECK_ARG(B > 0 && heads > 0 && N >= 128 && N % 128 == 0, "af_attention_bwd_bf16: N=%d must be a positive multiple of 128", N);
+namespace af {
+
+static int attention_bwd(const void* Q, long long ldq, const void* K, long long ldk, const void* Vp, long long ldv,
+                         const void* dOp, long long lddo, const void* QT, long long ldqt, const void* KT, long long ldkt,
+                         const void* dOT, long long lddot, const float* lse, const float* delta, const unsigned char* key_mask,
+                         void* dQ, long long lddq, void* dK, long long lddk, void* dV, long long lddv, int B, int heads,
+                         int N, int d, cudaStream_t stream) {
   const int dp = d == 40 ? 48 : 80;
-  AF_CHECK_ARG(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0 && lddo % 8 == 0 && ldqt % 8 == 0 && ldkt % 8 == 0 && lddot % 8 == 0 &&
-                   lddq % 8 == 0 && lddk % 8 == 0 && lddv % 8 == 0,
-               "af_attention_bwd_bf16: leading dims must be multiples of 8");
-  AF_CHECK_ARG(ldqt >= static_cast<long long>(B) * N && ldkt >= static_cast<long long>(B) * N && lddot >= static_cast<long long>(B) * N,
-               "af_attention_bwd_bf16: transposed operands need B*N columns");
+  const bool masked = key_mask != nullptr;
   int rc;
   {   // dQ: rows = queries (X = Q, Y = dO), columns = keys (U = K, W = V), B operand of the gradient MMA = K^T
     AttnBwdParams p;
@@ -376,10 +423,12 @@ extern "C" int af_attention_bwd_bf16(const void* Q, long long ldq, const void* K
     if ((rc = make_rows_map(&p.tmW, Vp, ldv, heads, dp, N, B, 64))) return rc;
     if ((rc = make_t_map(&p.tmT0, KT, ldkt, heads, dp))) return rc;
     p.tmT1 = p.tmT0;
-    p.lse = lse; p.delta = delta;
+    p.lse = lse; p.delta = delta; p.kmask = key_mask;
     p.out0 = static_cast<__nv_bfloat16*>(dQ); p.ld0 = lddq;
     p.B = B; p.heads = heads; p.N = N; p.d = d;
-    if ((rc = d == 40 ? launch_bwd<40, false>(p, stream) : launch_bwd<80, false>(p, stream))) return rc;
+    rc = d == 40 ? (masked ? launch_bwd<40, false, true>(p, stream) : launch_bwd<40, false, false>(p, stream))
+                 : (masked ? launch_bwd<80, false, true>(p, stream) : launch_bwd<80, false, false>(p, stream));
+    if (rc) return rc;
   }
   {   // dK, dV: rows = keys (X = K, Y = V), columns = queries (U = Q, W = dO), B operands = dO^T (dV) and Q^T (dK)
     AttnBwdParams p;
@@ -390,11 +439,49 @@ extern "C" int af_attention_bwd_bf16(const void* Q, long long ldq, const void* K
     if ((rc = make_rows_map(&p.tmW, dOp, lddo, heads, dp, N, B, 64))) return rc;
     if ((rc = make_t_map(&p.tmT0, dOT, lddot, heads, dp))) return rc;
     if ((rc = make_t_map(&p.tmT1, QT, ldqt, heads, dp))) return rc;
-    p.lse = lse; p.delta = delta;
+    p.lse = lse; p.delta = delta; p.kmask = key_mask;
     p.out0 = static_cast<__nv_bfloat16*>(dV); p.ld0 = lddv;
     p.out1 = static_cast<__nv_bfloat16*>(dK); p.ld1 = lddk;
     p.B = B; p.heads = heads; p.N = N; p.d = d;
-    if ((rc = d == 40 ? launch_bwd<40, true>(p, stream) : launch_bwd<80, true>(p, stream))) return rc;
+    rc = d == 40 ? (masked ? launch_bwd<40, true, true>(p, stream) : launch_bwd<40, true, false>(p, stream))
+                 : (masked ? launch_bwd<80, true, true>(p, stream) : launch_bwd<80, true, false>(p, stream));
+    if (rc) return rc;
   }
   return 0;
+}
+
+}  // namespace af
+
+#define AF_BWD_CHECK_ARGS(fn)                                                                                          \
+  AF_CHECK_ARG(Q && K && Vp && dOp && QT && KT && dOT && lse && delta && dQ && dK && dV, fn ": null pointer");          \
+  AF_CHECK_ARG(d == 40 || d == 80, fn ": head dim %d unsupported (40 / 80)", d);                                         \
+  AF_CHECK_ARG(B > 0 && heads > 0 && N >= 128 && N % 128 == 0, fn ": N=%d must be a positive multiple of 128", N);       \
+  AF_CHECK_ARG(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0 && lddo % 8 == 0 && ldqt % 8 == 0 && ldkt % 8 == 0 &&       \
+                   lddot % 8 == 0 && lddq % 8 == 0 && lddk % 8 == 0 && lddv % 8 == 0,                                  \
+               fn ": leading dims must be multiples of 8");                                                             \
+  AF_CHECK_ARG(ldqt >= static_cast<long long>(B) * N && ldkt >= static_cast<long long>(B) * N &&                        \
+                   lddot >= static_cast<long long>(B) * N,                                                              \
+               fn ": transposed operands need B*N columns")
+
+extern "C" int af_attention_bwd_bf16(const void* Q, long long ldq, const void* K, long long ldk, const void* Vp,
+                                     long long ldv, const void* dOp, long long lddo, const void* QT, long long ldqt,
+                                     const void* KT, long long ldkt, const void* dOT, long long lddot, const float* lse,
+                                     const float* delta, void* dQ, long long lddq, void* dK, long long lddk, void* dV,
+                                     long long lddv, int B, int heads, int N, int d, cudaStream_t stream) {
+  AF_BWD_CHECK_ARGS("af_attention_bwd_bf16");
+  return af::attention_bwd(Q, ldq, K, ldk, Vp, ldv, dOp, lddo, QT, ldqt, KT, ldkt, dOT, lddot, lse, delta, nullptr, dQ,
+                           lddq, dK, lddk, dV, lddv, B, heads, N, d, stream);
+}
+
+extern "C" int af_attention_bwd_masked_bf16(const void* Q, long long ldq, const void* K, long long ldk, const void* Vp,
+                                            long long ldv, const void* dOp, long long lddo, const void* QT, long long ldqt,
+                                            const void* KT, long long ldkt, const void* dOT, long long lddot,
+                                            const float* lse, const float* delta, const unsigned char* key_mask, void* dQ,
+                                            long long lddq, void* dK, long long lddk, void* dV, long long lddv, int B,
+                                            int heads, int N, int d, cudaStream_t stream) {
+  AF_BWD_CHECK_ARGS("af_attention_bwd_masked_bf16");
+  AF_CHECK_ARG(key_mask && (reinterpret_cast<uintptr_t>(key_mask) & 15) == 0,
+               "af_attention_bwd_masked_bf16: key_mask must be a 16-byte aligned [B, N] byte array");
+  return af::attention_bwd(Q, ldq, K, ldk, Vp, ldv, dOp, lddo, QT, ldqt, KT, ldkt, dOT, lddot, lse, delta, key_mask, dQ,
+                           lddq, dK, lddk, dV, lddv, B, heads, N, d, stream);
 }

@@ -13,6 +13,9 @@
 //   mode 3   C = alpha * P[row,col] * (acc - vec[row])     dS   = P   o (dP   - delta)
 //   mode 4   C = alpha * P[row,col] * (acc - vec[col])     dS^T = P^T o (dP^T - delta)
 // Entries with row >= valid_rows or col >= valid_cols are written as 0 (padded keys / queries).
+// With a key mask (bgemm_masked_kernel, modes 1-4: attention.py:223-232) masked keys - columns of modes 1 / 3, rows of
+// modes 2 / 4 - get P = 0 and dS = 0, or P = 1 / (number of valid keys) in modes 1 / 2 where vec = +inf (a sample that
+// keeps no key: the forward gave its rows the mean of V).  Kept keys take the unmasked arithmetic unchanged.
 #include "../../include/adaface_b200.h"
 #include "common.cuh"
 
@@ -26,6 +29,7 @@ struct BgemmParams {
   const __nv_bfloat16* P; long long ldp, sP0, sP1;
   int M, N, K, nb1, mode, valid_rows, valid_cols, staged;
   float alpha;
+  const uint8_t* kmask; long long sM0, sM1;      // masked kernel only
 };
 
 __device__ __forceinline__ void cp_async16(void* dst, const void* src, bool valid) {
@@ -52,8 +56,8 @@ constexpr int kBM = 128, kBK = 32, kPitch = kBK + 8, kStages = 3;
 
 // MODE is a template parameter: as a run-time field the epilogue carried a five-way option chain inside its 32-iteration
 // element loop (the same pattern that cost the tcgen05 GEMM epilogue 70 cycles per iteration).
-template <int BN, int MODE>
-__global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
+template <int BN, int MODE, bool MASK>
+__device__ __forceinline__ void bgemm_body(const BgemmParams& p) {
   constexpr int WARPS_N = BN / 32, WARPS_M = 8 / WARPS_N, WM = kBM / WARPS_M, MT = WM / 16;
   extern __shared__ __align__(16) uint8_t smem_b[];
   __nv_bfloat16* sA = reinterpret_cast<__nv_bfloat16*>(smem_b);                 // [stages][128][pitch]
@@ -136,6 +140,7 @@ __global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
 
   // ---- epilogue
   const float* vec = p.vec ? p.vec + b0 * p.sV0 + b1 * p.sV1 : nullptr;
+  const uint8_t* km = MASK ? p.kmask + b0 * p.sM0 + b1 * p.sM1 : nullptr;
   const __nv_bfloat16* P = Pt;
   uint8_t* Cb = static_cast<uint8_t*>(p.C) + (b0 * p.sC0 + b1 * p.sC1) * (p.c_f32 ? 4 : 2);
   if (staged) __syncthreads();          // every warp is done with the operand ring (sC aliases it); sP has landed
@@ -147,6 +152,7 @@ __global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
       const int row = m0 + lrow;
       if (row >= p.M) continue;
       const float rv = (vec && (MODE == 1 || MODE == 3) && row < p.valid_rows) ? vec[row] : 0.f;
+      const bool keep_row = !MASK || MODE == 1 || MODE == 3 || (row < p.valid_rows && km[row] != 0);
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int lcol = wn * 32 + j * 8 + (lane & 3) * 2;
@@ -166,6 +172,19 @@ __global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
           const float c0 = MODE == 3 ? rv : (ok0 ? vec[col] : 0.f), c1 = MODE == 3 ? rv : (ok1 ? vec[col + 1] : 0.f);
           v0 = p.alpha * __bfloat162float(pp.x) * (v0 - c0);
           v1 = p.alpha * __bfloat162float(pp.y) * (v1 - c1);
+        }
+        if constexpr (MASK) {
+          const bool k0 = MODE == 1 || MODE == 3 ? ok0 && km[col] != 0 : keep_row;
+          const bool k1 = MODE == 1 || MODE == 3 ? ok1 && km[col + 1] != 0 : keep_row;
+          float e0 = 0.f, e1 = 0.f;       // P of a masked key: 1 / valid keys in a sample that keeps none
+          if constexpr (MODE == 1) {
+            e0 = e1 = rv == INFINITY ? 1.f / static_cast<float>(p.valid_cols) : 0.f;
+          } else if constexpr (MODE == 2) {
+            e0 = ok0 && vec[col] == INFINITY ? 1.f / static_cast<float>(p.valid_rows) : 0.f;
+            e1 = ok1 && vec[col + 1] == INFINITY ? 1.f / static_cast<float>(p.valid_rows) : 0.f;
+          }
+          v0 = k0 ? v0 : e0;
+          v1 = k1 ? v1 : e1;
         }
         v0 = ok0 ? v0 : 0.f;
         v1 = ok1 ? v1 : 0.f;
@@ -191,49 +210,64 @@ __global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
 }
 
 template <int BN, int MODE>
+__global__ void __launch_bounds__(256) bgemm_kernel(const BgemmParams p) {
+  bgemm_body<BN, MODE, false>(p);
+}
+template <int BN, int MODE>
+__global__ void __launch_bounds__(256) bgemm_masked_kernel(const BgemmParams p) {
+  bgemm_body<BN, MODE, true>(p);
+}
+
+template <int BN, int MODE, bool MASK>
 static int launch_bgemm_m(const BgemmParams& p, int batch, cudaStream_t stream) {
   // operand ring (also the output staging tile: 128 x (BN + 8) bf16 fits) + the P tile of modes 3 / 4
   static_assert(kStages * (kBM + BN) * kPitch >= kBM * (BN + 8), "staging tile must fit in the operand ring");
   constexpr int smem = kStages * (kBM + BN) * kPitch * 2 + (MODE >= 3 ? kBM * (BN + 8) * 2 : 0);
+  const auto kernel = MASK ? bgemm_masked_kernel<BN, MODE> : bgemm_kernel<BN, MODE>;
   static bool configured = false;
   if (!configured) {
-    AF_CUDA(cudaFuncSetAttribute(bgemm_kernel<BN, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    AF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     configured = true;
   }
   dim3 grid((p.N + BN - 1) / BN, (p.M + kBM - 1) / kBM, batch);
-  bgemm_kernel<BN, MODE><<<grid, 256, smem, stream>>>(p);
-  AF_LAUNCH_CHECK("bgemm_kernel");
+  kernel<<<grid, 256, smem, stream>>>(p);
+  AF_LAUNCH_CHECK(MASK ? "bgemm_masked_kernel" : "bgemm_kernel");
   return 0;
 }
 template <int BN>
 static int launch_bgemm(const BgemmParams& p, int batch, cudaStream_t stream) {
+  if (p.kmask) {
+    switch (p.mode) {
+      case 1: return launch_bgemm_m<BN, 1, true>(p, batch, stream);
+      case 2: return launch_bgemm_m<BN, 2, true>(p, batch, stream);
+      case 3: return launch_bgemm_m<BN, 3, true>(p, batch, stream);
+      default: return launch_bgemm_m<BN, 4, true>(p, batch, stream);
+    }
+  }
   switch (p.mode) {
-    case 0: return launch_bgemm_m<BN, 0>(p, batch, stream);
-    case 1: return launch_bgemm_m<BN, 1>(p, batch, stream);
-    case 2: return launch_bgemm_m<BN, 2>(p, batch, stream);
-    case 3: return launch_bgemm_m<BN, 3>(p, batch, stream);
-    default: return launch_bgemm_m<BN, 4>(p, batch, stream);
+    case 0: return launch_bgemm_m<BN, 0, false>(p, batch, stream);
+    case 1: return launch_bgemm_m<BN, 1, false>(p, batch, stream);
+    case 2: return launch_bgemm_m<BN, 2, false>(p, batch, stream);
+    case 3: return launch_bgemm_m<BN, 3, false>(p, batch, stream);
+    default: return launch_bgemm_m<BN, 4, false>(p, batch, stream);
   }
 }
 
-}  // namespace af
-
-using namespace af;
-
-extern "C" int af_bgemm_bf16(const af_bgemm* g, cudaStream_t stream) {
-  AF_CHECK_ARG(g && g->A && g->B && g->C, "af_bgemm_bf16: null pointer");
-  AF_CHECK_ARG(g->M > 0 && g->N > 0 && g->K > 0 && g->nb0 > 0 && g->nb1 > 0, "af_bgemm_bf16: bad sizes");
-  AF_CHECK_ARG(g->K % 8 == 0 && g->N % 2 == 0, "af_bgemm_bf16: K=%d must be a multiple of 8, N=%d even", g->K, g->N);
+static int fill_params(const af_bgemm* g, BgemmParams* out, const char* fn) {
+  AF_CHECK_ARG(g && g->A && g->B && g->C, "%s: null pointer", fn);
+  AF_CHECK_ARG(g->M > 0 && g->N > 0 && g->K > 0 && g->nb0 > 0 && g->nb1 > 0, "%s: bad sizes", fn);
+  AF_CHECK_ARG(g->K % 8 == 0 && g->N % 2 == 0, "%s: K=%d must be a multiple of 8, N=%d even", fn, g->K, g->N);
   AF_CHECK_ARG(g->lda % 8 == 0 && g->ldb % 8 == 0 && g->sA0 % 8 == 0 && g->sA1 % 8 == 0 && g->sB0 % 8 == 0 && g->sB1 % 8 == 0,
-               "af_bgemm_bf16: operand pitches / batch strides must be multiples of 8 elements (16-byte cp.async)");
+               "%s: operand pitches / batch strides must be multiples of 8 elements (16-byte cp.async)", fn);
   AF_CHECK_ARG((reinterpret_cast<uintptr_t>(g->A) & 15) == 0 && (reinterpret_cast<uintptr_t>(g->B) & 15) == 0,
-               "af_bgemm_bf16: operands must be 16-byte aligned");
-  AF_CHECK_ARG(g->ldc % 2 == 0 && g->sC0 % 2 == 0 && g->sC1 % 2 == 0, "af_bgemm_bf16: C pitch / strides must be even");
-  AF_CHECK_ARG(g->mode >= 0 && g->mode <= 4, "af_bgemm_bf16: mode %d", g->mode);
-  AF_CHECK_ARG(g->mode == 0 || g->vec, "af_bgemm_bf16: mode %d needs vec", g->mode);
-  AF_CHECK_ARG(g->mode < 3 || (g->P && g->ldp % 2 == 0 && g->sP0 % 2 == 0 && g->sP1 % 2 == 0), "af_bgemm_bf16: mode %d needs P (even pitch)", g->mode);
-  AF_CHECK_ARG(static_cast<long long>(g->nb0) * g->nb1 <= 65535, "af_bgemm_bf16: batch too large");
-  BgemmParams p;
+               "%s: operands must be 16-byte aligned", fn);
+  AF_CHECK_ARG(g->ldc % 2 == 0 && g->sC0 % 2 == 0 && g->sC1 % 2 == 0, "%s: C pitch / strides must be even", fn);
+  AF_CHECK_ARG(g->mode >= 0 && g->mode <= 4, "%s: mode %d", fn, g->mode);
+  AF_CHECK_ARG(g->mode == 0 || g->vec, "%s: mode %d needs vec", fn, g->mode);
+  AF_CHECK_ARG(g->mode < 3 || (g->P && g->ldp % 2 == 0 && g->sP0 % 2 == 0 && g->sP1 % 2 == 0), "%s: mode %d needs P (even pitch)", fn, g->mode);
+  AF_CHECK_ARG(static_cast<long long>(g->nb0) * g->nb1 <= 65535, "%s: batch too large", fn);
+  BgemmParams& p = *out;
+  memset(&p, 0, sizeof(p));
   p.A = static_cast<const __nv_bfloat16*>(g->A); p.lda = g->lda; p.sA0 = g->sA0; p.sA1 = g->sA1;
   p.B = static_cast<const __nv_bfloat16*>(g->B); p.ldb = g->ldb; p.sB0 = g->sB0; p.sB1 = g->sB1;
   p.C = g->C; p.ldc = g->ldc; p.sC0 = g->sC0; p.sC1 = g->sC1; p.c_f32 = g->c_dtype == AF_DTYPE_F32;
@@ -248,6 +282,28 @@ extern "C" int af_bgemm_bf16(const af_bgemm* g, cudaStream_t stream) {
               (reinterpret_cast<uintptr_t>(g->C) & 15) == 0 &&
               (g->mode < 3 || (g->ldp % 8 == 0 && g->sP0 % 8 == 0 && g->sP1 % 8 == 0 &&
                                (reinterpret_cast<uintptr_t>(g->P) & 15) == 0))) ? 1 : 0;
+  return 0;
+}
+
+}  // namespace af
+
+using namespace af;
+
+extern "C" int af_bgemm_bf16(const af_bgemm* g, cudaStream_t stream) {
+  BgemmParams p;
+  if (int rc = fill_params(g, &p, "af_bgemm_bf16")) return rc;
+  const int batch = g->nb0 * g->nb1;
+  return g->N <= 64 ? launch_bgemm<64>(p, batch, stream) : launch_bgemm<128>(p, batch, stream);
+}
+
+extern "C" int af_bgemm_masked_bf16(const af_bgemm* g, const unsigned char* key_mask, long long sM0, long long sM1,
+                                    cudaStream_t stream) {
+  BgemmParams p;
+  if (int rc = fill_params(g, &p, "af_bgemm_masked_bf16")) return rc;
+  AF_CHECK_ARG(key_mask, "af_bgemm_masked_bf16: null key_mask");
+  AF_CHECK_ARG(g->mode >= 1, "af_bgemm_masked_bf16: mode %d takes no key mask (modes 1-4)", g->mode);
+  AF_CHECK_ARG(sM0 >= 0 && sM1 >= 0, "af_bgemm_masked_bf16: negative mask strides");
+  p.kmask = key_mask; p.sM0 = sM0; p.sM1 = sM1;
   const int batch = g->nb0 * g->nb1;
   return g->N <= 64 ? launch_bgemm<64>(p, batch, stream) : launch_bgemm<128>(p, batch, stream);
 }

@@ -581,9 +581,32 @@ def attention_lse(q, k, vt, out, lse, *, B, heads, Nq, Nk, d, ldq, ldk, ldvt, kv
     return out
 
 
+def check_key_mask(key_mask: torch.Tensor, B: int, N: int, name: str = "key_mask") -> None:
+    """A self-attention key mask as the masked backward kernels read it: uint8 [B, N] (1 = attend), contiguous, CUDA."""
+    if not isinstance(key_mask, torch.Tensor):
+        raise ValueError(f"{name}: expected a torch.Tensor, got {type(key_mask).__name__}")
+    if key_mask.dtype != torch.uint8:
+        raise ValueError(f"{name}: expected torch.uint8, got {key_mask.dtype}")
+    if tuple(key_mask.shape) != (B, N):
+        raise ValueError(f"{name}: expected shape {(B, N)}, got {tuple(key_mask.shape)}")
+    if not key_mask.is_contiguous():
+        raise ValueError(f"{name}: must be contiguous")
+    if not key_mask.is_cuda:
+        raise ValueError(f"{name}: expected a CUDA tensor (there is no CPU path)")
+    if key_mask.data_ptr() % 16:
+        raise ValueError(f"{name}: must start on a 16-byte boundary")
+
+
 def bgemm(A, lda, sA, Bm, ldb, sB, C, ldc, sC, *, M, N, K, nb0, nb1, mode=0, vec=None, sV=(0, 0), P=None, ldp=0,
-          sP=(0, 0), valid_rows=0, valid_cols=0, alpha=1.0):
-    """Batched strided C[z] = epi(A[z] . B[z]^T); A/B/C/P are (tensor, element offset) pairs or tensors."""
+          sP=(0, 0), valid_rows=0, valid_cols=0, alpha=1.0, key_mask=None):
+    """Batched strided C[z] = epi(A[z] . B[z]^T); A/B/C/P are (tensor, element offset) pairs or tensors.
+    key_mask: uint8 [nb0, keys] self-attention key mask (modes 1-4, af_bgemm_masked_bf16), keys = valid_cols of modes
+    1 / 3, valid_rows of modes 2 / 4; the same mask serves every head (z = (sample, head))."""
+    if key_mask is not None:
+        if mode not in (1, 2, 3, 4):
+            raise ValueError(f"bgemm: mode {mode} takes no key mask")
+        nk = (valid_cols or N) if mode in (1, 3) else (valid_rows or M)
+        check_key_mask(key_mask, nb0, nk)
     lib = _lib.load()
 
     def ptr(t):
@@ -601,8 +624,12 @@ def bgemm(A, lda, sA, Bm, ldb, sB, C, ldc, sC, *, M, N, K, nb0, nb1, mode=0, vec
     g.P, g.ldp, g.sP0, g.sP1 = (ptr(P) if P is not None else None), ldp, sP[0], sP[1]
     g.M, g.N, g.K, g.nb0, g.nb1, g.mode = M, N, K, nb0, nb1, mode
     g.valid_rows, g.valid_cols, g.alpha = valid_rows, valid_cols, float(alpha)
-    rc = lib.af_bgemm_bf16(byref(g), _stream())
-    _lib.check(rc, "af_bgemm_bf16")
+    if key_mask is None:
+        rc = lib.af_bgemm_bf16(byref(g), _stream())
+        _lib.check(rc, "af_bgemm_bf16")
+        return
+    rc = lib.af_bgemm_masked_bf16(byref(g), key_mask.data_ptr(), int(key_mask.shape[1]), 0, _stream())
+    _lib.check(rc, "af_bgemm_masked_bf16")
 
 
 def groupnorm_mean_rstd(x: torch.Tensor, st: GNStats, eps: float) -> torch.Tensor:
@@ -710,8 +737,11 @@ def conv_attn_scores(score, cols, *, B, heads, Hf, Wf, nk, ks):
     return ov
 
 
-def attention_bwd(q, k, vp, dop, qT, kT, dOT, lse, delta, *, B, heads, N, d):
-    """dQ [B*N, h*dp], dK [B*N, h*dp], dV [B*N, h*d] (bf16) of the long self-attention (af_attention_bwd_bf16)."""
+def attention_bwd(q, k, vp, dop, qT, kT, dOT, lse, delta, *, B, heads, N, d, key_mask=None):
+    """dQ [B*N, h*dp], dK [B*N, h*dp], dV [B*N, h*d] (bf16) of the long self-attention (af_attention_bwd_bf16).
+    key_mask: uint8 [B, N] self-attention key mask (af_attention_bwd_masked_bf16)."""
+    if key_mask is not None:
+        check_key_mask(key_mask, B, N)
     lib = _lib.load()
     dp = 48 if d == 40 else d
     dev = q.device
@@ -721,12 +751,21 @@ def attention_bwd(q, k, vp, dop, qT, kT, dOT, lse, delta, *, B, heads, N, d):
     for t in (q, k, vp, dop, qT, kT, dOT):
         if t.dtype != torch.bfloat16 or t.stride(-1) != 1:
             raise ValueError("attention_bwd: bf16 row-major operands expected")
-    rc = lib.af_attention_bwd_bf16(q.data_ptr(), int(q.stride(0)), k.data_ptr(), int(k.stride(0)), vp.data_ptr(),
-                                   int(vp.stride(0)), dop.data_ptr(), int(dop.stride(0)), qT.data_ptr(), int(qT.stride(0)),
-                                   kT.data_ptr(), int(kT.stride(0)), dOT.data_ptr(), int(dOT.stride(0)), lse.data_ptr(),
-                                   delta.data_ptr(), dq.data_ptr(), heads * dp, dk.data_ptr(), heads * dp, dv.data_ptr(),
-                                   heads * d, B, heads, N, d, _stream())
-    _lib.check(rc, "af_attention_bwd_bf16")
+    if key_mask is None:
+        rc = lib.af_attention_bwd_bf16(q.data_ptr(), int(q.stride(0)), k.data_ptr(), int(k.stride(0)), vp.data_ptr(),
+                                       int(vp.stride(0)), dop.data_ptr(), int(dop.stride(0)), qT.data_ptr(),
+                                       int(qT.stride(0)), kT.data_ptr(), int(kT.stride(0)), dOT.data_ptr(),
+                                       int(dOT.stride(0)), lse.data_ptr(), delta.data_ptr(), dq.data_ptr(), heads * dp,
+                                       dk.data_ptr(), heads * dp, dv.data_ptr(), heads * d, B, heads, N, d, _stream())
+        _lib.check(rc, "af_attention_bwd_bf16")
+        return dq, dk, dv
+    rc = lib.af_attention_bwd_masked_bf16(q.data_ptr(), int(q.stride(0)), k.data_ptr(), int(k.stride(0)), vp.data_ptr(),
+                                          int(vp.stride(0)), dop.data_ptr(), int(dop.stride(0)), qT.data_ptr(),
+                                          int(qT.stride(0)), kT.data_ptr(), int(kT.stride(0)), dOT.data_ptr(),
+                                          int(dOT.stride(0)), lse.data_ptr(), delta.data_ptr(), key_mask.data_ptr(),
+                                          dq.data_ptr(), heads * dp, dk.data_ptr(), heads * dp, dv.data_ptr(), heads * d,
+                                          B, heads, N, d, _stream())
+    _lib.check(rc, "af_attention_bwd_masked_bf16")
     return dq, dk, dv
 
 

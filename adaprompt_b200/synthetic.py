@@ -64,13 +64,36 @@ def stage1_stack(dev, unet=None):
     return step, trainable_parameters(sbg)
 
 
-def stage1_batch(dev, bs: int, latent: int, generator: torch.Generator):
+def stage1_batch(dev, bs: int, latent: int, generator: torch.Generator, masks: bool = False):
     """One synthetic micro-batch: x0 / noise / t / a fixed teacher eps (the diffusers teacher is unavailable, SURVEY.md
-    section 8(d) config 4) / L2-normalised 512-d ArcFace embeddings / the tokens of "a photo of a z, , ...". """
+    section 8(d) config 4) / L2-normalised 512-d ArcFace embeddings / the tokens of "a photo of a z, , ...".
+    masks: also "img_mask" and "fg_mask" (float [bs, 1, H, H]) drawn after everything else, so the other tensors are
+    those of masks=False: see synthetic_masks."""
     g, H = generator, latent
     prompt = [49406, 320, 1125, 539, 320, 345] + [267] * 15 + [49407] * 56
-    return {"x0": torch.randn(bs, 4, H, H, generator=g).to(dev), "noise": torch.randn(bs, 4, H, H, generator=g).to(dev),
-            "t": torch.randint(0, 1000, (bs,), generator=g).to(dev),
-            "teacher_eps": torch.randn(bs, 4, H, H, generator=g).to(dev),
-            "face_embs": torch.nn.functional.normalize(torch.randn(bs, 512, generator=g), dim=-1).to(dev),
-            "tokens": torch.tensor([prompt] * bs).to(dev)}
+    batch = {"x0": torch.randn(bs, 4, H, H, generator=g).to(dev), "noise": torch.randn(bs, 4, H, H, generator=g).to(dev),
+             "t": torch.randint(0, 1000, (bs,), generator=g).to(dev),
+             "teacher_eps": torch.randn(bs, 4, H, H, generator=g).to(dev),
+             "face_embs": torch.nn.functional.normalize(torch.randn(bs, 512, generator=g), dim=-1).to(dev),
+             "tokens": torch.tensor([prompt] * bs).to(dev)}
+    if masks:
+        img_mask, fg_mask = synthetic_masks(bs, H, g)
+        batch["img_mask"], batch["fg_mask"] = img_mask.to(dev), fg_mask.to(dev)
+    return batch
+
+
+def synthetic_masks(bs: int, H: int, generator: torch.Generator):
+    """Plausible masks of a face-image batch at latent size H x H (CPU, float [bs, 1, H, H]):
+      img_mask: the image inside a zero border of 0 .. H/8 pixels on each side (augmentation padding);
+      fg_mask:  a face box of 3/8 .. 5/8 of the side, placed inside the image."""
+    g = generator
+    img = torch.zeros(bs, 1, H, H)
+    fg = torch.zeros(bs, 1, H, H)
+    for b in range(bs):
+        t, bo, l, r = (int(v) for v in torch.randint(0, H // 8 + 1, (4,), generator=g))
+        img[b, :, t:H - bo, l:H - r] = 1
+        side = int(torch.randint(3 * H // 8, 5 * H // 8 + 1, (1,), generator=g))
+        y0 = t + int(torch.randint(0, max(1, H - bo - t - side + 1), (1,), generator=g))
+        x0 = l + int(torch.randint(0, max(1, H - r - l - side + 1), (1,), generator=g))
+        fg[b, :, y0:y0 + side, x0:x0 + side] = 1
+    return img, fg * img

@@ -3,7 +3,10 @@
 Reference: LatentDiffusion.guided_denoise (ldm/models/diffusion/ddpm.py:2483-2532) runs UNetModel.forward WITH grad;
 the UNet weights are frozen (ddpm.py:783-786), so its backward is activation gradients only - they flow to the
 trainable SubjBasisGenerator through the 16 layerwise cross-attention contexts (openaimodel.py:866,978).  The loss is
-the (masked) MSE against the teacher's noise prediction (calc_recon_loss ddpm.py:3571-3595, :3010-3037).
+the (masked) MSE against the teacher's noise prediction (calc_recon_loss ddpm.py:3571-3595, :3010-3037): distill_loss
+without image masks, calc_recon_loss with them.  A batch of real face images carries an image mask (which latent pixels
+hold image rather than augmentation padding), used by the student UNet as a self-attention key mask, and a face mask;
+both weight the loss.
 
 torch.autograd is used as the *tape* only (plumbing: which op ran, which buffers it saved); every forward and
 backward op below is a hand-written kernel behind the C ABI:
@@ -273,10 +276,11 @@ class GegluFn(Function):
 class AttentionFn(Function):
     """softmax(q k^T) v per (sample, head) (attention.py:198-242).  q bf16 [B*Nq, >= h*dp] (pre-scaled, log2 domain),
     k bf16 [B*nk_pad, >= h*dp], v bf16 [B*nk_pad, h*d]; q / k may be column views of one fused [Q|K] buffer.
-    Returns o bf16 [B*Nq, h*d].  nk <= nk_pad valid keys per sample."""
+    Returns o bf16 [B*Nq, h*d].  nk <= nk_pad valid keys per sample.  key_mask: None or uint8 [B, nk] (1 = attend), the
+    self-attention key mask of attention.py:223-232; its backward runs the masked kernels."""
 
     @staticmethod
-    def forward(ctx, q, k, v, B, heads, d, Nq, nk, nk_pad):
+    def forward(ctx, q, k, v, B, heads, d, Nq, nk, nk_pad, key_mask=None):
         dp = head_pad(d)
         C = heads * d
         dev = q.device
@@ -284,9 +288,12 @@ class AttentionFn(Function):
         vt = ops.transpose_to_bf16(v.contiguous(), ldvt)                     # V^T [C, ldvt] (forward kernel operand)
         o = torch.empty(B * Nq, C, dtype=torch.bfloat16, device=dev)
         lse = torch.empty(B, heads, Nq, dtype=torch.float32, device=dev)
+        if key_mask is not None:
+            ops.check_key_mask(key_mask, B, nk)
         ops.attention_lse(q, k, vt, o, lse, B=B, heads=heads, Nq=Nq, Nk=nk, d=d, ldq=int(q.stride(0)),
-                          ldk=int(k.stride(0)), ldvt=ldvt, kv_stride=nk_pad)
+                          ldk=int(k.stride(0)), ldvt=ldvt, kv_stride=nk_pad, key_mask=key_mask)
         ctx.save_for_backward(q, k, v, o, lse)
+        ctx.key_mask = key_mask
         ctx.geom = (B, heads, d, dp, Nq, nk, nk_pad)
         return o
 
@@ -299,6 +306,7 @@ class AttentionFn(Function):
         dO = dO.contiguous()
         ldq, ldk = int(q.stride(0)), int(k.stride(0))
         delta = ops.rowdot_heads(dO, o, B, Nq, h, d)                                  # [B, h, Nq]
+        km = ctx.key_mask                       # None: the unmasked kernels; else their masked instantiations
         Tq, Tk = B * Nq, B * nkp
         if d in (40, 80) and Nq == nk == nkp and Nq % 128 == 0 and ops.attention_bwd is not None:
             # long self-attention: fused tcgen05 backward (attention_bwd.cu), P / dS never leave the SM
@@ -307,7 +315,7 @@ class AttentionFn(Function):
             qT = ops.transpose_to_bf16(q[:, :h * dp].contiguous())
             kT = ops.transpose_to_bf16(k[:, :h * dp].contiguous())
             dOT = ops.transpose_to_bf16(dop)
-            dq, dk, dv = ops.attention_bwd(q, k, vp, dop, qT, kT, dOT, lse, delta, B=B, heads=h, N=Nq, d=d)
+            dq, dk, dv = ops.attention_bwd(q, k, vp, dop, qT, kT, dOT, lse, delta, B=B, heads=h, N=Nq, d=d, key_mask=km)
             if q.shape[1] != h * dp:
                 full = torch.zeros(q.shape, dtype=torch.bfloat16, device=dev)
                 full[:, :h * dp] = dq
@@ -316,7 +324,7 @@ class AttentionFn(Function):
                 full = torch.zeros(k.shape, dtype=torch.bfloat16, device=dev)
                 full[:, :h * dp] = dk
                 dk = full
-            return dq, dk, dv, None, None, None, None, None, None
+            return dq, dk, dv, None, None, None, None, None, None, None
         qT = ops.transpose_to_bf16(q[:, :h * dp].contiguous())                       # [h*dp, Tq_p]
         kT = ops.transpose_to_bf16(k[:, :h * dp].contiguous())                       # [h*dp, Tk_p]
         dOT = ops.transpose_to_bf16(dO)                                              # [C, Tq_p]
@@ -327,16 +335,16 @@ class AttentionFn(Function):
         qa, ka = q, k                                                                # views: data_ptr() carries the offset
         # P = exp2(S - lse), P^T likewise (S^T recomputed; padded keys -> 0)
         ops.bgemm(qa, ldq, (Nq * ldq, dp), ka, ldk, (nkp * ldk, dp), P, nkp, sP, M=Nq, N=nkp, K=dp, nb0=B, nb1=h,
-                  mode=1, vec=lse, sV=(h * Nq, Nq), valid_cols=nk)
+                  mode=1, vec=lse, sV=(h * Nq, Nq), valid_cols=nk, key_mask=km)
         ops.bgemm(ka, ldk, (nkp * ldk, dp), qa, ldq, (Nq * ldq, dp), Pt, Nq, sP, M=nkp, N=Nq, K=dp, nb0=B, nb1=h,
-                  mode=2, vec=lse, sV=(h * Nq, Nq), valid_rows=nk)
+                  mode=2, vec=lse, sV=(h * Nq, Nq), valid_rows=nk, key_mask=km)
         # dS = ln2 * P o (dO V^T - delta)  and its transpose
         dS = torch.empty_like(P)
         dSt = torch.empty_like(Pt)
         ops.bgemm(dO, C, (Nq * C, d), v, C, (nkp * C, d), dS, nkp, sP, M=Nq, N=nkp, K=d, nb0=B, nb1=h, mode=3,
-                  vec=delta, sV=(h * Nq, Nq), P=P, ldp=nkp, sP=sP, valid_cols=nk, alpha=LN2)
+                  vec=delta, sV=(h * Nq, Nq), P=P, ldp=nkp, sP=sP, valid_cols=nk, alpha=LN2, key_mask=km)
         ops.bgemm(v, C, (nkp * C, d), dO, C, (Nq * C, d), dSt, Nq, sP, M=nkp, N=Nq, K=d, nb0=B, nb1=h, mode=4,
-                  vec=delta, sV=(h * Nq, Nq), P=Pt, ldp=Nq, sP=sP, valid_rows=nk, alpha=LN2)
+                  vec=delta, sV=(h * Nq, Nq), P=Pt, ldp=Nq, sP=sP, valid_rows=nk, alpha=LN2, key_mask=km)
         # dQ = dS K, dK = dS^T Q, dV = P^T dO
         dq = torch.zeros(Tq, h * dp, dtype=torch.bfloat16, device=dev)
         dk = torch.zeros(Tk, h * dp, dtype=torch.bfloat16, device=dev)
@@ -354,7 +362,7 @@ class AttentionFn(Function):
             full = torch.zeros(k.shape, dtype=torch.bfloat16, device=dev)
             full[:, :h * dp] = dk
             dk = full
-        return dq, dk, dv, None, None, None, None, None, None
+        return dq, dk, dv, None, None, None, None, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------ modules
@@ -382,8 +390,10 @@ def _ln(block: BasicTransformerBlock, name: str, x: torch.Tensor) -> torch.Tenso
 
 
 def transformer_block_train(block: BasicTransformerBlock, t: torch.Tensor, B: int, N: int,
-                            ctx_k: Optional[torch.Tensor], ctx_v: Optional[torch.Tensor]) -> torch.Tensor:
-    """BasicTransformerBlock._forward (attention.py:275-285) with grad; t fp32 [B*N, C]; ctx_* fp32 [B, nk, 768]."""
+                            ctx_k: Optional[torch.Tensor], ctx_v: Optional[torch.Tensor],
+                            key_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """BasicTransformerBlock._forward (attention.py:275-285) with grad; t fp32 [B*N, C]; ctx_* fp32 [B, nk, 768];
+    key_mask: uint8 [B, N] self-attention key mask (attn1 only, :277) or None."""
     a1, a2, ff = block.attn1, block.attn2, block.ff
     h, d = a1.heads, a1.dim_head
     dp = head_pad(d)
@@ -391,7 +401,7 @@ def transformer_block_train(block: BasicTransformerBlock, t: torch.Tensor, B: in
     ln1 = _ln(block, "norm1", t)
     qk = linear(ln1, p1["wqk"], b1["wqk"], out_dtype=torch.bfloat16)
     v = linear(ln1, p1["wv"], b1["wv"], out_dtype=torch.bfloat16)
-    o = AttentionFn.apply(qk, qk[:, h * dp:], v, B, h, d, N, N, N)
+    o = AttentionFn.apply(qk, qk[:, h * dp:], v, B, h, d, N, N, N, key_mask)
     x1 = linear(o, p1["wo"], b1["wo"], p1["bo"], residual=t)
     p2, b2 = a2.packed(), bwd_packs(a2)
     ln2 = _ln(block, "norm2", x1)
@@ -412,15 +422,17 @@ def transformer_block_train(block: BasicTransformerBlock, t: torch.Tensor, B: in
     return linear(hid, pf["w2"], bf_["w2"], pf["b2"], residual=x2)
 
 
-def spatial_transformer_train(st: SpatialTransformer, x: torch.Tensor, ctx) -> torch.Tensor:
-    """SpatialTransformer.forward (attention.py:321-341) with grad; x fp32 NHWC; ctx = (v_ctx, k_ctx) fp32 [B,nk,768]."""
+def spatial_transformer_train(st: SpatialTransformer, x: torch.Tensor, ctx,
+                              key_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """SpatialTransformer.forward (attention.py:321-341) with grad; x fp32 NHWC; ctx = (v_ctx, k_ctx) fp32 [B,nk,768];
+    key_mask: uint8 [B, H*W] (the image mask at this layer's resolution, :332) or None."""
     pk, pb = st.packed(), bwd_packs(st)
     B, H, W, C = x.shape
     T = B * H * W
     xn = _gn(x, pk["gn_w"], pk["gn_b"], pk["gn_eps"], False)
     t = linear(xn.reshape(T, C), pk["w_in"], pb["w_in"], pk["b_in"])
     v_ctx, k_ctx = ctx
-    tb = transformer_block_train(st.transformer_blocks[0], t, B, H * W, k_ctx, v_ctx)
+    tb = transformer_block_train(st.transformer_blocks[0], t, B, H * W, k_ctx, v_ctx, key_mask)
     out = linear(CastBF16.apply(tb), pk["w_out"], pb["w_out"], pk["b_out"], residual=x.reshape(T, C).contiguous())
     return out.reshape(B, H, W, C)
 
@@ -428,18 +440,34 @@ def spatial_transformer_train(st: SpatialTransformer, x: torch.Tensor, ctx) -> t
 def unet_forward_train(unet: UNetModel, x: torch.Tensor, timesteps: torch.Tensor, context: torch.Tensor,
                        extra_info: dict) -> torch.Tensor:
     """UNetModel.forward (openaimodel.py:827-1052) with grad w.r.t. `context` [16*B, nk, 768].
-    Returns eps fp32 NCHW [B, 4, H, W].  Image masks / conv attention / attention capture are not part of the
-    zero-shot distillation branch (ddpm.py:3010-3013) and raise."""
+    Returns eps fp32 NCHW [B, 4, H, W].  extra_info["img_mask"]: None or float / bool [B, 1, H, W] at the latent's
+    resolution; every self-attention layer masks the keys of its nearest-resized copy (attention.py:332 -> :277, as
+    the inference path does).  Attention capture and conv attention are not part of the zero-shot distillation branch
+    (ddpm.py:3010-3013) and raise."""
     if not extra_info.get("use_layerwise_context", False):
         raise ValueError("extra_info['use_layerwise_context'] must be True")
-    if extra_info.get("img_mask", None) is not None or extra_info.get("capture_distill_attn", False):
-        raise NotImplementedError("training step: img_mask / capture_distill_attn")
+    if extra_info.get("capture_distill_attn", False):
+        raise NotImplementedError("training step: capture_distill_attn")
     if extra_info.get("use_conv_attn_kernel_size", -1) > 0 and extra_info.get("placeholder2indices", None) is not None:
         raise NotImplementedError("training step: the backward of conv attention is not built (zero-shot distillation runs "
                                   "with use_conv_attn_kernel_size = -1)")
+    img_mask = extra_info.get("img_mask", None)
+    if img_mask is not None:
+        check_image_mask(img_mask, x, "extra_info['img_mask']")
     iter_type = extra_info.get("iter_type", "normal_recon")
     pk = unet.packed()
     B = x.shape[0]
+    key_masks = {}
+
+    def key_mask(H, W):
+        """uint8 [B, H*W] key mask of a self-attention layer at H x W (attention.py:435-437), built once per resolution."""
+        if img_mask is None:
+            return None
+        km = key_masks.get((H, W))
+        if km is None:
+            m2 = torch.nn.functional.interpolate(img_mask.float(), size=(H, W), mode="nearest")
+            km = key_masks[(H, W)] = m2.reshape(B, H * W).bool().to(torch.uint8).contiguous()
+        return km
     with torch.no_grad():
         _, rows = unet.time_embedding(timesteps)
     offs = pk["emb_offs"]
@@ -458,7 +486,7 @@ def unet_forward_train(unet: UNetModel, x: torch.Tensor, timesteps: torch.Tensor
                 o, n = offs[id(layer)]
                 h = resblock_train(layer, h, rows[:, o:o + n])
             elif isinstance(layer, SpatialTransformer):
-                h = spatial_transformer_train(layer, h, layer_ctx(layer_idx))
+                h = spatial_transformer_train(layer, h, layer_ctx(layer_idx), key_mask(h.shape[1], h.shape[2]))
             elif isinstance(layer, Upsample):
                 h = UpsampleConvFn.apply(h, layer.packed()["w"], bwd_packs(layer)["w"], layer.packed()["b"])
             elif isinstance(layer, Downsample):
@@ -493,25 +521,70 @@ def distill_loss(eps: torch.Tensor, teacher_eps: torch.Tensor, num_denoising_ste
     return torch.nn.functional.mse_loss(eps, teacher_eps) / math.sqrt(num_denoising_steps)
 
 
+def check_image_mask(mask, x: torch.Tensor, name: str) -> None:
+    """An image / face mask of the latent batch x [B, C, H, W]: a float or bool tensor [B, 1, H, W] on x's device."""
+    if not isinstance(mask, torch.Tensor):
+        raise ValueError(f"{name}: expected a tensor, got {type(mask).__name__}")
+    if not (mask.dtype == torch.bool or mask.dtype.is_floating_point):
+        raise ValueError(f"{name}: expected a float or bool tensor, got {mask.dtype}")
+    want = (x.shape[0], 1, x.shape[2], x.shape[3])
+    if tuple(mask.shape) != want:
+        raise ValueError(f"{name}: expected shape {want} (the latent's batch and resolution), got {tuple(mask.shape)}")
+    if mask.device != x.device:
+        raise ValueError(f"{name}: on {mask.device}, the latents are on {x.device}")
+
+
+def calc_recon_loss(eps: torch.Tensor, target: torch.Tensor, img_mask: Optional[torch.Tensor] = None,
+                    fg_mask: Optional[torch.Tensor] = None, fg_pixel_weight: float = 1.,
+                    bg_pixel_weight: float = 1.) -> torch.Tensor:
+    """Masked, foreground / background weighted MSE of calc_recon_loss (ddpm.py:3571-3595), restated:
+        pix = (eps*img - target*img)^2,  wf = fg*img*fg_pixel_weight,  wb = (1 - fg)*img*bg_pixel_weight,
+        loss = (sum pix*wf + sum pix*wb) / (sum wf + sum wb)
+    with the [B, 1, H, W] masks broadcast over the channels of eps / target [B, C, H, W]; a missing mask is all ones, so
+    with neither mask this is F.mse_loss.  Parity unpinned: no reference outputs exist to pin this restatement to (as
+    for tests/vae_encoder_oracle.py).  The reference's call-site weights are not restated; callers pass their own
+    (DistillStep: fg_pixel_weight / bg_pixel_weight, default 1).  Plain tensor arithmetic, no host read-back."""
+    ones = torch.ones_like(eps[:, :1])
+    img = ones if img_mask is None else img_mask.to(eps.dtype)
+    fg = ones if fg_mask is None else fg_mask.to(eps.dtype)
+    pix = (eps * img - target * img) ** 2
+    wf = (fg * img * fg_pixel_weight).expand_as(eps)
+    wb = ((1 - fg) * img * bg_pixel_weight).expand_as(eps)
+    return ((pix * wf).sum() + (pix * wb).sum()) / (wf.sum() + wb.sum())
+
+
 class GraphedUNetLoss:
     """loss = distill_loss(UNet(x_noisy, t, c), teacher_eps) and dloss/dc replayed from ONE CUDA graph.
 
     The UNet is frozen (ddpm.py:783-786), so the ~3500 kernel launches of its forward and backward-to-context depend
     only on the shapes: they are captured once per geometry (static input / output buffers, torch.autograd.grad inside
     the capture) and replayed per micro-batch - the host-side launch gaps of the eager tape (a fifth of the step)
-    disappear.  Weights are read through the version-keyed packs, so a repack invalidates the capture."""
+    disappear.  Weights are read through the version-keyed packs, so a repack invalidates the capture.
+    With an image and / or face mask the loss is calc_recon_loss with the given pixel weights and the image mask also
+    masks the UNet's self-attention keys; the masks are static buffers of the capture, and the geometry key records
+    which of them are present, so masked and unmasked micro-batches never share a graph."""
 
-    def __init__(self, unet: UNetModel, extra_info: dict):
+    def __init__(self, unet: UNetModel, extra_info: dict, fg_pixel_weight: float = 1., bg_pixel_weight: float = 1.):
         self.unet, self.extra_info = unet, dict(extra_info)
+        self.fg_pixel_weight, self.bg_pixel_weight = fg_pixel_weight, bg_pixel_weight
         self._g = {}
 
-    def _build(self, x, t, c, teacher):
+    def _build(self, x, t, c, teacher, img_mask, fg_mask):
         from .attention import PackedModule
-        st = {"x": x.clone(), "t": t.clone(), "c": c.clone().requires_grad_(True), "teacher": teacher.clone()}
+        st = {"x": x.clone(), "t": t.clone(), "c": c.clone().requires_grad_(True), "teacher": teacher.clone(),
+              "img_mask": None if img_mask is None else img_mask.clone(),
+              "fg_mask": None if fg_mask is None else fg_mask.clone()}
 
         def run():
-            eps = unet_forward_train(self.unet, st["x"], st["t"], st["c"], dict(self.extra_info))
-            loss = distill_loss(eps, st["teacher"])
+            extra = dict(self.extra_info)
+            if st["img_mask"] is not None:
+                extra["img_mask"] = st["img_mask"]
+            eps = unet_forward_train(self.unet, st["x"], st["t"], st["c"], extra)
+            if st["img_mask"] is None and st["fg_mask"] is None:
+                loss = distill_loss(eps, st["teacher"])
+            else:
+                loss = calc_recon_loss(eps, st["teacher"], st["img_mask"], st["fg_mask"], self.fg_pixel_weight,
+                                       self.bg_pixel_weight)
             (gc,) = torch.autograd.grad(loss, st["c"])
             return loss.detach(), gc
 
@@ -527,15 +600,22 @@ class GraphedUNetLoss:
         st["graph"], st["epoch"] = graph, PackedModule.PACK_EPOCH
         return st
 
-    def __call__(self, x_noisy, t, c, teacher_eps):
+    def __call__(self, x_noisy, t, c, teacher_eps, img_mask=None, fg_mask=None):
         from .attention import PackedModule
-        key = (tuple(x_noisy.shape), tuple(c.shape), t.dtype)
+        for name, m in (("img_mask", img_mask), ("fg_mask", fg_mask)):
+            if m is not None:
+                check_image_mask(m, x_noisy, name)
+        key = (tuple(x_noisy.shape), tuple(c.shape), t.dtype,
+               None if img_mask is None else img_mask.dtype, None if fg_mask is None else fg_mask.dtype)
         st = self._g.get(key)
         if st is None or st["epoch"] != PackedModule.PACK_EPOCH:
-            st = self._g[key] = self._build(x_noisy, t, c, teacher_eps)
+            st = self._g[key] = self._build(x_noisy, t, c, teacher_eps, img_mask, fg_mask)
         st["x"].copy_(x_noisy)
         st["t"].copy_(t)
         st["teacher"].copy_(teacher_eps)
+        for name, m in (("img_mask", img_mask), ("fg_mask", fg_mask)):
+            if m is not None:
+                st[name].copy_(m)
         with torch.no_grad():
             st["c"].copy_(c)
         st["graph"].replay()

@@ -24,7 +24,7 @@ from torch.autograd import Function
 from . import ops
 from .adaface_util import _ScaleGradFn, _tokenize, arc2face_forward_face_embs
 from .clip_text import CLIPEncoderLayer, CLIPTextTransformer
-from .train import LayerNormFn, distill_loss, linear, unet_forward_train
+from .train import LayerNormFn, calc_recon_loss, check_image_mask, distill_loss, linear, unet_forward_train
 
 N_CA_LAYERS = 16
 
@@ -369,16 +369,44 @@ class _QSampleOnly:
         return a.sqrt() * x0 + (1 - a).sqrt() * noise
 
 
+MASK_KEYS = ("img_mask", "fg_mask")
+
+
+def batch_masks(batch: Dict[str, torch.Tensor]):
+    """-> (img_mask, fg_mask) of a micro-batch, each None or a float / bool [B, 1, H, W] matching batch["x0"]
+    (ValueError otherwise)."""
+    out = []
+    for k in MASK_KEYS:
+        m = batch.get(k)
+        if m is not None:
+            check_image_mask(m, batch["x0"], f'batch["{k}"]')
+        out.append(m)
+    return tuple(out)
+
+
+def check_mask_presence(batches: Sequence[Dict[str, torch.Tensor]]) -> None:
+    """The micro-batches of one optimizer step must carry the same masks (one capture serves them all)."""
+    present = [tuple(b.get(k) is not None for k in MASK_KEYS) for b in batches]
+    if any(p != present[0] for p in present):
+        raise ValueError(f"the micro-batches of one optimizer step disagree on which of {MASK_KEYS} they carry: {present}")
+
+
 class DistillStep:
     """One Stage-1 zero-shot distillation micro-step (ddpm.py:2953-3039 with num_denoising_steps = 1):
     x_noisy = sqrt(a_t) x0 + sqrt(1 - a_t) noise (:416-419) -> student UNet with the AdaFace prompt ->
     MSE against the teacher's noise prediction.  The teacher's eps is either an input (`teacher_eps` in the batch) or
     computed by `teacher` = arc2face_teacher.Arc2FaceTeacher (ddpm.py:5402-5478, SURVEY.md section 8(f) N4) on the
-    21-token Arc2Face ID prompt (ddpm.py:5427) when the batch carries none."""
+    21-token Arc2Face ID prompt (ddpm.py:5427) when the batch carries none.
+    A batch of real images may carry "img_mask" (latent pixels that hold image rather than padding) and "fg_mask" (the
+    face), float or bool [B, 1, H, W] at the latent's resolution.  img_mask masks the student UNet's self-attention keys
+    (the teacher is unchanged), and with either mask the loss is calc_recon_loss with fg_pixel_weight /
+    bg_pixel_weight; without masks it is distill_loss, as before."""
 
     def __init__(self, unet, frozen_tm: CLIPTextTransformer, sbg, arc2face_text_encoder, tokenizer, alphas_cumprod,
-                 placeholder_token: int, extra_info: Optional[dict] = None, teacher=None):
+                 placeholder_token: int, extra_info: Optional[dict] = None, teacher=None, fg_pixel_weight: float = 1.,
+                 bg_pixel_weight: float = 1.):
         self.teacher = teacher
+        self.fg_pixel_weight, self.bg_pixel_weight = fg_pixel_weight, bg_pixel_weight
         self.unet, self.frozen_tm, self.sbg = unet, frozen_tm, sbg
         self.arc2face, self.tokenizer = arc2face_text_encoder, tokenizer
         self.acp = torch.as_tensor(alphas_cumprod, dtype=torch.float32)
@@ -417,12 +445,32 @@ class DistillStep:
         preds, _, _, _ = self.teacher(ddpm, x0, noise, t, prompt_embs, num_denoising_steps=1)
         return preds[0]
 
-    def loss(self, x0, t, noise, teacher_eps, face_embs, tokens) -> torch.Tensor:
+    def student_extra_info(self, img_mask=None) -> dict:
+        extra = dict(self.extra_info)
+        if img_mask is not None:
+            extra["img_mask"] = img_mask
+        return extra
+
+    def recon_loss(self, eps, target, img_mask=None, fg_mask=None) -> torch.Tensor:
+        """distill_loss without masks (bit-identical to the unmasked step), calc_recon_loss with them."""
+        if img_mask is None and fg_mask is None:
+            return distill_loss(eps, target)
+        return calc_recon_loss(eps, target, img_mask, fg_mask, self.fg_pixel_weight, self.bg_pixel_weight)
+
+    def graphed(self):
+        from .train import GraphedUNetLoss
+        return self.__dict__.setdefault("_graphed", GraphedUNetLoss(self.unet, self.extra_info, self.fg_pixel_weight,
+                                                                    self.bg_pixel_weight))
+
+    def loss(self, x0, t, noise, teacher_eps, face_embs, tokens, img_mask=None, fg_mask=None) -> torch.Tensor:
+        for name, m in (("img_mask", img_mask), ("fg_mask", fg_mask)):
+            if m is not None:
+                check_image_mask(m, x0, name)
         if teacher_eps is None:
             teacher_eps = self.teacher_eps(x0, t, noise, face_embs)
         c = self.context(face_embs, tokens)
-        eps = unet_forward_train(self.unet, self.q_sample(x0, t, noise), t, c, dict(self.extra_info))
-        return distill_loss(eps, teacher_eps)
+        eps = unet_forward_train(self.unet, self.q_sample(x0, t, noise), t, c, self.student_extra_info(img_mask))
+        return self.recon_loss(eps, teacher_eps, img_mask, fg_mask)
 
     def multi_step_backward(self, batch: Dict[str, torch.Tensor], num_denoising_steps: int, accum: int = 1,
                             use_graph: bool = False) -> torch.Tensor:
@@ -437,6 +485,7 @@ class DistillStep:
         if self.teacher is None:
             raise RuntimeError("DistillStep.multi_step_backward needs the Arc2Face teacher")
         x0, t, noise, face_embs, tokens = batch["x0"], batch["t"], batch["noise"], batch["face_embs"], batch["tokens"]
+        img_mask, fg_mask = batch_masks(batch)
         ND = int(num_denoising_steps)
         with torch.no_grad():
             prompt_embs, _ = arc2face_forward_face_embs(self.tokenizer, self.arc2face, face_embs, input_max_length=21,
@@ -448,16 +497,15 @@ class DistillStep:
         norm = 1.0 / math.sqrt(ND)
         total, grad_c = None, None
         if use_graph:
-            from .train import GraphedUNetLoss
-            g = self.__dict__.setdefault("_graphed", GraphedUNetLoss(self.unet, self.extra_info))
+            g = self.graphed()
         for s in range(loss_start_step, ND):
             x_s = self.q_sample(pred_x0s[s - 1].float(), ts[s], noises[s].float())
             if use_graph:
-                ls, gs = g(x_s, ts[s], c.detach(), preds[s].float())
+                ls, gs = g(x_s, ts[s], c.detach(), preds[s].float(), img_mask, fg_mask)
                 grad_c = gs if grad_c is None else grad_c + gs
             else:
-                eps = unet_forward_train(self.unet, x_s, ts[s], c, dict(self.extra_info))
-                ls = distill_loss(eps, preds[s].float())
+                eps = unet_forward_train(self.unet, x_s, ts[s], c, self.student_extra_info(img_mask))
+                ls = self.recon_loss(eps, preds[s].float(), img_mask, fg_mask)
             total = ls if total is None else total + ls
         total = total * norm
         if use_graph:
@@ -470,22 +518,22 @@ class DistillStep:
         """loss / accum backpropagated into the trainable parameters' .grad; returns the detached loss (no host sync).
         use_graph: UNet forward + backward-to-context replayed from one CUDA graph (train.GraphedUNetLoss)."""
         x0, t, noise, face_embs, tokens = batch["x0"], batch["t"], batch["noise"], batch["face_embs"], batch["tokens"]
+        img_mask, fg_mask = batch_masks(batch)
         teacher_eps = batch.get("teacher_eps")
         if teacher_eps is None:
             teacher_eps = self.teacher_eps(x0, t, noise, face_embs)
         if not use_graph:
-            loss = self.loss(x0, t, noise, teacher_eps, face_embs, tokens)
+            loss = self.loss(x0, t, noise, teacher_eps, face_embs, tokens, img_mask, fg_mask)
             (loss / accum).backward()
             return loss.detach()
-        from .train import GraphedUNetLoss
         c = self.context(face_embs, tokens)
-        g = self.__dict__.setdefault("_graphed", GraphedUNetLoss(self.unet, self.extra_info))
-        loss, grad_c = g(self.q_sample(x0, t, noise), t, c.detach(), teacher_eps)
+        loss, grad_c = self.graphed()(self.q_sample(x0, t, noise), t, c.detach(), teacher_eps, img_mask, fg_mask)
         c.backward(grad_c * (1.0 / accum))
         return loss
 
     def micro_step(self, batch: Dict[str, torch.Tensor], accum: int = 1) -> float:
-        loss = self.loss(batch["x0"], batch["t"], batch["noise"], batch.get("teacher_eps"), batch["face_embs"], batch["tokens"])
+        loss = self.loss(batch["x0"], batch["t"], batch["noise"], batch.get("teacher_eps"), batch["face_embs"], batch["tokens"],
+                         *batch_masks(batch))
         (loss / accum).backward()
         return float(loss.detach())
 
@@ -503,8 +551,9 @@ class GraphedAccumStep:
     * Every parameter gradient is accumulated in place into its GradBucket view; nothing on the path reads back to the
       host (no .item(), no nonzero, token ids and the schedule resident on the device), so the only per-replay host
       work is copying the batches into the static buffers.
-    Recaptured when the geometry, the parameter storage (Prodigy re-binds parameters into its bucket at its first step)
-    or a weight pack of a frozen module changes."""
+    Recaptured when the geometry, the set of masks the micro-batches carry (MASK_KEYS: static buffers too), the
+    parameter storage (Prodigy re-binds parameters into its bucket at its first step) or a weight pack of a frozen
+    module changes."""
 
     KEYS = ("x0", "t", "noise", "face_embs", "tokens", "teacher_eps")
 
@@ -512,14 +561,17 @@ class GraphedAccumStep:
         self.step, self.bucket, self.accum, self.fuse_unet = step, bucket, accum, fuse_unet
         self._g = {}
 
+    def _keys(self, batch):
+        return self.KEYS + tuple(k for k in MASK_KEYS if batch.get(k) is not None)
+
     def _key(self, batches):
         from .attention import PackedModule
         ps = self.bucket.params
-        return (tuple((tuple(b[k].shape), b[k].dtype) for b in batches for k in self.KEYS), ps[0].data_ptr(),
+        return (tuple((k, tuple(b[k].shape), b[k].dtype) for b in batches for k in self._keys(b)), ps[0].data_ptr(),
                 ps[-1].data_ptr(), PackedModule.PACK_EPOCH, self.fuse_unet)
 
     def _build(self, batches):
-        st = {"in": [{k: b[k].clone() for k in self.KEYS} for b in batches]}
+        st = {"in": [{k: b[k].clone() for k in self._keys(b)} for b in batches]}
         step, n = self.step, len(batches)
 
         def run():
@@ -534,17 +586,19 @@ class GraphedAccumStep:
                 # sum_k MSE_k / accum has the same gradient either way.
                 ck = c.detach().clone().requires_grad_(True)
                 x0, t, noise = (torch.cat([i[key] for i in ins]) for key in ("x0", "t", "noise"))
-                eps = unet_forward_train(step.unet, step.q_sample(x0, t, noise), t, ck, dict(step.extra_info))
+                img_mask = torch.cat([i["img_mask"] for i in ins]) if "img_mask" in ins[0] else None
+                eps = unet_forward_train(step.unet, step.q_sample(x0, t, noise), t, ck, step.student_extra_info(img_mask))
                 per = eps.shape[0] // n
-                ls = [distill_loss(eps[k * per:(k + 1) * per], i["teacher_eps"]) for k, i in enumerate(ins)]
+                ls = [step.recon_loss(eps[k * per:(k + 1) * per], i["teacher_eps"], i.get("img_mask"), i.get("fg_mask"))
+                      for k, i in enumerate(ins)]
                 (g,) = torch.autograd.grad(sum(ls), ck)
                 c.backward(g * (1.0 / self.accum))
                 return torch.stack([l.detach() for l in ls])
             for k, i in enumerate(ins):
                 ck = c.detach()[k * rows:(k + 1) * rows].clone().requires_grad_(True)
                 eps = unet_forward_train(step.unet, step.q_sample(i["x0"], i["t"], i["noise"]), i["t"], ck,
-                                         dict(step.extra_info))
-                loss = distill_loss(eps, i["teacher_eps"])
+                                         step.student_extra_info(i.get("img_mask")))
+                loss = step.recon_loss(eps, i["teacher_eps"], i.get("img_mask"), i.get("fg_mask"))
                 (g,) = torch.autograd.grad(loss, ck)
                 losses.append(loss.detach())
                 grads.append(g)
@@ -569,13 +623,16 @@ class GraphedAccumStep:
 
     def __call__(self, batches: Sequence[Dict[str, torch.Tensor]]) -> torch.Tensor:
         """-> the micro-batch losses [accum] (detached); the gradients of sum_i loss_i / accum are added to the bucket."""
+        check_mask_presence(batches)
+        for b in batches:
+            batch_masks(b)
         key = self._key(batches)
         st = self._g.get(key)
         if st is None:
             self._g.clear()                             # one live geometry: a stale capture holds GBs of activations
             st = self._g[key] = self._build(batches)
         for dst, b in zip(st["in"], batches):
-            for k in self.KEYS:
+            for k in dst:
                 dst[k].copy_(b[k])
         st["graph"].replay()
         return st["losses"].clone()
@@ -604,6 +661,9 @@ class Stage1Trainer:
         """-> {"loss": 0-d tensor (mean over the micro-batches), "grad_norm": 0-d tensor (before clipping)}."""
         if len(batches) != self.accum:
             raise ValueError(f"expected {self.accum} micro-batches, got {len(batches)}")
+        check_mask_presence(batches)
+        for b in batches:
+            batch_masks(b)
         self.bucket.begin_step()
         if self._gstep is not None:
             # the teacher (no grad) runs outside the captured step

@@ -158,6 +158,20 @@ int af_attention_bwd_bf16(const void* Q, long long ldq, const void* K, long long
                           void* dK, long long lddk, void* dV, long long lddv, int B, int heads, int N, int d,
                           af_stream_t stream);
 
+/* Same with a key mask: key_mask [B][N] bytes, 1 = attend, 16-byte aligned; the backward of af_attention_bf16_lse with
+ * that mask (attention.py:223-232; the reference fills masked scores with -finfo.max before the softmax, so its
+ * autograd gives masked keys no score gradient).  Where a sample keeps a key: P_ij = m_j ? exp2(S_ij - lse_i) : 0 and
+ * dS_ij = m_j ? ln2 P_ij (dP_ij - delta_i) : 0, so the dK / dV rows of masked keys are exactly 0.  Where it keeps none
+ * (lse = +inf in every row; the forward output is the mean of V): P_ij = 1/N and dS = 0, so dQ = dK = 0 and
+ * dV_j = (1/N) sum_i dO_i.  The mask is applied by selection: masked K / V rows reach no gradient whatever they hold,
+ * and an all-ones mask gives results bit-identical to af_attention_bwd_bf16. */
+int af_attention_bwd_masked_bf16(const void* Q, long long ldq, const void* K, long long ldk, const void* Vp,
+                                 long long ldv, const void* dOp, long long lddo, const void* QT, long long ldqt,
+                                 const void* KT, long long ldkt, const void* dOT, long long lddot, const float* lse,
+                                 const float* delta, const unsigned char* key_mask, void* dQ, long long lddq, void* dK,
+                                 long long lddk, void* dV, long long lddv, int B, int heads, int N, int d,
+                                 af_stream_t stream);
+
 /* af_attention_bf16 on the long-sequence kernel (d in {40, 80}, Nk > 128 and a multiple of 128 / 64, no mask) with an
  * in-kernel clock64 timeline - a measurement aid (scripts/attn_tile_trace.py), results are those of af_attention_bf16.
  * trace: caller-owned device buffer of 512*64*8 + 512 + 2*64*8 int64: [first 512 CTAs (linear id)][key block < 64][8]
@@ -290,6 +304,13 @@ typedef struct af_bgemm {
   float alpha;
 } af_bgemm;
 int af_bgemm_bf16(const af_bgemm* g, af_stream_t stream);
+/* af_bgemm_bf16 modes 1-4 with a key mask (attention.py:223-232, as af_attention_bwd_masked_bf16): the mask bytes of
+ * batch z start at key_mask + b0*sM0 + b1*sM1 and index the columns of modes 1 / 3 (keys are columns) and the rows of
+ * modes 2 / 4 (keys are rows).  A masked key gets P = 0 and dS = 0, except that where vec = +inf (a sample that keeps
+ * no key) modes 1 / 2 write P = 1/valid_cols resp. 1/valid_rows.  Selection only; an all-ones mask gives results
+ * bit-identical to af_bgemm_bf16. */
+int af_bgemm_masked_bf16(const af_bgemm* g, const unsigned char* key_mask, long long sM0, long long sM1,
+                         af_stream_t stream);
 
 /* GroupNorm(32)(+SiLU) backward w.r.t. the fp32 input: x [B,HW,C], mean_rstd [B,32,2] (af_groupnorm_finalize),
  * dy bf16 [B,HW,C] (gradient of the bf16 output), dres fp32 or NULL (added: gradient of a residual branch), dx fp32.
